@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- contrastive fwd+bwd pairs/s of the CVCL hot path on B200 (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload ...]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
 
 Workload (default `flat512`, BASELINE.json configs[1]): CVCL flat-embedding contrastive train
 step, 512 synthetic pairs per GPU (max utterance length 25, E=512, K=2048, V=2350), bf16 operands
@@ -20,6 +20,11 @@ One JSON line on stdout (rank 0):
   cpu_baseline the oracle port (same ATen fp32 op sequence as the reference) on the host cores
 
 `--impl reference` times that CPU path alone (rank 0 only) and prints the same line shape.
+
+`--dump-outputs DIR` writes what the timed step returned in its last timed step as DIR/<name>.npy (float32):
+the five loss / metric scalars and the gradients of s, the head weight and bias and the embedding table
+(rank 0's, about 9 MB).  Inputs and weights come from fixed seeds, so two builds can be compared array by
+array; on one GPU the reference arm runs the same batch and writes the same names.
 """
 import argparse
 import json
@@ -73,6 +78,37 @@ def synth_batch(seed, B):
 def synth_weights():
     from oracle import cvcl_oracle as O
     return O.synth_weights(np.random.RandomState(0), E, K, V)
+
+
+SCALAR_NAMES = ("loss", "image_accuracy", "text_accuracy", "image_entropy", "text_entropy")
+
+
+def step_outputs(m, out, world):
+    """host float32 copies of what the timed B200 step returned: flat_contrastive_step's (out5, ., ., grads) at
+    N = 1, flat_step_sharded's ([out5 | grads], ., .) at N > 1, or the loss of the public API (eager fallback)."""
+    if torch.is_tensor(out):
+        return {"loss": out.detach().float().cpu().numpy().reshape(())}
+    stats, flat = (out[0], out[3]) if world == 1 else (out[0][:8], out[0][8:])
+    stats, flat = stats.detach().cpu().numpy(), flat.detach()
+    res = {name: stats[i].reshape(()) for i, name in enumerate(SCALAR_NAMES)}
+    ds, db, dtable, dW = m.ops.split_flat_grads(flat, E, K, V)
+    res.update(grad_s=ds.cpu().numpy().reshape(()), grad_fc_bias=db.cpu().numpy(),
+               grad_embedding=dtable.cpu().numpy(), grad_fc_weight=dW.cpu().numpy())
+    return res
+
+
+def reference_outputs(out):
+    """the same names from the oracle step's result dict (cvcl_oracle.contrastive_step)."""
+    res = {name: out[name].detach().float().numpy().reshape(()) for name in SCALAR_NAMES}
+    res.update(grad_s=out["ds"].numpy().reshape(()), grad_fc_bias=out["db"].numpy(),
+               grad_embedding=out["dtable"].numpy(), grad_fc_weight=out["dW"].numpy())
+    return res
+
+
+def write_outputs(d, arrays):
+    os.makedirs(d, exist_ok=True)
+    for name, v in arrays.items():
+        np.save(os.path.join(d, name + ".npy"), np.asarray(v, dtype=np.float32))
 
 
 class ClockSampler:
@@ -433,13 +469,13 @@ def cpu_reference_step_fn(B):
     tW, tb, tt = torch.from_numpy(W), torch.from_numpy(b), torch.from_numpy(table)
 
     def fn():
-        return O.contrastive_step(tf, tids, tl, tW, tb, tt, S_FIXED)["loss"]
+        return O.contrastive_step(tf, tids, tl, tW, tb, tt, S_FIXED)
     return fn
 
 
 def time_cpu(B, steps, warmup, budget_s=None):
-    """-> (seconds per step, steps timed).  budget_s bounds the timed region: the number of timed steps
-    is cut to what fits (estimated from the warm-up steps), never below 3."""
+    """-> (seconds per step, steps timed, result of the last step).  budget_s bounds the timed region: the
+    number of timed steps is cut to what fits (estimated from the warm-up steps), never below 3."""
     torch.set_num_threads(os.cpu_count() or 1)
     fn = cpu_reference_step_fn(B)
     t0 = time.perf_counter()
@@ -450,9 +486,9 @@ def time_cpu(B, steps, warmup, budget_s=None):
         steps = max(3, min(steps, int(budget_s / est)))
     t0 = time.perf_counter()
     for _ in range(steps):
-        fn()
+        out = fn()
     dt = (time.perf_counter() - t0) / steps
-    return dt, steps
+    return dt, steps, out
 
 
 # ----------------------------------------------------------------------------------------------
@@ -465,7 +501,10 @@ def main():
     ap.add_argument("--pairs-per-gpu", type=int, default=512)
     ap.add_argument("--no-breakdown", action="store_true", help="(kept for old command lines; ignored)")
     ap.add_argument("--no-configs", action="store_true", help="skip the bounded runs of BASELINE configs 1, 3, 4, 5")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step as DIR/<name>.npy")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
     if a.warmup < 3:
         a.warmup = 3
     rank = int(os.environ.get("RANK", "0"))
@@ -488,12 +527,14 @@ def main():
         if rank != 0:
             return
         # the same workload as the B200 arm at this N: the global batch of B * world pairs in one process
-        # (the reference is single-process); timed steps are bounded to about 90 s of CPU work
+        # (the reference is single-process)
         Bref = B * max(world, a.gpus, 1)
         config["global_batch"] = Bref
         config["workload"] = config["workload"].replace("global InfoNCE batch %d" % (B * max(world, 1)),
                                                         "global InfoNCE batch %d" % Bref)
-        dt, steps = time_cpu(Bref, a.steps, a.warmup, budget_s=90.0)
+        dt, steps, last = time_cpu(Bref, a.steps, a.warmup)
+        if a.dump_outputs:
+            write_outputs(a.dump_outputs, reference_outputs(last))
         val = Bref / dt
         cores = os.cpu_count() or 1
         print(json.dumps({
@@ -501,9 +542,9 @@ def main():
             "steps": steps, "warmup": a.warmup, "ms_per_step": dt * 1e3, "higher_is_better": True,
             "scaling": "weak", "vs_baseline": None, "dtype": "f32", "data": "synthetic", "config": config,
             "cpu_baseline": {"value": val, "unit": "pairs/s", "cores": cores, "kind": "port",
-                             "sample": "%d of the %d requested steps (bounded to ~90 s) of the B=%d flat train step "
+                             "sample": "%d steps of the B=%d flat train step "
                                        "(oracle port of the reference's ATen fp32 op sequence, torch %d threads)"
-                                       % (steps, a.steps, Bref, cores)},
+                                       % (steps, Bref, cores)},
             "e2e": {"value": val, "unit": "pairs/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
             "gpu_launches": 0}))
         return
@@ -599,10 +640,13 @@ def main():
     for _ in range(a.steps):
         flush.zero_()
         e0 = torch.cuda.Event(enable_timing=True); e1 = torch.cuda.Event(enable_timing=True)
-        e0.record(); run_step(); e1.record()
+        e0.record(); out = run_step(); e1.record()
         evs.append((e0, e1))
     barrier()
     t_wall = time.perf_counter() - t_wall0
+    dumped = None
+    if a.dump_outputs and rank == 0:
+        dumped = step_outputs(m, g_out if graph is not None else out, world)
     step_ms = [e0.elapsed_time(e1) for e0, e1 in evs]
     ms = statistics.mean(step_ms)
     n_launch = lib.cvcl_launch_count() - n0
@@ -619,13 +663,15 @@ def main():
         for _ in range(a.steps):
             flush.zero_()
             e0 = torch.cuda.Event(enable_timing=True); e1 = torch.cuda.Event(enable_timing=True)
-            e0.record(); raw_step(); e1.record()
+            e0.record(); out = raw_step(); e1.record()
             evs2.append((e0, e1))
         barrier()
         direct_ms = [e0.elapsed_time(e1) for e0, e1 in evs2]
         ms_direct = statistics.mean(direct_ms)
         if ms_direct < ms:
             ms, step_ms, launch_form = ms_direct, direct_ms, "direct launch"
+            if dumped is not None:
+                dumped = step_outputs(m, out, world)
     # The clock samples belong to the device-timed region.  K steps can be shorter than the poller's 50 ms period, so
     # the same step keeps running (untimed) until two samples exist; then the poller is stopped: its driver queries
     # must not sit on the host path of the wall-clock e2e loops below.
@@ -653,7 +699,7 @@ def main():
 
     # ------------------------------------------------------------------ e2e through the public API
     # (a) eager: MultiModalModel.calculate_contrastive_loss(...) + backward(), pinned host inputs
-    e2e_steps = max(500, min(a.steps, 2000))     # wall-clock timed: enough calls that start-up effects do not dominate
+    e2e_steps = a.steps     # --steps sets the wall-clock timed loops too; few steps let start-up effects show
     for _ in range(3):
         x.copy_(x_host, non_blocking=True); step_api(model, x, ids_d, lens_d, world).item()
     barrier()
@@ -731,7 +777,7 @@ def main():
         # the headline e2e, which starts from pinned memory as the contract says
         src_sets = [(torch.from_numpy(f).to(torch.bfloat16), torch.from_numpy(ids), torch.from_numpy(lens)),
                     (torch.from_numpy(f2).to(torch.bfloat16), torch.from_numpy(ids2), torch.from_numpy(lens2))]
-        n_rs = max(100, e2e_steps // 2)
+        n_rs = e2e_steps
         barrier()
         t0 = time.perf_counter()
         for k in range(n_rs):
@@ -792,10 +838,12 @@ def main():
         finish()
         return
 
+    if dumped is not None:
+        write_outputs(a.dump_outputs, dumped)
     cpu = None
     if world == 1:
         n_cpu = 40
-        cdt, n_cpu = time_cpu(B, n_cpu, 3, budget_s=30.0)
+        cdt, n_cpu, _ = time_cpu(B, n_cpu, 3, budget_s=30.0)
         cores = os.cpu_count() or 1
         cpu = {"value": B / cdt, "unit": "pairs/s", "cores": cores, "kind": "port", "ms_per_step": cdt * 1e3,
                "sample": "%d steps of the same B=%d flat train step (oracle port: the reference's ATen fp32 op "

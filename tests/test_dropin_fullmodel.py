@@ -1,25 +1,23 @@
 """BASELINE config 1 and the true drop-in case (INTEGRATION.md section 2).
 
-CPU (build container only, skipped where /root/reference is absent): the drop-in MultiModalModel is constructed with
-the REFERENCE's own VisionEncoder / TextEncoder objects -- exactly what multimodal_lit.py:61-65 does after the import
-swap -- and must expose the reference's state_dict keys, attributes and trunk boundary.
+CPU: the drop-in MultiModalModel with the full seeded ResNeXt-50 trunk keeps the reference's parameter paths,
+attributes and temperature (tests/golden/state_dict_keys.json) and, run on the host, gives the trunk-boundary
+activations and image features the unmodified reference gave on the same seeded trunk and images.
 
 GPU: the full model (seeded ResNeXt-50 trunk as the stock torch module + this library's head) through
 calculate_contrastive_loss / forward / encode_image against goldens produced by the unmodified reference
 (oracle/make_golden_fullmodel.py), flat and spatial (mean, max)."""
 import argparse
+import json
 import os
 
 import numpy as np
 import pytest
 import torch
 
-from _util import ROOT, assert_logits_close, golden, t
-from oracle import ref_import as R
+from _util import GOLD, O, ROOT, assert_logits_close, golden, t
 from oracle.make_golden import case_inputs
 from oracle.make_golden_fullmodel import load_trunk, seeded_images, seeded_trunk
-
-needs_ref = pytest.mark.skipif(not R.reference_available(), reason="reference tree not present (GPU box)")
 
 
 def _load_head(model, inp, embedding_type):
@@ -34,47 +32,55 @@ def _load_head(model, inp, embedding_type):
         model.text_embed.embedding.weight.copy_(torch.from_numpy(inp["table"]))
 
 
-@needs_ref
 @pytest.mark.parametrize("embedding_type,sim,fix", [("flat", "mean", False), ("flat", "mean", True), ("spatial", "max", False)])
-def test_dropin_with_reference_encoders_cpu(embedding_type, sim, fix):
-    import contextlib, io, warnings
+def test_dropin_full_model_matches_reference_cpu(embedding_type, sim, fix):
     import multimodal_baby_b200 as cv
-    ref_mm, _ = R.load_reference()
-    args = R.make_args(embedding_type, sim, 512, fix)
-    vocab = R.reference_vocab()
-    with contextlib.redirect_stdout(io.StringIO()), warnings.catch_warnings():
-        warnings.simplefilter("ignore")
-        ve = ref_mm.VisionEncoder(args)
-        te = ref_mm.TextEncoder(vocab, ve.last_cnn_out_dim, args)
-        ref_model = ref_mm.MultiModalModel(ve, te, args)
-    mine = cv.MultiModalModel(ve, te, args)               # the reference's OWN encoder objects
-    assert list(mine.state_dict().keys()) == list(ref_model.state_dict().keys())
+    name = "fullmodel_flat_b8" if embedding_type == "flat" else "fullmodel_spatial_%s_b8" % sim
+    g = golden(name)
+    args = argparse.Namespace(embedding_type=embedding_type, embedding_dim=int(g["E"]), normalize_features=True,
+                              fix_temperature=fix, temperature=0.07, text_encoder="embedding",
+                              cnn_model="resnext50_32x4d", finetune_cnn=False, sim=sim)
+    vocab = {str(i): i for i in range(2350)}
+    mine = cv.MultiModalModel(cv.VisionEncoder(args, trunk="resnext"), cv.TextEncoder(vocab, 2048, args), args)
+    # the trunk parameters sit at torchvision's paths (load_trunk rejects missing or unexpected trunk keys) ...
+    load_trunk(mine.image_embed, seeded_trunk(), embedding_type)
     assert len(mine.state_dict()) > 300                    # the whole ResNeXt trunk is in there
-    for name in ("normalize_features", "sim", "embedding_type", "fix_temperature", "image_embed", "text_embed",
+    # ... and everything outside the trunk where the reference keeps it
+    with open(os.path.join(GOLD, "state_dict_keys.json")) as fh:
+        ref = json.load(fh)["%s_fix%d" % (embedding_type, int(fix))]
+    ref_keys = [k[len("model."):] for k in ref["state_dict"] if k.startswith("model.")]
+    assert sorted(k for k in mine.state_dict() if not k.startswith("image_embed.")) == \
+        [k for k in ref_keys if not k.startswith("image_embed.")]
+    for attr in ("normalize_features", "sim", "embedding_type", "fix_temperature", "image_embed", "text_embed",
                  "logit_neg_log_temperature"):
-        assert hasattr(mine, name)
-    assert isinstance(mine.logit_neg_log_temperature, torch.nn.Parameter) == (not fix)
-    assert float(mine.logit_neg_log_temperature) == pytest.approx(float(ref_model.logit_neg_log_temperature))
+        assert hasattr(mine, attr)
+    assert isinstance(mine.logit_neg_log_temperature, torch.nn.Parameter) == ref["temperature_is_parameter"] == (not fix)
+    assert mine.logit_neg_log_temperature.item() == pytest.approx(ref["temperature_value"])
     # the head parameters are found where the reference keeps them
     w, b = mine._head()
     assert tuple(w.shape) == (512, 2048) and tuple(b.shape) == (512,)
-    # trunk boundary on CPU (the trunk is a stock torch module): pooled / layer4 activations equal the reference's
-    ve.eval()
-    x = seeded_images(5, n=2)
+    # trunk boundary on CPU (the trunk is a stock torch module) and the head on top of it: what the reference computed
+    inp = case_inputs(int(g["seed"]), int(g["B"]), int(g["E"]), embedding_type)
+    _load_head(mine, inp, embedding_type)
+    mine.eval()
+    x = seeded_images(int(g["seed"]) + 1)
     with torch.no_grad():
         boundary, fmap = cv.split_trunk_forward(mine.image_embed, x, run_head=False)
-        ref_feat, ref_fmap = ve(x)
-    assert torch.equal(fmap, ref_fmap)
+        feats = O.encode_image(boundary, w, b, embedding_type)
+    assert tuple(fmap.shape) == tuple(g["feature_map_shape"])
+    assert abs(float(fmap.mean()) - float(g["feature_map_mean"])) <= 1e-5 * abs(float(g["feature_map_mean"]))
+    assert abs(float(fmap.abs().max()) - float(g["feature_map_abs_max"])) <= 1e-5 * float(g["feature_map_abs_max"])
     if embedding_type == "flat":
-        assert tuple(boundary.shape) == (2, 2048)
-        assert torch.allclose(boundary, torch.flatten(torch.nn.functional.adaptive_avg_pool2d(ref_fmap, 1), 1), atol=1e-6)
-        # head applied by torch on CPU reproduces the reference's features: the split is exact
-        assert torch.allclose(torch.nn.functional.linear(boundary, w, b), ref_feat, atol=1e-5)
+        assert torch.allclose(boundary, fmap.mean((2, 3)), atol=1e-6)
+        assert float((boundary[:, :16] - torch.from_numpy(g["pooled_head"])).abs().max()) <= \
+            1e-5 * float(np.abs(g["pooled_head"]).max())
+        assert float((feats - torch.from_numpy(g["image_features"])).abs().max()) <= 1e-5
     else:
         assert torch.equal(boundary, fmap)
+        assert float((feats[:2, :, :2, :2] - torch.from_numpy(g["image_features_slice"])).abs().max()) <= 1e-5
     # the CUDA-only contract: CPU tensors raise instead of silently taking another path
     with pytest.raises(RuntimeError):
-        mine.calculate_contrastive_loss(x, torch.zeros(2, 25, dtype=torch.int64), torch.full((2,), 3, dtype=torch.int64))
+        mine.calculate_contrastive_loss(x, t(inp["ids"]), t(inp["lens"]))
 
 
 def _mirror_model(name, dev):

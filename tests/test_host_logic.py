@@ -16,13 +16,6 @@ from _util import GOLD, ROOT
 import multimodal_baby_b200 as cv
 
 
-def _vocab():
-    try:
-        return cv.load_vocab()
-    except FileNotFoundError:
-        return None
-
-
 def _args(**kw):
     d = dict(embedding_type="flat", embedding_dim=64, normalize_features=True, fix_temperature=False,
              temperature=0.07, text_encoder="embedding", sim="mean", dropout_o=0.0)
@@ -131,9 +124,9 @@ def test_state_dict_keys_match_reference(et, fix):
 
 
 def test_tokenize_matches_reference_golden():
-    vocab = _vocab()
-    if vocab is None:
-        pytest.skip("vocab.json not available")
+    """tokenize == the reference's tokenize on the same texts, with the entries of the reference's vocab.json that
+    these texts use (tokenize_vocab.json): <sos> / <eos>, <unk> for an unknown word, truncation to 25, padding."""
+    vocab = cv.load_vocab(os.path.join(GOLD, "tokenize_vocab.json"))
     with open(os.path.join(GOLD, "tokenize.json")) as fh:
         g = json.load(fh)
     a = _args()
