@@ -388,6 +388,26 @@ int cvcl_bicubic_upsample(const float* in, int N, int h, int w, int H, int W, fl
 int cvcl_eval_nway_fwd(const float* img, const float* txt, const int* txt_index, int n_trials, int n_way,
                        int E, int normalize, float log_scale, int* pred, float* logits, void* stream);
 
+/* ---- spatial-embedding evaluation (fp32 SIMT) ------------------------------------------------
+ * The batched form of the per-trial loop (eval.py:196-214, multimodal_lit.py:466-511) and of the n-category
+ * classification (multimodal_saycam_data_module.py:545-606) for embedding_type = "spatial".
+ *
+ * conv1x1: the 1x1-conv head (multimodal.py:181-185, applied at :101) in fp32 with fp32 FMA accumulation, the
+ * same arithmetic class as cvcl_linear_f32.  x [B,K,HW] is the layer4 map as the trunk emits it (NCHW, read in
+ * place), w [E,K] (16-byte aligned), bias [E] (nullable) -> out [B*HW, E] NHWC rows:
+ * out[b*HW + p, e] = bias[e] + sum_k w[e,k] x[b,k,p].  K % 4 == 0. */
+int cvcl_conv1x1_f32(const float* x, const float* w, const float* bias, int B, int K, int HW, int E, float* out,
+                     void* stream);
+/* spatial "max" logits (multimodal.py:771-780, then :783-787):
+ *   out = exp(log_scale) * (sum_{l < len[c]} max_p <img[m,p,:], tok[c,l,:]>) / len[c]
+ * img [M,HW,E] fp32 normalised location features (NHWC rows), tok [C,L,E] fp32 per-token text features, lens [C].
+ * Trial mode (n_way >= 1, M a multiple of n_way): image m is scored against label txt_index[m / n_way] (NULL =
+ * identity, then C >= M / n_way), out [M]; a label index outside [0, C) gives NaN.  Category mode (n_way = 0):
+ * every image against all C labels, out [M, C].  Each image block is read from HBM once; no atomics (a replay is
+ * bit-identical).  HW <= 256; the HW x E block must fit in shared memory (49 x 1024 does). */
+int cvcl_spatial_max_scores_f32(const float* img, const float* tok, const int64_t* lens, const int* txt_index, int M,
+                                int HW, int E, int C, int L, int n_way, float log_scale, float* out, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -202,9 +202,16 @@ int cvcl_spatial_pool(const float* src, int B, int HW, int E, float* out_f32, vo
     CVCL_REQUIRE(src && (out_f32 || out_bf16 || out_bf16_t), "spatial_pool: null pointer");
     CVCL_REQUIRE(E > 0 && E % 4 == 0 && HW > 0, "spatial_pool: bad shape");
     if (B == 0) return CVCL_OK;
-    dim3 grid(ceil_div(E / 4, 128), B);
-    CVCL_CHECK_CUDA(launch_pdl(spatial_pool_kernel, dim3(grid), dim3(128), 0, as_stream(stream), src, B, HW, E, out_f32, static_cast<__nv_bfloat16*>(out_bf16), ld, static_cast<__nv_bfloat16*>(out_bf16_t), ld_t));
-    count_launch();
+    for (int b0 = 0; b0 < B; b0 += 65535) {              // grid.y holds at most 65535 maps per launch
+        const int nb = B - b0 < 65535 ? B - b0 : 65535;
+        dim3 grid(ceil_div(E / 4, 128), nb);
+        CVCL_CHECK_CUDA(launch_pdl(spatial_pool_kernel, dim3(grid), dim3(128), 0, as_stream(stream),
+                                   src + static_cast<size_t>(b0) * HW * E, nb, HW, E,
+                                   out_f32 ? out_f32 + static_cast<size_t>(b0) * E : nullptr,
+                                   out_bf16 ? static_cast<__nv_bfloat16*>(out_bf16) + static_cast<size_t>(b0) * ld : nullptr, ld,
+                                   out_bf16_t ? static_cast<__nv_bfloat16*>(out_bf16_t) + b0 : nullptr, ld_t));
+        count_launch();
+    }
     return CVCL_OK;
 }
 
@@ -217,6 +224,73 @@ int cvcl_linear_f32(const float* A, int lda, const float* W, int ldw, const floa
     if (M == 0) return CVCL_OK;
     dim3 grid(ceil_div(N, 64), ceil_div(M, 64));
     CVCL_CHECK_CUDA(launch_pdl(linear_f32_kernel, grid, dim3(256), 0, as_stream(stream), A, lda, W, ldw, bias, M, N, K, C, ldc));
+    count_launch();
+    return CVCL_OK;
+}
+
+int cvcl_conv1x1_f32(const float* x, const float* w, const float* bias, int B, int K, int HW, int E, float* out,
+                     void* stream) {
+    CVCL_REQUIRE(x && w && out, "conv1x1_f32: null pointer");
+    CVCL_REQUIRE(B >= 0 && K > 0 && K % 4 == 0 && HW > 0 && E > 0, "conv1x1_f32: bad shape B=%d K=%d HW=%d E=%d", B, K, HW, E);
+    CVCL_REQUIRE((reinterpret_cast<uintptr_t>(w) & 15) == 0, "conv1x1_f32: weight not 16-byte aligned");
+    const long long M = static_cast<long long>(B) * HW;
+    CVCL_REQUIRE(M <= 0x7fffffffLL - 64 && ceil_div(E, 64) <= 65535, "conv1x1_f32: too many rows / channels");
+    if (M == 0) return CVCL_OK;
+    dim3 grid(static_cast<unsigned>((M + 63) / 64), ceil_div(E, 64));
+    CVCL_CHECK_CUDA(launch_pdl(conv1x1_f32_kernel, grid, dim3(256), 0, as_stream(stream), x, w, bias,
+                               static_cast<int>(M), E, K, HW, out));
+    count_launch();
+    return CVCL_OK;
+}
+
+int cvcl_spatial_max_scores_f32(const float* img, const float* tok, const int64_t* lens, const int* txt_index, int M,
+                                int HW, int E, int C, int L, int n_way, float log_scale, float* out, void* stream) {
+    CVCL_REQUIRE(img && tok && lens && out, "spatial_max_scores_f32: null pointer");
+    CVCL_REQUIRE(M >= 0 && C > 0 && L > 0 && n_way >= 0, "spatial_max_scores_f32: bad shape M=%d C=%d L=%d n_way=%d",
+                 M, C, L, n_way);
+    CVCL_REQUIRE(HW > 0 && HW <= 256, "spatial_max_scores_f32: HW=%d must be in [1, 256]", HW);
+    CVCL_REQUIRE(E > 0 && E % 4 == 0, "spatial_max_scores_f32: E=%d must be a multiple of 4", E);
+    CVCL_REQUIRE(((reinterpret_cast<uintptr_t>(img) | reinterpret_cast<uintptr_t>(tok)) & 15) == 0,
+                 "spatial_max_scores_f32: 16-byte alignment required");
+    CVCL_REQUIRE(n_way == 0 || M % n_way == 0, "spatial_max_scores_f32: M=%d is not a multiple of n_way=%d", M, n_way);
+    CVCL_REQUIRE(n_way == 0 || txt_index || M / n_way <= C,
+                 "spatial_max_scores_f32: %d trials without txt_index need as many labels (C=%d)", M / n_way, C);
+    if (M == 0) return CVCL_OK;
+    const int E4 = E / 4;
+    // token rows per chunk: every row a label needs in one chunk where possible, at most 4 rows per work item and
+    // 256 work items per block
+    const int rows_wanted = n_way > 0 ? L : (C * L < 64 ? C * L : 64);
+    int tt = (rows_wanted + 3) / 4 * 4;
+    const int tt_cap = 4 * (256 / HW) < 64 ? 4 * (256 / HW) : 64;
+    if (tt > tt_cap) tt = tt_cap;
+    int max_smem = 0, dev = 0;
+    CVCL_CHECK_CUDA(cudaGetDevice(&dev));
+    CVCL_CHECK_CUDA(cudaDeviceGetAttribute(&max_smem, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev));
+    int ks = 0, ld4 = 0;
+    size_t smem = 0;
+    for (;; tt -= 4) {
+        CVCL_REQUIRE(tt >= 4, "spatial_max_scores_f32: the %d x %d image block does not fit in shared memory", HW, E);
+        const int items = (tt / 4) * HW;
+        ks = 1;
+        while (ks < 32 && 2 * ks * items <= 256 && E4 % (2 * ks) == 0) ks *= 2;
+        // quarter-warps of 8 lanes read 8 distinct 16-byte bank groups when the row stride is = ks (mod 8)
+        ld4 = ks >= 8 ? E4 : E4 + ((ks - E4 % 8) + 8) % 8;
+        smem = static_cast<size_t>(HW) * ld4 * 16 + static_cast<size_t>(tt) * E4 * 16 +
+               static_cast<size_t>(tt) * HW * 4 + static_cast<size_t>(tt) * 12 + 8;
+        if (smem <= static_cast<size_t>(max_smem)) break;
+    }
+    static thread_local unsigned attr_mask = 0;         // per device: function attributes live in the device's context
+    const int attr_dev = dev >= 0 && dev < 32 ? dev : 0;
+    if (!((attr_mask >> attr_dev) & 1u)) {
+        CVCL_CHECK_CUDA(cudaFuncSetAttribute(spatial_max_scores_f32_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                             max_smem));
+        attr_mask |= 1u << attr_dev;
+    }
+    SpatialMaxScoreParams p{};
+    p.img = img; p.tok = tok; p.lens = reinterpret_cast<const long long*>(lens); p.txt_index = txt_index;
+    p.M = M; p.HW = HW; p.E = E; p.C = C; p.L = L; p.n_way = n_way; p.tt = tt; p.ks = ks; p.ld4 = ld4;
+    p.scale = expf(log_scale); p.out = out;
+    CVCL_CHECK_CUDA(launch_pdl(spatial_max_scores_f32_kernel, dim3(M), dim3(256), smem, as_stream(stream), p));
     count_launch();
     return CVCL_OK;
 }

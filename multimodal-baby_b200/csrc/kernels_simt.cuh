@@ -870,6 +870,221 @@ __global__ void __launch_bounds__(256) row_argmax_f32_kernel(const float* scores
     }
 }
 
+// out[b*HW + p, e] = bias[e] + sum_k W[e,k] x[b,k,p]: the spatial 1x1-conv head in fp32 (reference Conv2d(2048, E, 1),
+// multimodal.py:181-185), reading the layer4 map x [B,K,HW] in the NCHW layout the trunk emits and writing NHWC rows.
+// Same tiling and fp32 FMA order as linear_f32_kernel (64 x 64 tile, 4 x 4 per thread, 16-deep k slabs); only the
+// A loader differs: for a fixed k the 64 rows of a tile are consecutive locations, so each thread fetches 4 scalars
+// of one row at k, k+4, k+8, k+12 (coalesced along p) instead of a float4 along k.  Row tiles run along blockIdx.x
+// (B*HW reaches millions of rows).
+__global__ void __launch_bounds__(256) conv1x1_f32_kernel(const float* x, const float* W, const float* bias, int M,
+                                                          int N, int K, int HW, float* C) {
+    ptx::pdl_launch_dependents(); ptx::pdl_wait();
+    __shared__ float sa[16][65];
+    __shared__ float sw[16][65];
+    const int m0 = blockIdx.x * 64, n0 = blockIdx.y * 64;
+    const int tx = threadIdx.x & 15, ty = threadIdx.x >> 4;
+    const int lr = threadIdx.x >> 2, lk = (threadIdx.x & 3) * 4;        // W loader, as linear_f32_kernel
+    const int am = threadIdx.x & 63, ak = threadIdx.x >> 6;             // A loader: row am, k = ak + 4j
+    const int m_a = m0 + am;
+    const float* arow = nullptr;
+    if (m_a < M) {
+        const int b = m_a / HW, p = m_a - b * HW;
+        arow = x + static_cast<size_t>(b) * K * HW + p;
+    }
+    float acc[4][4];
+#pragma unroll
+    for (int i = 0; i < 4; ++i)
+#pragma unroll
+        for (int j = 0; j < 4; ++j) acc[i][j] = 0.f;
+    for (int k0 = 0; k0 < K; k0 += 16) {
+        float va[4];
+#pragma unroll
+        for (int j = 0; j < 4; ++j) {
+            const int k = k0 + ak + 4 * j;
+            va[j] = (arow && k < K) ? __ldg(arow + static_cast<size_t>(k) * HW) : 0.f;
+        }
+        float4 vw = make_float4(0.f, 0.f, 0.f, 0.f);
+        if (n0 + lr < N && k0 + lk < K) vw = __ldg(reinterpret_cast<const float4*>(W + static_cast<size_t>(n0 + lr) * K + k0 + lk));
+        __syncthreads();
+#pragma unroll
+        for (int j = 0; j < 4; ++j) sa[ak + 4 * j][am] = va[j];
+        sw[lk][lr] = vw.x; sw[lk + 1][lr] = vw.y; sw[lk + 2][lr] = vw.z; sw[lk + 3][lr] = vw.w;
+        __syncthreads();
+#pragma unroll
+        for (int kk = 0; kk < 16; ++kk) {
+            float a[4], w[4];
+#pragma unroll
+            for (int i = 0; i < 4; ++i) { a[i] = sa[kk][ty * 4 + i]; w[i] = sw[kk][tx * 4 + i]; }
+#pragma unroll
+            for (int i = 0; i < 4; ++i)
+#pragma unroll
+                for (int j = 0; j < 4; ++j) acc[i][j] = fmaf(a[i], w[j], acc[i][j]);
+        }
+    }
+#pragma unroll
+    for (int i = 0; i < 4; ++i) {
+        const int m = m0 + ty * 4 + i;
+        if (m >= M) continue;
+#pragma unroll
+        for (int j = 0; j < 4; ++j) {
+            const int n = n0 + tx * 4 + j;
+            if (n < N) C[static_cast<size_t>(m) * N + n] = acc[i][j] + (bias ? __ldg(bias + n) : 0.f);
+        }
+    }
+}
+
+// Spatial "max" score in fp32 for evaluation (multimodal.py:771-780):
+//   logit[m, c] = scale * (sum_{l < len[c]} max_p <img[m,p,:], tok[c,l,:]>) / len[c]
+// Rows of a label past its length are <pad> rows, zero after the per-token normalisation, and add exactly 0 in the
+// reference, so they are skipped.  Trial mode (n_way >= 1): image m is scored against label txt_index[m / n_way]
+// (identity when null) and out is [M]; category mode (n_way == 0): against all C labels, out [M, C].
+// One block per image.  The image's HW x E block is read from HBM once into shared memory (row stride ld4 float4,
+// padded so the quarter-warps of a k-split read distinct banks); the label token rows follow in chunks of <= tt rows,
+// staged in shared memory as well.  Thread (w, ks) owns work item w = (group of 4 token rows, location p) and the
+// k-slice ks (float4 indices ks, ks + KS, ...): four fp32 FMA chains, then a fixed butterfly over the KS lanes of the
+// item.  Maximum over the locations (NaN propagates, as torch.amax), then one thread adds the token maxima of each
+// label in position order.  No atomics: a replay is bit-identical.  A label index outside [0, C) scores NaN.
+struct SpatialMaxScoreParams {
+    const float* img;          // [M, HW, E] fp32, normalised location features (NHWC rows)
+    const float* tok;          // [C, L, E]  fp32 per-token text features
+    const long long* lens;     // [C]
+    const int* txt_index;      // [M / n_way] (trial mode, nullable)
+    int M, HW, E, C, L, n_way;
+    int tt;                    // token rows per chunk (multiple of 4)
+    int ks;                    // k-split lanes per work item (power of 2 <= 32, divides E/4)
+    int ld4;                   // shared-memory row stride of the image block, float4 units
+    float scale;               // exp(s)
+    float* out;
+};
+
+__global__ void __launch_bounds__(256) spatial_max_scores_f32_kernel(const SpatialMaxScoreParams p) {
+    extern __shared__ __align__(16) unsigned char sms_smem[];
+    ptx::pdl_launch_dependents(); ptx::pdl_wait();
+    const int m = blockIdx.x;
+    const int tid = threadIdx.x;
+    const int E4 = p.E >> 2;
+    float4* img_s = reinterpret_cast<float4*>(sms_smem);                         // [HW][ld4]
+    float4* tok_s = img_s + static_cast<size_t>(p.HW) * p.ld4;                   // [tt][E4]
+    float* dots = reinterpret_cast<float*>(tok_s + static_cast<size_t>(p.tt) * E4);   // [tt][HW]
+    float* tmax = dots + static_cast<size_t>(p.tt) * p.HW;                       // [tt]
+    int* slot_c = reinterpret_cast<int*>(tmax + p.tt);                           // [tt] label of the row
+    int* slot_l = slot_c + p.tt;                                                 // [tt] position (-1: last of label)
+    int* ctrl = slot_l + p.tt;                                                   // [0] rows in the chunk, [1] done
+
+    const float4* src = reinterpret_cast<const float4*>(p.img) + static_cast<size_t>(m) * p.HW * E4;
+    const int n4 = p.HW * E4;
+    for (int i0 = tid; i0 < n4; i0 += 4 * 256) {                                 // 4 loads in flight per thread
+        float4 v[4];
+#pragma unroll
+        for (int u = 0; u < 4; ++u) {
+            const int i = i0 + u * 256;
+            if (i < n4) v[u] = __ldcs(src + i);
+        }
+#pragma unroll
+        for (int u = 0; u < 4; ++u) {
+            const int i = i0 + u * 256;
+            if (i < n4) { const int q = i / E4; img_s[q * p.ld4 + (i - q * E4)] = v[u]; }
+        }
+    }
+
+    int c_cur = 0, c_end = p.C, l_cur = 0;           // thread 0's cursor over (label, position)
+    float run = 0.f;                                 // thread 0's running sum of the current label
+    if (p.n_way > 0) {
+        const int trial = m / p.n_way;
+        c_cur = p.txt_index ? __ldg(p.txt_index + trial) : trial;
+        c_end = c_cur + 1;
+        if (c_cur < 0 || c_cur >= p.C) {
+            if (tid == 0) p.out[m] = __int_as_float(0x7fffffff);
+            return;
+        }
+    }
+    const int ks = tid & (p.ks - 1);
+    const int w = tid / p.ks;
+    while (true) {
+        __syncthreads();                             // previous chunk consumed (and the image block stored)
+        if (tid == 0) {
+            int nt = 0;
+            while (nt < p.tt && c_cur < c_end) {
+                const long long len = __ldg(p.lens + c_cur);
+                const int n = static_cast<int>(len < 0 ? 0 : (len > p.L ? p.L : len));
+                if (n == 0) {                        // no token: 0 / len as the reference computes it
+                    const float v = (0.f / static_cast<float>(len)) * p.scale;
+                    p.out[p.n_way > 0 ? static_cast<size_t>(m) : static_cast<size_t>(m) * p.C + c_cur] = v;
+                    ++c_cur; continue;
+                }
+                slot_c[nt] = c_cur;
+                slot_l[nt] = (l_cur == n - 1) ? -1 : l_cur;
+                ++nt;
+                if (++l_cur == n) { l_cur = 0; ++c_cur; }
+            }
+            ctrl[0] = nt; ctrl[1] = nt == 0;
+        }
+        __syncthreads();
+        const int nt = ctrl[0];
+        if (ctrl[1]) break;
+        for (int i = tid; i < p.tt * E4; i += 256) {
+            const int r = i / E4, e = i - r * E4;
+            float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
+            if (r < nt) {
+                const int c = slot_c[r];
+                int l = slot_l[r];
+                if (l < 0) {                                         // last row of its label: position len - 1
+                    const long long len = __ldg(p.lens + c);
+                    l = static_cast<int>(len > p.L ? p.L : len) - 1;
+                }
+                v = __ldg(reinterpret_cast<const float4*>(p.tok) + (static_cast<size_t>(c) * p.L + l) * E4 + e);
+            }
+            tok_s[i] = v;
+        }
+        __syncthreads();
+        const int n_items = ((nt + 3) >> 2) * p.HW;
+        {
+            float acc[4] = {0.f, 0.f, 0.f, 0.f};
+            const int g = w / p.HW, q = w - g * p.HW;
+            if (w < n_items) {
+                const float4* xr = img_s + q * p.ld4;
+                const float4* t0 = tok_s + static_cast<size_t>(g) * 4 * E4;
+                for (int i = ks; i < E4; i += p.ks) {
+                    const float4 xv = xr[i];
+#pragma unroll
+                    for (int r = 0; r < 4; ++r) {
+                        const float4 tv = t0[r * E4 + i];
+                        acc[r] = fmaf(xv.x, tv.x, acc[r]); acc[r] = fmaf(xv.y, tv.y, acc[r]);
+                        acc[r] = fmaf(xv.z, tv.z, acc[r]); acc[r] = fmaf(xv.w, tv.w, acc[r]);
+                    }
+                }
+            }
+            for (int o = p.ks >> 1; o > 0; o >>= 1)
+#pragma unroll
+                for (int r = 0; r < 4; ++r) acc[r] += __shfl_xor_sync(0xffffffffu, acc[r], o);
+            if (w < n_items && ks == 0)
+#pragma unroll
+                for (int r = 0; r < 4; ++r) dots[(g * 4 + r) * p.HW + q] = acc[r];
+        }
+        __syncthreads();
+        if (tid < nt) {
+            float mx = -INFINITY;
+            for (int q = 0; q < p.HW; ++q) {
+                const float v = dots[tid * p.HW + q];
+                if (mx == mx && !(v <= mx)) mx = v;                  // a NaN location wins and stays
+            }
+            tmax[tid] = mx;
+        }
+        __syncthreads();
+        if (tid == 0) {
+            for (int r = 0; r < nt; ++r) {
+                run += tmax[r];
+                if (slot_l[r] < 0) {
+                    const int c = slot_c[r];
+                    const float v = (run / static_cast<float>(__ldg(p.lens + c))) * p.scale;
+                    p.out[p.n_way > 0 ? static_cast<size_t>(m) : static_cast<size_t>(m) * p.C + c] = v;
+                    run = 0.f;
+                }
+            }
+        }
+    }
+}
+
 // g[n,:] from u[n,:] and target[n,:]: one warp per image (F.normalize backward, eps 1e-12)
 __global__ void __launch_bounds__(128) gradcam_g_kernel(const float* u, const float* target, float* g, int N, int E,
                                                         int normalize) {

@@ -243,11 +243,19 @@ class MultiModalLitModel(_Base):
     @torch.no_grad()
     def evaluate_trials(self, trial_features, label_ids, label_lens, label_index=None, n_way=4,
                         from_trunk_boundary=True, want_logits=True):
-        """trial_features: [N, n_way, 2048] trunk-boundary activations (target first) or, with
-        from_trunk_boundary=False, [N, n_way, E] head outputs before normalisation.
+        """trial_features (target first): flat models take [N, n_way, 2048] trunk-boundary activations or,
+        with from_trunk_boundary=False, [N, n_way, E] head outputs before normalisation; spatial models
+        (embedding_type="spatial", sim "max" or "mean") take [N, n_way, 2048, H, W] layer4 maps or
+        [N, n_way, E, H, W] head outputs before normalisation.
         label_ids / label_lens: [C, L] / [C] token rows; label_index [N] picks the row per trial
-        (None: C == N).  Returns (pred int32 [N], logits fp32 [N, n_way] | empty); fp32 end to end."""
+        (None: C == N).  Returns (pred int32 [N], logits fp32 [N, n_way] | empty), the logits being
+        `logits_per_text[0]` of the reference's per-trial forward; fp32 end to end, first maximum wins."""
         m = self.model
+        if m.embedding_type == "spatial":
+            img = self._spatial_head_outputs(trial_features, (n_way,), from_trunk_boundary, "evaluate_trials")
+            txt = self._spatial_text(label_ids, label_lens, img.shape[1])
+            return ops.eval_nway_spatial(img, txt, label_lens, label_index, n_way, m.sim, bool(m.normalize_features),
+                                         ops._scalar(m.logit_neg_log_temperature), want_logits)
         table = m.text_embed.embedding.weight
         s = ops._scalar(m.logit_neg_log_temperature)
         txt = ops.text_features_flat(label_ids, label_lens, table, normalize=False)
@@ -262,14 +270,50 @@ class MultiModalLitModel(_Base):
     def classify_frames(self, frame_features, label_ids, label_lens, from_trunk_boundary=True, want_logits=True):
         """n-category classification (the reference's other Labeled-S form, multimodal_saycam_data_module.py:545-606:
         every frame against ALL C category labels, argmax over the categories).  frame_features [N, 2048] trunk-
-        boundary rows (or [N, E] head outputs with from_trunk_boundary=False); label_ids / label_lens [C, L] / [C].
+        boundary rows (or [N, E] head outputs with from_trunk_boundary=False); spatial models take [N, 2048, H, W]
+        layer4 maps (or [N, E, H, W] head outputs).  label_ids / label_lens [C, L] / [C].
         -> (pred int32 [N] = category row, logits_per_image fp32 [N, C] | empty); fp32 end to end."""
         m = self.model
         s = ops._scalar(m.logit_neg_log_temperature)
+        if m.embedding_type == "spatial":
+            img = self._spatial_head_outputs(frame_features, (), from_trunk_boundary, "classify_frames")
+            txt = self._spatial_text(label_ids, label_lens, img.shape[1])
+            return ops.classify_ncat_spatial(img, txt, label_lens, m.sim, bool(m.normalize_features), s, want_logits)
         txt = ops.text_features_flat(label_ids, label_lens, m.text_embed.embedding.weight, normalize=False)
         feats = frame_features.reshape(-1, frame_features.shape[-1]).float()
         if from_trunk_boundary:
             w, b = m._head()
             feats = ops.linear_f32(feats, w, b)
         return ops.classify_ncat(feats, txt, bool(m.normalize_features), s, want_logits)
+
+    def _spatial_head_outputs(self, x, lead, from_trunk_boundary, who):
+        """[N, *lead, channels, H, W] -> head outputs before normalisation as NHWC rows [N*prod(lead), H*W, E]:
+        the fp32 1x1-conv head on layer4 maps (channels = 2048), or the given head outputs (channels = E)."""
+        w, b = self.model._head()
+        chans = w.shape[1] if from_trunk_boundary else w.shape[0]
+        want = "[N, %s%d, H, W]" % ("".join("%d, " % d for d in lead), chans)
+        what = "layer4 maps" if from_trunk_boundary else "head outputs"
+        if (x.dim() != len(lead) + 4 or tuple(x.shape[1:1 + len(lead)]) != tuple(lead)
+                or x.shape[1 + len(lead)] != chans):
+            raise ValueError("%s: a spatial model takes %s of shape %s, got %s"
+                             % (who, what, want, tuple(x.shape)))
+        H, W = x.shape[-2:]
+        x = x.reshape(-1, chans, H, W)
+        if from_trunk_boundary:
+            rows = ops.conv1x1_f32(x, w, b)                               # fp32 head, NCHW read in place
+        else:
+            rows = x.float().permute(0, 2, 3, 1).reshape(-1, chans)        # NHWC rows
+        return rows.view(x.shape[0], H * W, -1)
+
+    def _spatial_text(self, label_ids, label_lens, hw):
+        """text side of the spatial scores from the model's own table: per-token features ("max") or the pooled
+        factor sum_l tok / (HW len) ("mean"), normalised per token iff normalize_features."""
+        m = self.model
+        table = m.text_embed.embedding.weight
+        if m.sim == "max":
+            tok, _ = ops.text_features_spatial(label_ids, label_lens, table, m.normalize_features)
+            return tok
+        _, pooled = ops.text_features_spatial(label_ids, label_lens, table, m.normalize_features, 1.0 / hw,
+                                              want_tok=False)
+        return pooled
 

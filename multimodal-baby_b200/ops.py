@@ -12,6 +12,8 @@ Reference call sites replaced (paths relative to the reference repo):
   sim_infonce       multimodal/multimodal.py:755, 783-787, 801-818 (+ autograd)
   flat_contrastive_step   multimodal/multimodal.py:796-822 + loss.backward()
   eval_nway         multimodal/multimodal_lit.py:466-511, eval.py:196-214
+  conv1x1_f32, eval_nway_spatial, classify_ncat_spatial
+                    the same evaluation for spatial embeddings (multimodal/multimodal.py:181-185, 757-787)
 """
 from __future__ import annotations
 
@@ -1073,6 +1075,11 @@ class _FlatContrastiveStepSharded(torch.autograd.Function):
 def linear_f32(x: Tensor, w: Tensor, bias: Optional[Tensor]) -> Tensor:
     """x [M,K] . w[N,K]^T + bias in fp32 with fp32 accumulation (cvcl_linear_f32): the exact-mode projection head
     of the evaluation path (no tensor cores, no library GEMM)."""
+    if x.dim() != 2 or w.dim() != 2 or w.shape[1] != x.shape[1]:
+        raise ValueError("linear_f32: x %s and w %s do not fit (need x [M,K], w [N,K])"
+                         % (tuple(x.shape), tuple(w.shape)))
+    if bias is not None and tuple(bias.shape) != (w.shape[0],):
+        raise ValueError("linear_f32: bias %s does not fit w %s" % (tuple(bias.shape), tuple(w.shape)))
     _need_cuda(x, w, bias)
     x = _f32(x); w = _f32(w)
     bias = _f32(bias) if bias is not None else None
@@ -1110,6 +1117,146 @@ def classify_ncat(img: Tensor, txt: Tensor, normalize: bool = True, log_scale: f
     if not want_logits:
         return pred, scores.new_empty((0,))
     return pred, scores * math.exp(float(log_scale))
+
+
+def _row_argmax(scores: Tensor) -> Tensor:
+    """first maximum of each row of a contiguous [M, N] fp32 matrix (torch.argmax semantics, NaN wins) -> int32 [M]."""
+    M, N = scores.shape
+    best = torch.empty((M,), dtype=torch.float32, device=scores.device)
+    pred = torch.empty((M,), dtype=torch.int32, device=scores.device)
+    _cabi.call("cvcl_row_argmax_f32", _p(scores), N, M, N, 0, 0, _p(best), _p(pred), _stream())
+    return pred
+
+
+# ----------------------------------------------------------------------------------------
+# spatial-embedding evaluation: fp32 1x1-conv head, spatial "max" / "mean" scores
+# ----------------------------------------------------------------------------------------
+def _conv_weight(w: Tensor) -> Tensor:
+    if w.dim() == 4 and tuple(w.shape[2:]) == (1, 1):
+        w = w.reshape(w.shape[0], w.shape[1])
+    if w.dim() != 2:
+        raise ValueError("conv1x1_f32: weight %s is not [E,K] or [E,K,1,1]" % (tuple(w.shape),))
+    return w
+
+
+@torch.library.custom_op(_NS + "::conv1x1_f32", mutates_args=())
+def conv1x1_f32(x: Tensor, w: Tensor, bias: Optional[Tensor]) -> Tensor:
+    """The spatial head Conv2d(K, E, 1) (multimodal.py:181-185) in fp32 with fp32 accumulation (cvcl_conv1x1_f32):
+    x [B,K,H,W] NCHW layer4 map (read in place), w [E,K] or [E,K,1,1], bias [E] | None -> [B*H*W, E] NHWC rows."""
+    w = _conv_weight(w)
+    if x.dim() != 4 or x.shape[1] != w.shape[1]:
+        raise ValueError("conv1x1_f32: x %s does not fit the weight %s (need x [B,%d,H,W])"
+                         % (tuple(x.shape), tuple(w.shape), w.shape[1]))
+    if bias is not None and tuple(bias.shape) != (w.shape[0],):
+        raise ValueError("conv1x1_f32: bias %s does not fit the weight %s" % (tuple(bias.shape), tuple(w.shape)))
+    _need_cuda(x, w, bias)
+    x = _f32(x); w = _f32(w)
+    bias = _f32(bias) if bias is not None else None
+    B, K, H, W = x.shape
+    E = w.shape[0]
+    out = torch.empty((B * H * W, E), dtype=torch.float32, device=x.device)
+    _cabi.call("cvcl_conv1x1_f32", _p(x), _p(w), _p(bias), B, K, H * W, E, _p(out), _stream())
+    return out
+
+
+@conv1x1_f32.register_fake
+def _(x, w, bias):
+    return x.new_empty((x.shape[0] * x.shape[2] * x.shape[3], w.shape[0]), dtype=torch.float32)
+
+
+def _location_rows(img: Tensor, normalize: bool) -> Tensor:
+    """[M, HW, E] head outputs -> the same as fp32 rows, F.normalize'd per location when `normalize`
+    (multimodal.py:736, dim=1 of the NCHW map = the E of each location)."""
+    M, HW, E = img.shape
+    rows = _f32(img).reshape(M * HW, E)
+    return (normalize_rows_f32(rows) if normalize else rows).view(M, HW, E)
+
+
+def _check_spatial_text(txt: Tensor, lens: Tensor, sim: str, E: int, who: str):
+    if sim == "max":
+        if txt.dim() != 3 or txt.shape[2] != E:
+            raise ValueError("%s: sim='max' takes per-token text features [C, L, %d], got %s" % (who, E, tuple(txt.shape)))
+        if lens.dim() != 1 or lens.shape[0] != txt.shape[0]:
+            raise ValueError("%s: lens %s does not fit %d labels" % (who, tuple(lens.shape), txt.shape[0]))
+    elif sim == "mean":
+        if txt.dim() != 2 or txt.shape[1] != E:
+            raise ValueError("%s: sim='mean' takes the pooled text factor [C, %d], got %s" % (who, E, tuple(txt.shape)))
+    else:
+        raise ValueError("%s: sim must be 'max' or 'mean' (got %r)" % (who, sim))
+
+
+def _spatial_max_scores(rows: Tensor, tok: Tensor, lens: Tensor, txt_index: Optional[Tensor], n_way: int,
+                        log_scale: float) -> Tensor:
+    M, HW, E = rows.shape
+    C, L, _ = tok.shape
+    tok = _f32(tok)
+    lens = _i64(lens)
+    out = torch.empty((M,) if n_way > 0 else (M, C), dtype=torch.float32, device=rows.device)
+    _cabi.call("cvcl_spatial_max_scores_f32", _p(rows), _p(tok), _p(lens), _p(txt_index), M, HW, E, C, L, n_way,
+               float(log_scale), _p(out), _stream())
+    return out
+
+
+@torch.library.custom_op(_NS + "::eval_nway_spatial", mutates_args=())
+def eval_nway_spatial(img: Tensor, txt: Tensor, lens: Tensor, txt_index: Optional[Tensor], n_way: int, sim: str,
+                      normalize: bool, log_scale: float, want_logits: bool = True) -> Tuple[Tensor, Tensor]:
+    """n-way trials of a spatial-embedding model, fp32 end to end (eval.py:196-214 / multimodal_lit.py:466-511 with
+    multimodal.py:757-787).  img [N*n_way, HW, E] head outputs before normalisation (NHWC rows, target first);
+    txt: sim="max" per-token text features [C, L, E] (lens [C] their lengths), sim="mean" the pooled text factor
+    [C, E] (cvcl_text_encoder_fwd with per_token=1, pool_scale=1/HW); txt_index [N] | None (None: C >= N, trial n
+    uses label n).  -> (pred int32 [N], logits = exp(s) * match fp32 [N, n_way] | empty); first maximum wins."""
+    if img.dim() != 3 or n_way < 1 or img.shape[0] % n_way != 0:
+        raise ValueError("eval_nway_spatial: img %s is not [N*n_way, HW, E] with n_way=%d" % (tuple(img.shape), n_way))
+    M, HW, E = img.shape
+    N = M // n_way
+    _check_spatial_text(txt, lens, sim, E, "eval_nway_spatial")
+    if txt_index is not None:
+        if tuple(txt_index.shape) != (N,):
+            raise ValueError("eval_nway_spatial: txt_index %s does not fit %d trials" % (tuple(txt_index.shape), N))
+        txt_index = txt_index.to(torch.int32).contiguous()
+    elif txt.shape[0] < N:
+        raise ValueError("eval_nway_spatial: %d trials without txt_index need as many labels (got %d)" % (N, txt.shape[0]))
+    _need_cuda(img, txt, lens, txt_index)
+    rows = _location_rows(img, normalize)
+    if sim == "mean":
+        # multimodal.py:765-770 factorises: sum over the locations . pooled text / (HW len) -> K7 on the two factors
+        return _raw(eval_nway)(_raw(spatial_pool_fwd)(rows), txt, txt_index, n_way, False, log_scale, want_logits)
+    logits = _spatial_max_scores(rows, txt, lens, txt_index, n_way, log_scale).view(N, n_way)
+    pred = _row_argmax(logits)
+    return pred, logits if want_logits else logits.new_empty((0, n_way))
+
+
+@eval_nway_spatial.register_fake
+def _(img, txt, lens, txt_index, n_way, sim, normalize, log_scale, want_logits=True):
+    N = img.shape[0] // n_way
+    return (img.new_empty((N,), dtype=torch.int32),
+            img.new_empty((N, n_way) if want_logits else (0, n_way), dtype=torch.float32))
+
+
+@torch.library.custom_op(_NS + "::classify_ncat_spatial", mutates_args=())
+def classify_ncat_spatial(img: Tensor, txt: Tensor, lens: Tensor, sim: str, normalize: bool, log_scale: float,
+                          want_logits: bool = True) -> Tuple[Tensor, Tensor]:
+    """Category classification of frames for a spatial-embedding model (multimodal_saycam_data_module.py:545-606 with
+    multimodal.py:757-787): img [N, HW, E] head outputs before normalisation, txt / lens as for eval_nway_spatial with
+    the C category labels.  -> (pred int32 [N], logits_per_image fp32 [N, C] | empty); first maximum wins."""
+    if img.dim() != 3:
+        raise ValueError("classify_ncat_spatial: img %s is not [N, HW, E]" % (tuple(img.shape),))
+    M, HW, E = img.shape
+    _check_spatial_text(txt, lens, sim, E, "classify_ncat_spatial")
+    _need_cuda(img, txt, lens)
+    rows = _location_rows(img, normalize)
+    if sim == "mean":
+        return classify_ncat(_raw(spatial_pool_fwd)(rows), txt, False, log_scale, want_logits)
+    logits = _spatial_max_scores(rows, txt, lens, None, 0, log_scale)
+    pred = _row_argmax(logits)
+    return pred, logits if want_logits else logits.new_empty((0,))
+
+
+@classify_ncat_spatial.register_fake
+def _(img, txt, lens, sim, normalize, log_scale, want_logits=True):
+    N, C = img.shape[0], txt.shape[0]
+    return (img.new_empty((N,), dtype=torch.int32),
+            img.new_empty((N, C) if want_logits else (0,), dtype=torch.float32))
 
 
 @torch.no_grad()
