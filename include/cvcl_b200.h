@@ -297,6 +297,23 @@ int cvcl_match_infonce_fwd(const float* match, int B, float log_scale, float inv
                            float* lse0, float* lse1, int* argmax0, int* argmax1, float* out5, void* stream);
 int cvcl_match_infonce_bwd(const float* match, int B, float log_scale, float coef, const float* lse0,
                            const float* lse1, float* dmatch, float* dscale, void* stream);
+/* One rank's share of the same loss when the batch is sharded over a process group (multimodal.py:771-822 on the
+ * global batch; rank r owns pairs [r*b, (r+1)*b), N = world*b, diag_off = r*b): the row block match_r [b,N] (local
+ * images x all texts) gives the image->text CE of the local images, the column block match_c [N,b] (all images x
+ * local texts) the text->image CE of the local texts.  out5 = partial sums scaled by inv_rows = 1/N (summed over the
+ * ranks by the caller); lse0 / argmax0 [b] per local image, lse1 / argmax1 [b] per local text; workspace
+ * cvcl_sim_workspace_bytes(b, N, b, N).  b = N, diag_off = 0, match_r = match_c is cvcl_match_infonce_fwd.
+ * Backward: dmatch_r = exp(s) G_r, dmatch_c = exp(s) G_c with the gathered LSEs of all ranks (lse1_all, lse0_all
+ * [N]); *dscale = sum G_r * logits over the row block (the caller sums it over the ranks), written in a fixed
+ * summation order through the workspace (cvcl_match_infonce_block_bwd_workspace_bytes, 256-byte aligned). */
+int cvcl_match_infonce_block_fwd(const float* match_r, const float* match_c, int b, int N, int diag_off,
+                                 float log_scale, float inv_rows, void* workspace, float* lse0, float* lse1,
+                                 int* argmax0, int* argmax1, float* out5, void* stream);
+size_t cvcl_match_infonce_block_bwd_workspace_bytes(int b, int N);
+int cvcl_match_infonce_block_bwd(const float* match_r, const float* match_c, int b, int N, int diag_off,
+                                 float log_scale, float coef, const float* lse0, const float* lse1_all,
+                                 const float* lse0_all, const float* lse1, float* dmatch_r, float* dmatch_c,
+                                 float* dscale, void* workspace, void* stream);
 
 /* ---- all-gather over NVLink peer memory (the exchange step of the sharded loss, SURVEY 8e) ------
  * peer_ptrs: HOST array of `world` device pointers, entry r = rank r's block (symmetric memory, peer

@@ -78,6 +78,9 @@ PROTOTYPES = {
     "cvcl_spatial_max_bwd": (c_int, [_P, _P, _P, _P, _P, _P, _P, _I, _I, _I, _I, _I, _P, _P, _P, _P]),
     "cvcl_match_infonce_fwd": (c_int, [_P, _I, _F, _F, _P, _P, _P, _P, _P, _P, _P]),
     "cvcl_match_infonce_bwd": (c_int, [_P, _I, _F, _F, _P, _P, _P, _P, _P]),
+    "cvcl_match_infonce_block_fwd": (c_int, [_P, _P, _I, _I, _I, _F, _F, _P, _P, _P, _P, _P, _P, _P]),
+    "cvcl_match_infonce_block_bwd_workspace_bytes": (c_size_t, [_I, _I]),
+    "cvcl_match_infonce_block_bwd": (c_int, [_P, _P, _I, _I, _I, _F, _F, _P, _P, _P, _P, _P, _P, _P, _P, _P]),
     "cvcl_p2p_gather": (c_int, [_P, _I, _I, ctypes.c_longlong, _P, ctypes.c_longlong, _P]),
     "cvcl_peer_flag_words": (c_size_t, []),
     "cvcl_peer_max_blocks": (c_int, []),

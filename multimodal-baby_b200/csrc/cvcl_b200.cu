@@ -1227,31 +1227,78 @@ int cvcl_spatial_max_bwd(const float* gmatch, const int64_t* lens, const int64_t
     return CVCL_OK;
 }
 
-int cvcl_match_infonce_fwd(const float* match, int B, float log_scale, float inv_rows, void* workspace,
-                           float* lse0, float* lse1, int* argmax0, int* argmax1, float* out5, void* stream) {
-    CVCL_REQUIRE(match && workspace && lse0 && lse1 && out5, "match_infonce_fwd: null pointer");
-    CVCL_REQUIRE(B > 0, "match_infonce_fwd: bad shape");
-    SimWs w = carve_sim_ws(workspace, B, B, B, B);
-    CVCL_CHECK_CUDA(launch_pdl(match_stats_kernel, dim3(warps_grid(2ll * B)), dim3(256), 0, as_stream(stream), match, B, B, expf(log_scale), w.part[0], w.part[1], w.diag[0], w.diag[1], w.ticket));
+int cvcl_match_infonce_block_fwd(const float* match_r, const float* match_c, int b, int N, int diag_off,
+                                 float log_scale, float inv_rows, void* workspace, float* lse0, float* lse1,
+                                 int* argmax0, int* argmax1, float* out5, void* stream) {
+    CVCL_REQUIRE(match_r && match_c && workspace && lse0 && lse1 && out5, "match_infonce_fwd: null pointer");
+    CVCL_REQUIRE(b > 0 && N > 0, "match_infonce_fwd: bad shape");
+    CVCL_REQUIRE(diag_off >= 0 && b + diag_off <= N, "match_infonce_fwd: positives out of range (b=%d N=%d diag_off=%d)",
+                 b, N, diag_off);
+    SimWs w = carve_sim_ws(workspace, b, N, b, N);
+    CVCL_CHECK_CUDA(launch_pdl(match_stats_kernel, dim3(warps_grid(2ll * b)), dim3(256), 0, as_stream(stream), match_r, match_c, b, N, diag_off, expf(log_scale), w.part[0], w.part[1], w.diag[0], w.diag[1], w.ticket));
     count_launch();
     FinalizeParams fp{};
     for (int z = 0; z < 2; ++z) {
         fp.part[z] = w.part[z]; fp.m_pad[z] = w.m_pad[z]; fp.n_tiles[z] = 1; fp.diag[z] = w.diag[z];
-        fp.diag_off[z] = 0; fp.M[z] = B;
+        fp.diag_off[z] = diag_off; fp.M[z] = b;
     }
     fp.lse[0] = lse0; fp.lse[1] = lse1; fp.argmax[0] = argmax0; fp.argmax[1] = argmax1;
     fp.inv_rows = inv_rows; fp.block_part = w.block_part; fp.ticket = w.ticket; fp.out = out5;
-    CVCL_CHECK_CUDA(launch_pdl(infonce_finalize_kernel, dim3(ceil_div(2 * B, 256)), dim3(256), 0, as_stream(stream), fp));
+    CVCL_CHECK_CUDA(launch_pdl(infonce_finalize_kernel, dim3(ceil_div(2 * b, 256)), dim3(256), 0, as_stream(stream), fp));
     count_launch();
     return CVCL_OK;
+}
+
+int cvcl_match_infonce_fwd(const float* match, int B, float log_scale, float inv_rows, void* workspace,
+                           float* lse0, float* lse1, int* argmax0, int* argmax1, float* out5, void* stream) {
+    return cvcl_match_infonce_block_fwd(match, match, B, B, 0, log_scale, inv_rows, workspace, lse0, lse1, argmax0,
+                                        argmax1, out5, stream);
+}
+
+namespace {
+int match_grad_blocks(int b, int N) { return static_cast<int>((static_cast<long long>(b) * N + 255) / 256); }
+
+int match_grad_launch(const float* match_r, const float* match_c, int b, int N, int diag_off, float log_scale,
+                      float coef, const float* lse0, const float* lse1_all, const float* lse0_all, const float* lse1,
+                      float* dmatch_r, float* dmatch_c, float* dscale, void* workspace, void* stream) {
+    const int nb = match_grad_blocks(b, N);
+    unsigned int* ticket = nullptr;
+    float* ds_part = nullptr;
+    if (workspace) {
+        ticket = static_cast<unsigned int*>(workspace);
+        ds_part = reinterpret_cast<float*>(static_cast<unsigned char*>(workspace) + 256);
+        CVCL_CHECK_CUDA(cudaMemsetAsync(ticket, 0, sizeof(unsigned int), as_stream(stream)));
+    }
+    CVCL_CHECK_CUDA(launch_pdl(match_grad_kernel, dim3(nb, dmatch_c ? 2 : 1), dim3(256), 0, as_stream(stream),
+                               match_r, match_c, b, N, diag_off, expf(log_scale), coef, lse0, lse1_all, lse0_all, lse1,
+                               dmatch_r, dmatch_c, dscale, ds_part, ticket));
+    count_launch();
+    return CVCL_OK;
+}
+}  // namespace
+
+size_t cvcl_match_infonce_block_bwd_workspace_bytes(int b, int N) {
+    return 256 + align_up(sizeof(float) * static_cast<size_t>(match_grad_blocks(b, N)), 256);
+}
+
+int cvcl_match_infonce_block_bwd(const float* match_r, const float* match_c, int b, int N, int diag_off,
+                                 float log_scale, float coef, const float* lse0, const float* lse1_all,
+                                 const float* lse0_all, const float* lse1, float* dmatch_r, float* dmatch_c,
+                                 float* dscale, void* workspace, void* stream) {
+    CVCL_REQUIRE(match_r && match_c && lse0 && lse1_all && lse0_all && lse1 && dmatch_r && dmatch_c && dscale && workspace,
+                 "match_infonce_block_bwd: null pointer");
+    CVCL_REQUIRE(b > 0 && N > 0 && diag_off >= 0 && b + diag_off <= N,
+                 "match_infonce_block_bwd: bad shape (b=%d N=%d diag_off=%d)", b, N, diag_off);
+    CVCL_REQUIRE((reinterpret_cast<uintptr_t>(workspace) & 255) == 0, "match_infonce_block_bwd: workspace must be 256-byte aligned");
+    return match_grad_launch(match_r, match_c, b, N, diag_off, log_scale, coef, lse0, lse1_all, lse0_all, lse1,
+                             dmatch_r, dmatch_c, dscale, workspace, stream);
 }
 
 int cvcl_match_infonce_bwd(const float* match, int B, float log_scale, float coef, const float* lse0,
                            const float* lse1, float* dmatch, float* dscale, void* stream) {
     CVCL_REQUIRE(match && lse0 && lse1 && dmatch, "match_infonce_bwd: null pointer");
-    CVCL_CHECK_CUDA(launch_pdl(match_grad_kernel, dim3(ceil_div(B * B, 256)), dim3(256), 0, as_stream(stream), match, B, B, expf(log_scale), coef, lse0, lse1, dmatch, dscale));
-    count_launch();
-    return CVCL_OK;
+    return match_grad_launch(match, match, B, B, 0, log_scale, coef, lse0, lse1, lse0, lse1, dmatch, nullptr, dscale,
+                             nullptr, stream);
 }
 
 // ------------------------------------------------------------------------------------ peer-memory gather

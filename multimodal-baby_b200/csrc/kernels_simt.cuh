@@ -1548,24 +1548,27 @@ __global__ void __launch_bounds__(256) spatial_max_dimg_kernel(const float* g, c
 }
 
 // --------------------------------------------------------------------------------------
-// InfoNCE statistics from a MATERIALISED similarity matrix match [Bi,Bt] (spatial "max" path:
-// the [B,B] matrix is small next to the B*B*L*HW contraction that produced it).
-// One warp per row (z=0: image rows) or per column (z=1: text rows of match^T); writes the same
-// RowStat partials (n_tiles = 1) that infonce_finalize_kernel merges.
+// InfoNCE statistics from MATERIALISED similarity blocks (spatial "max" path: the match matrix is
+// small next to the B*B*L*HW contraction that produced it).  Row block match_r [b,N] (b image
+// rows against all N texts) and column block match_c [N,b] (all N images against b texts); the
+// positive of local row / column m sits at (m, m + diag_off) / (m + diag_off, m).  One device:
+// match_r == match_c == match [B,B], b = N = B, diag_off = 0.
+// One warp per row (z=0: image rows of match_r) or per column (z=1: text columns of match_c);
+// writes the same RowStat partials (n_tiles = 1) that infonce_finalize_kernel merges.
 // --------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(256) match_stats_kernel(const float* match, int Bi, int Bt, float scale,
-                                                          RowStat* part0, RowStat* part1, float* diag0,
-                                                          float* diag1, unsigned int* ticket) {
+__global__ void __launch_bounds__(256) match_stats_kernel(const float* match_r, const float* match_c, int b, int N,
+                                                          int diag_off, float scale, RowStat* part0, RowStat* part1,
+                                                          float* diag0, float* diag1, unsigned int* ticket) {
     ptx::pdl_launch_dependents(); ptx::pdl_wait();
     if (blockIdx.x == 0 && threadIdx.x == 0) *ticket = 0u;        // finalize's ticket (runs after us)
     const int warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     const int lane = threadIdx.x & 31;
-    if (warp >= Bi + Bt) return;
-    const int z = warp < Bi ? 0 : 1;
-    const int m = z ? warp - Bi : warp;
-    const int n = z ? Bi : Bt;
-    const size_t stride = z ? Bt : 1;
-    const float* base = z ? match + m : match + static_cast<size_t>(m) * Bt;
+    if (warp >= 2 * b) return;
+    const int z = warp < b ? 0 : 1;
+    const int m = z ? warp - b : warp;
+    const int n = N;
+    const size_t stride = z ? b : 1;
+    const float* base = z ? match_c + m : match_r + static_cast<size_t>(m) * N;
     float mx = -INFINITY; int arg = 0x7fffffff;
     for (int j = lane; j < n; j += 32) {
         const float x = base[j * stride] * scale;
@@ -1587,29 +1590,63 @@ __global__ void __launch_bounds__(256) match_stats_kernel(const float* match, in
     if (lane == 0) {
         RowStat rs; rs.m = mx; rs.l = l; rs.a = a; rs.arg = arg;
         (z ? part1 : part0)[m] = rs;
-        if (m < n) (z ? diag1 : diag0)[m] = base[m * stride] * scale;
+        (z ? diag1 : diag0)[m] = base[static_cast<size_t>(m + diag_off) * stride] * scale;
     }
 }
 
-// d loss / d match = scale * G,  G = coef * (exp(x - lse0[i]) + exp(x - lse1[t]) - 2 delta_it),
-// x = scale * match;  *dscale += sum G * x.
-__global__ void __launch_bounds__(256) match_grad_kernel(const float* match, int Bi, int Bt, float scale,
-                                                         float coef, const float* lse0, const float* lse1,
-                                                         float* dmatch, float* dscale) {
+// d loss / d match = scale * G,  x = scale * match, over the row block (blockIdx.y = 0) and the column block
+// (blockIdx.y = 1, skipped when dmatch_c is null):
+//   G_r[i,t] = coef * (exp(x - lse0[i])     + exp(x - lse1_all[t]) - 2 [t = i + diag_off])   match_r [b,N]
+//   G_c[i,t] = coef * (exp(x - lse0_all[i]) + exp(x - lse1[t])     - 2 [i = t + diag_off])   match_c [N,b]
+// d scale = sum G_r * x over the row block only (each pair's logit counted once over the ranks).  With ds_part
+// ([gridDim.x] floats) and ticket (zeroed before the launch) the row-block blocks write their partial sums and the
+// last one to finish adds them in block order, so a replay is bit-identical; without them each warp adds its sum
+// into *dscale atomically.
+__global__ void __launch_bounds__(256) match_grad_kernel(const float* match_r, const float* match_c, int b, int N,
+                                                         int diag_off, float scale, float coef, const float* lse0,
+                                                         const float* lse1_all, const float* lse0_all,
+                                                         const float* lse1, float* dmatch_r, float* dmatch_c,
+                                                         float* dscale, float* ds_part, unsigned int* ticket) {
     ptx::pdl_launch_dependents(); ptx::pdl_wait();
-    const int idx = blockIdx.x * blockDim.x + threadIdx.x;
+    const int z = blockIdx.y;
+    if (z == 1 && !dmatch_c) return;
+    const long long idx = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
+    const int cols = z ? b : N;
     float ds = 0.f;
-    if (idx < Bi * Bt) {
-        const int i = idx / Bt, t = idx % Bt;
-        const float x = match[idx] * scale;
-        float gg = __expf(x - lse0[i]) + __expf(x - lse1[t]);
-        if (i == t) gg -= 2.f;
+    if (idx < static_cast<long long>(b) * N) {
+        const int i = static_cast<int>(idx / cols), t = static_cast<int>(idx % cols);
+        const float x = (z ? match_c : match_r)[idx] * scale;
+        float gg = z ? __expf(x - lse0_all[i]) + __expf(x - lse1[t]) : __expf(x - lse0[i]) + __expf(x - lse1_all[t]);
+        if (z ? i == t + diag_off : t == i + diag_off) gg -= 2.f;
         gg *= coef;
-        dmatch[idx] = gg * scale;
+        (z ? dmatch_c : dmatch_r)[idx] = gg * scale;
         ds = gg * x;
     }
+    if (z == 1) return;
     ds = warp_sum(ds);
-    if ((threadIdx.x & 31) == 0 && dscale) atomicAdd(dscale, ds);
+    if (!ds_part) {
+        if ((threadIdx.x & 31) == 0 && dscale) atomicAdd(dscale, ds);
+        return;
+    }
+    __shared__ float red[8];
+    __shared__ bool is_last;
+    if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = ds;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        float s = 0.f;
+        for (int k = 0; k < (blockDim.x >> 5); ++k) s += red[k];
+        ds_part[blockIdx.x] = s;
+        __threadfence();
+        is_last = atomicAdd(ticket, 1u) == gridDim.x - 1;
+    }
+    __syncthreads();
+    if (is_last && threadIdx.x < 32) {          // fixed lane-strided order + tree
+        __threadfence();
+        float s = 0.f;
+        for (unsigned int k = threadIdx.x; k < gridDim.x; k += 32) s += ds_part[k];
+        s = warp_sum(s);
+        if (threadIdx.x == 0) { *dscale = s; *ticket = 0u; }
+    }
 }
 
 

@@ -365,18 +365,22 @@ class MultiModalModel(nn.Module):
                     img_f, txt_f = ops.spatial_mean_factors(nhwc, y, y_len, table, self.normalize_features)
                 else:
                     img_f = txt_f = None
-            if img_f is None and self.process_group is not None:
-                raise NotImplementedError("spatial embeddings with sim='max' are not sharded over a process group "
-                                          "(the loss would silently be the local-batch loss)")
             if img_f is not None:
                 # flat features are unit vectors when normalize_features is on (one similarity pass at large batch);
                 # the pooled spatial factors are not
                 unit = self.embedding_type == "flat" and bool(self.normalize_features)
                 loss, iacc, tacc, ient, tent, _, _ = ops.sim_infonce(img_f, txt_f, s, self.process_group, unit)
-            else:
+            elif self.process_group is None:
                 tok, _ = ops.text_features_spatial(y, y_len, table, self.normalize_features)
                 match = ops.spatial_max_similarity(nhwc, tok, y_len, y, split=self._split())
                 loss, iacc, tacc, ient, tent, lpi, lpt = ops.infonce_from_match(match, s)
+            else:
+                # global-batch loss; the logits are this rank's [b,b] block, as on the sharded mean path
+                tok, _ = ops.text_features_spatial(y, y_len, table, self.normalize_features)
+                loss, iacc, tacc, ient, tent, _, _, mloc = ops.spatial_max_infonce(
+                    nhwc, tok, y_len, y, s, self.process_group, split=self._split(), local_match=True)
+                lpi = mloc * math.exp(ops._scalar(s))
+                lpt = lpi.t()
         logits_per_image = logits_per_text = None
         if self.materialize_logits and img_f is not None and img_f.numel() == 0:
             raise RuntimeError("materialize_logits=True needs materialize_features=True on the fused path")

@@ -10,6 +10,7 @@ Reference call sites replaced (paths relative to the reference repo):
   head_features     multimodal/multimodal.py:181-192 (applied at :101), 736
   sim_logits        multimodal/multimodal.py:755, 783-794
   sim_infonce       multimodal/multimodal.py:755, 783-787, 801-818 (+ autograd)
+  spatial_max_infonce     multimodal/multimodal.py:771-822 with the batch sharded over a process group
   flat_contrastive_step   multimodal/multimodal.py:796-822 + loss.backward()
   eval_nway         multimodal/multimodal_lit.py:466-511, eval.py:196-214
   conv1x1_f32, eval_nway_spatial, classify_ncat_spatial
@@ -1470,6 +1471,155 @@ def infonce_from_match(match, s):
     with torch.no_grad():
         lpi = match * math.exp(_scalar(s))
     return loss, iacc, tacc, ient, tent, lpi, lpi.t()
+
+
+# ----------------------------------------------------------------------------------------
+# the same loss sharded over a process group: one rank's row block [b,N] and column block [N,b]
+# ----------------------------------------------------------------------------------------
+def _check_blocks(match_r: Tensor, match_c: Tensor, diag_off: int):
+    b, N = match_r.shape
+    if tuple(match_c.shape) != (N, b) or not 0 <= diag_off <= N - b:
+        raise ValueError("match blocks [b,N] / [N,b] with 0 <= diag_off <= N-b expected, got %s, %s, diag_off=%d"
+                         % (tuple(match_r.shape), tuple(match_c.shape), diag_off))
+    return b, N
+
+
+@torch.library.custom_op(_NS + "::match_infonce_block_fwd", mutates_args=())
+def match_infonce_block_fwd(match_r: Tensor, match_c: Tensor, diag_off: int, log_scale: float, inv_rows: float
+                            ) -> Tuple[Tensor, Tensor, Tensor, Tensor, Tensor]:
+    """row block [b,N] + column block [N,b] -> (out5 [8] partial sums scaled by inv_rows, lse0 [b], lse1 [b],
+    argmax0 [b], argmax1 [b]); positives at (m, m + diag_off) and (m + diag_off, m)."""
+    _need_cuda(match_r, match_c)
+    match_r = _f32(match_r); match_c = _f32(match_c)
+    b, N = _check_blocks(match_r, match_c, diag_off)
+    dev = match_r.device
+    ws = torch.empty((_cabi.load().cvcl_sim_workspace_bytes(b, N, b, N),), dtype=torch.uint8, device=dev)
+    out5 = torch.zeros((8,), dtype=torch.float32, device=dev)
+    lse0 = torch.empty((b,), dtype=torch.float32, device=dev); lse1 = torch.empty_like(lse0)
+    a0 = torch.empty((b,), dtype=torch.int32, device=dev); a1 = torch.empty_like(a0)
+    _cabi.call("cvcl_match_infonce_block_fwd", _p(match_r), _p(match_c), b, N, int(diag_off), float(log_scale),
+               float(inv_rows), _p(ws), _p(lse0), _p(lse1), _p(a0), _p(a1), _p(out5), _stream())
+    return out5, lse0, lse1, a0, a1
+
+
+@match_infonce_block_fwd.register_fake
+def _(match_r, match_c, diag_off, log_scale, inv_rows):
+    b = match_r.shape[0]
+    f = dict(dtype=torch.float32)
+    return (match_r.new_empty((8,), **f), match_r.new_empty((b,), **f), match_r.new_empty((b,), **f),
+            match_r.new_empty((b,), dtype=torch.int32), match_r.new_empty((b,), dtype=torch.int32))
+
+
+@torch.library.custom_op(_NS + "::match_infonce_block_bwd", mutates_args=())
+def match_infonce_block_bwd(match_r: Tensor, match_c: Tensor, diag_off: int, log_scale: float, coef: float,
+                            lse0: Tensor, lse1_all: Tensor, lse0_all: Tensor, lse1: Tensor
+                            ) -> Tuple[Tensor, Tensor, Tensor]:
+    """-> (dmatch_r [b,N], dmatch_c [N,b], dscale [1] of the row block, in a fixed summation order)."""
+    _need_cuda(match_r, match_c, lse0, lse1_all, lse0_all, lse1)
+    match_r = _f32(match_r); match_c = _f32(match_c)
+    b, N = _check_blocks(match_r, match_c, diag_off)
+    dev = match_r.device
+    ws = torch.empty((_cabi.load().cvcl_match_infonce_block_bwd_workspace_bytes(b, N),), dtype=torch.uint8, device=dev)
+    dr = torch.empty_like(match_r); dc = torch.empty_like(match_c)
+    ds = torch.empty((1,), dtype=torch.float32, device=dev)
+    _cabi.call("cvcl_match_infonce_block_bwd", _p(match_r), _p(match_c), b, N, int(diag_off), float(log_scale),
+               float(coef), _p(_f32(lse0)), _p(_f32(lse1_all)), _p(_f32(lse0_all)), _p(_f32(lse1)), _p(dr), _p(dc),
+               _p(ds), _p(ws), _stream())
+    return dr, dc, ds
+
+
+@match_infonce_block_bwd.register_fake
+def _(match_r, match_c, diag_off, log_scale, coef, lse0, lse1_all, lse0_all, lse1):
+    f = dict(dtype=torch.float32)
+    return match_r.new_empty(match_r.shape, **f), match_c.new_empty(match_c.shape, **f), match_r.new_empty((1,), **f)
+
+
+def _spatial_max_block_fwd(split):
+    """The CUDA arithmetic of sharding.spatial_max_infonce_forward: both blocks through spatial_max_fwd, then the block
+    InfoNCE statistics.  The gathered features are fp32 (split: the two-term operands and the bf16 backward operands
+    are built here, exactly as the one-device _SpatialMax builds them for the same pairs) or already bf16."""
+    def fwd_operand(x, pattern):
+        n, k, E = x.shape
+        if split:
+            return split_bf16_cat(x.reshape(n * k, E), pattern).view(n, k, 3 * E)
+        return x
+
+    def bf16(x):
+        n, k, E = x.shape
+        return to_bf16_pair(x.reshape(n * k, E), False)[0].view(n, k, E)
+
+    def compute(img_r, tok_r, lens_r, ids_r, img_all, tok_all, lens_all, ids_all, ls, diag_off, inv_rows):
+        fwd = _raw(spatial_max_fwd)
+        match_r, ait_r, ati_r = fwd(fwd_operand(img_r, "hhl"), fwd_operand(tok_all, "hlh"), lens_all)
+        match_c, ait_c, ati_c = fwd(fwd_operand(img_all, "hhl"), fwd_operand(tok_r, "hlh"), lens_r)
+        out5, lse0, lse1, a0, a1 = _raw(match_infonce_block_fwd)(match_r, match_c, diag_off, ls, inv_rows)
+        state = (match_r, match_c, ait_r, ati_r, ait_c, ati_c, bf16(img_r), bf16(tok_r), bf16(img_all), bf16(tok_all),
+                 lens_r, ids_r, lens_all, ids_all, ls)
+        return out5, lse0, lse1, a0, a1, state
+    return compute
+
+
+def _spatial_max_block_bwd(state, diag_off, coef, lse0, lse1_all, lse0_all, lse1):
+    (match_r, match_c, ait_r, ati_r, ait_c, ati_c, i16_r, t16_r, i16_all, t16_all,
+     lens_r, ids_r, lens_all, ids_all, ls) = state
+    g_r, g_c, ds = _raw(match_infonce_block_bwd)(match_r, match_c, diag_off, ls, coef, lse0, lse1_all, lse0_all, lse1)
+    bwd = _raw(spatial_max_bwd)
+    dimg, _ = bwd(g_r, lens_all, ids_all, ait_r, ati_r, i16_r, t16_all, True, False)
+    del g_r
+    _, dtok = bwd(g_c, lens_r, ids_r, ait_c, ati_c, i16_all, t16_r, False, True)
+    return dimg, dtok, ds
+
+
+class _SpatialMaxInfoNCE(torch.autograd.Function):
+    """spatial_max_similarity + infonce_from_match with the batch sharded over a process group (sharding.py): the
+    location and token features are all-gathered, each rank evaluates its row block and column block of the match
+    matrix.  Same outputs and gradient contract as _SimInfoNCE: the five scalars and d s are global on every rank,
+    d img / d tok are for the local pairs.  The eighth output is the rank's own [b,b] block of the match matrix."""
+
+    @staticmethod
+    def forward(ctx, img, tok, lens, ids, s, group, split):
+        from . import sharding
+        split = bool(split) and img.dtype == torch.float32 and tok.dtype == torch.float32
+        if split:
+            gi, gt = img.detach(), tok.detach()
+        else:
+            gi = to_bf16_pair(img.reshape(-1, img.shape[-1]), False)[0].view(img.shape)
+            gt = to_bf16_pair(tok.reshape(-1, tok.shape[-1]), False)[0].view(tok.shape)
+        out5, saved, (a0, a1) = sharding.spatial_max_infonce_forward(gi, gt, lens, ids, _scalar(s), group,
+                                                                     _spatial_max_block_fwd(split))
+        ctx.saved = saved
+        ctx.group = group
+        ctx.meta = (img.dtype, tok.dtype, torch.is_tensor(s))
+        ctx.set_materialize_grads(False)          # only the loss is differentiated: no zero gradients for the metrics
+        state, _, _, rank, b = saved[:5]
+        local = state[0][:, rank * b:(rank + 1) * b].clone()      # match_r restricted to this rank's texts
+        o = out5[:5].unbind(0)
+        ctx.mark_non_differentiable(o[1], o[2], o[3], o[4], a0, a1, local)
+        return o[0], o[1], o[2], o[3], o[4], a0, a1, local
+
+    @staticmethod
+    def backward(ctx, gloss, *unused):
+        from . import sharding
+        if gloss is None:
+            return None, None, None, None, None, None, None
+        idt, tdt, s_is_tensor = ctx.meta
+        dimg, dtok, ds = sharding.spatial_max_infonce_backward(ctx.saved, ctx.group, _spatial_max_block_bwd)
+        dimg = (dimg * gloss).to(idt)
+        dtok = (dtok * gloss).to(tdt)
+        ds_out = (ds[0] * gloss) if (s_is_tensor and ctx.needs_input_grad[4]) else None
+        return dimg, dtok, None, None, ds_out, None, None
+
+
+def spatial_max_infonce(img_nhwc, tok, lens, ids, s, group=None, split=False, local_match=False):
+    """symmetric InfoNCE of the spatial "max" similarity (multimodal.py:771-822) with the batch sharded over `group`:
+    img_nhwc [b,HW,E] and tok [b,L,E] (fp32, or bf16) are this rank's pairs; ranks may hold different L.
+    -> (loss, image_accuracy, text_accuracy, image_entropy, text_entropy, image_pred, text_pred), all global but the
+    two arg-max vectors (this rank's images / texts, indices into the global batch); local_match=True appends the
+    rank's own [b,b] block of the match matrix.  split=True: two-term bf16 operands for the scores (see
+    spatial_max_similarity).  Gradients: d img / d tok for the local pairs, d s global; replicated parameters get
+    local partials to be summed with sharding.allreduce_gradients."""
+    out = _SpatialMaxInfoNCE.apply(img_nhwc, tok, lens, ids, s, group, bool(split))
+    return out if local_match else out[:7]
 
 
 # ----------------------------------------------------------------------------------------

@@ -7,7 +7,8 @@ features.  Each rank then evaluates its ROW block  S[R, :] = e^s I_R T_all^T  (i
 its b images) and its COLUMN block  S[:, R]^T = e^s T_R I_all^T  (text->image CE of its b texts);
 the positives sit at column offset r*b.  Backward: all-gather the 2*B fp32 log-sum-exps, then
   dI_R = e^s G[R, :] T_all,   dT_R = e^s G[:, R]^T I_all,   G = (P_row + P_col - 2 I) / (2B)
-so no reduce-scatter of feature gradients is needed; d s is all-reduced.
+so no reduce-scatter of feature gradients is needed; d s is all-reduced.  The spatial "max" similarity shards the
+same way on its materialised match blocks (`spatial_max_infonce_forward` / `_backward`).
 
 The collectives live here; the arithmetic is injected (`compute_fwd` / `compute_bwd`): the
 product passes the CUDA ops of `ops.py`, the CPU (gloo) tests pass a torch restatement so the
@@ -63,6 +64,61 @@ def infonce_backward(saved, group, compute_bwd):
     if world > 1:
         dist.all_reduce(ds, group=group)
     return dimg, dtxt, ds
+
+
+def spatial_max_infonce_forward(img, tok, lens, ids, log_scale, group, compute_fwd, pad_id=0):
+    """Spatial "max" InfoNCE sharded by pairs (same row / column decomposition as `infonce_forward`).
+
+    img [b, HW, ...] location features, tok [b, L, ...] per-token features, lens [b], ids [b, L] (or None) of this
+    rank's pairs; the feature tensors are gathered as given (fp32 or bf16: the caller chooses).  Ranks may hold
+    different L (the collate pads to each batch's longest utterance): one all-gather of (b, L) finds the longest,
+    and every rank pads its tokens with zero rows and its ids with `pad_id` to that length before the gathers --
+    positions beyond len[t] do not enter match[i, t].  A rank count b that differs between ranks raises the same
+    ValueError on every rank (the gathers need equal blocks).
+
+    compute_fwd(img_r, tok_r, lens_r, ids_r, img_all, tok_all, lens_all, ids_all, log_scale, diag_off, inv_rows)
+      -> (out5, lse0 [b], lse1 [b], argmax0 [b], argmax1 [b], state)
+    evaluates the row block spatial_max(img_r, tok_all) [b, N] and the column block spatial_max(img_all, tok_r)
+    [N, b].  Returns (out5 global, saved-for-backward tuple, local argmax pair)."""
+    world, rank = group_info(group)
+    b, L = tok.shape[0], tok.shape[1]
+    if img.shape[0] != b or lens.shape[0] != b:
+        raise ValueError("spatial max InfoNCE: %d images, %d texts and %d lengths on rank %d"
+                         % (img.shape[0], b, lens.shape[0], rank))
+    sizes = all_gather_rows(torch.tensor([[b, L]], dtype=torch.int64, device=img.device), group, world)
+    bs, Ls = sizes[:, 0].tolist(), sizes[:, 1].tolist()
+    if len(set(bs)) != 1:
+        raise ValueError("sharded spatial max InfoNCE needs the same number of pairs on every rank, got %s" % (bs,))
+    Lm = max(Ls)
+    if Lm > L:
+        tok = torch.cat([tok, tok.new_zeros((b, Lm - L) + tuple(tok.shape[2:]))], dim=1)
+        if ids is not None:
+            ids = torch.cat([ids, ids.new_full((b, Lm - L), pad_id)], dim=1)
+    img_all = all_gather_rows(img, group, world)
+    tok_all = all_gather_rows(tok, group, world)
+    lens_all = all_gather_rows(lens, group, world)
+    ids_all = None if ids is None else all_gather_rows(ids, group, world)
+    Bg = world * b
+    out5, lse0, lse1, a0, a1, state = compute_fwd(img, tok, lens, ids, img_all, tok_all, lens_all, ids_all,
+                                                  log_scale, rank * b, 1.0 / Bg)
+    out5 = out5.clone()
+    if world > 1:
+        dist.all_reduce(out5, group=group)       # partial sums already scaled by 1/B_global
+    saved = (state, lse0, lse1, rank, b, world, L)
+    return out5, saved, (a0, a1)
+
+
+def spatial_max_infonce_backward(saved, group, compute_bwd):
+    """-> (dimg [b, HW, E], dtok [b, L, E] at this rank's own L, dscale [1] summed over the ranks) for upstream
+    gradient 1.  compute_bwd(state, diag_off, coef, lse0, lse1_all, lse0_all, lse1) -> (dimg, dtok, ds of the row
+    block).  Each image's row and each text's column live on its own rank: no reduce-scatter."""
+    state, lse0, lse1, rank, b, world, L = saved
+    lse0_all = all_gather_rows(lse0, group, world)
+    lse1_all = all_gather_rows(lse1, group, world)
+    dimg, dtok, ds = compute_bwd(state, rank * b, 0.5 / (world * b), lse0, lse1_all, lse0_all, lse1)
+    if world > 1:
+        dist.all_reduce(ds, group=group)
+    return dimg, (dtok if dtok.shape[1] == L else dtok[:, :L].contiguous()), ds
 
 
 def allreduce_gradients(params, group=None):
