@@ -1059,13 +1059,17 @@ static int flat_step_fused_impl(const void* x16, const void* w16, const int64_t*
         maps_valid = true;
     }
 
-    static thread_local unsigned attr_mask = 0;     // per device: function attributes live in the device's context
-    int attr_dev = 0;
+    // the instance follows the entry, not the world size: the sharded entry at world 1 still runs the sharded
+    // instance (epoch counter, flag words), so that the two can be compared against each other.  (nvcc lists the
+    // instance named last first in `cuobjdump -sass`, where test_host_logic.py looks for the peer-memory barrier.)
+    void (*kernel)(const fused::StepMaps, const fused::StepParams) =
+        sh == nullptr ? fused::flat_step_kernel<false> : fused::flat_step_kernel<true>;
+    static thread_local unsigned attr_mask[2] = {0, 0};   // per device and instance: function attributes live in the
+    int attr_dev = 0;                                      // device's context
     if (cudaGetDevice(&attr_dev) != cudaSuccess || attr_dev < 0 || attr_dev > 31) attr_dev = 0;
-    if (!((attr_mask >> attr_dev) & 1u)) {
-        CVCL_CHECK_CUDA(cudaFuncSetAttribute(fused::flat_step_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                             fused::kSmemBytes));
-        attr_mask |= 1u << attr_dev;
+    if (!((attr_mask[sh != nullptr] >> attr_dev) & 1u)) {
+        CVCL_CHECK_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, fused::kSmemBytes));
+        attr_mask[sh != nullptr] |= 1u << attr_dev;
     }
     cudaLaunchConfig_t cfg{};
     cfg.gridDim = dim3(f.grid);
@@ -1076,7 +1080,7 @@ static int flat_step_fused_impl(const void* x16, const void* w16, const int64_t*
     at[0].id = cudaLaunchAttributeCooperative;          // all CTAs co-resident: the grid barriers cannot starve
     at[0].val.cooperative = 1;
     cfg.attrs = at; cfg.numAttrs = 1;
-    CVCL_CHECK_CUDA(cudaLaunchKernelEx(&cfg, fused::flat_step_kernel, maps, p));
+    CVCL_CHECK_CUDA(cudaLaunchKernelEx(&cfg, kernel, maps, p));
     count_launch();
     return CVCL_OK;
 }

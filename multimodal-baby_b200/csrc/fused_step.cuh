@@ -192,11 +192,11 @@ __device__ __forceinline__ unsigned int ld_acquire_sys(const unsigned int* p) {
     return v;
 }
 
-// xstage >= 0 (sharded runs): the barrier also spans the ranks.  Every CTA fences its stores at system scope
-// before it arrives; the LAST local arrival (it has seen all the others through the counter) stores this
-// launch's epoch into flag word [xstage][rank] of every peer, and every CTA then also waits until its own
+// xstage >= 0 (sharded runs; only the kSharded instance has this code): the barrier also spans the ranks.  Every
+// CTA fences its stores at system scope before it arrives; the LAST local arrival (it has seen all the others
+// through the counter) stores this launch's epoch into flag word [xstage][rank] of every peer, and every CTA then also waits until its own
 // words [xstage][peer] carry the epoch: all stores a peer issued before ITS barrier have landed here.
-template <bool kWriterFence>
+template <bool kWriterFence, bool kSharded>
 CVCL_HELPER void grid_sync(const StepParams& p, int k, int xstage = -1, unsigned int epoch = 0) {
     if (kWriterFence) fence_proxy_async_all();
     __syncthreads();
@@ -205,7 +205,7 @@ CVCL_HELPER void grid_sync(const StepParams& p, int k, int xstage = -1, unsigned
         // signals and the `world` polls run side by side instead of one release (fence + store) after the other
         // (measured at 8 ranks: ~14 us per barrier for seven serial releases)
         const int lane = threadIdx.x;
-        const bool cross = xstage >= 0 && p.world > 1;
+        const bool cross = kSharded && xstage >= 0 && p.world > 1;
         const unsigned int target = static_cast<unsigned int>(k + 1) * gridDim.x;
         unsigned int prev = 0;
         if (lane == 0) {
@@ -264,6 +264,7 @@ struct Ring {
 
 // one utterance per warp: feat = normalise(sum_l table[ids[b,l]] / len[b]) in position order
 // (same arithmetic, same order as text_encoder_fwd_kernel; E <= 512)
+template <bool kSharded>
 CVCL_HELPER void text_row(const StepParams& p, int b, int lane) {
     const int nch = p.E >> 7;
     constexpr int kInFlight = 12;          // covers half of the utterances (mean length 14) in one round trip
@@ -315,7 +316,7 @@ CVCL_HELPER void text_row(const StepParams& p, int b, int lane) {
             const int e = (c * 32 + lane) * 4;
             const float4 t = make_float4(acc[c].x * inv, acc[c].y * inv, acc[c].z * inv, acc[c].w * inv);
             if (p.txt_f32) *reinterpret_cast<float4*>(p.txt_f32 + static_cast<size_t>(b) * p.E + e) = t;
-            for (int pp = 0; pp < p.world; ++pp)          // texts are the keys of direction 0
+            for (int pp = 0; pp < (kSharded ? p.world : 1); ++pp)      // texts are the keys of direction 0
                 store_bf16x4(p.peer_kf[0][pp] + static_cast<size_t>(p.diag_off + b) * p.ldk + e, t);
         }
     }
@@ -388,6 +389,11 @@ CVCL_HELPER float merge_ml(const float2* base, size_t stride, int n) {
 
 #define CVCL_STAMP(i) do { if (cta == 0 && p.timing) p.timing[i] = globaltimer_ns(); } while (0)
 
+// Two instances: kSharded = true serves the sharded entry (any world size, world 1 included) and keeps every
+// cross-rank path; kSharded = false is the single-GPU step, compiled without them.  The phases run once per launch
+// and the L2 flush between training steps evicts the code too, so every SASS byte of a path that the single-GPU
+// step never takes is still fetched on the way through (the sharded-only code is a quarter of the kernel).
+template <bool kSharded>
 __global__ void __launch_bounds__(kThreads, 1)
 flat_step_kernel(const __grid_constant__ StepMaps maps, const __grid_constant__ StepParams p) {
     extern __shared__ unsigned char smem_raw[];
@@ -442,10 +448,11 @@ flat_step_kernel(const __grid_constant__ StepMaps maps, const __grid_constant__ 
     constexpr float kLog2e = 1.4426950408889634f;
     int sync_k = 0;
     // cross-rank flag value of this launch (sharded runs; every CTA reads it before any CTA can bump it at exit)
-    const unsigned int xepoch = p.epoch ? *reinterpret_cast<volatile unsigned int*>(p.epoch) + 1u : 0u;
+    const bool reduce = kSharded && p.reduce;        // sum the gradients over the ranks in P5 / P6
+    const unsigned int xepoch = (kSharded && p.epoch) ? *reinterpret_cast<volatile unsigned int*>(p.epoch) + 1u : 0u;
 
     if (p.phase_limit == 100) {            // measurement: the cost of the grid barrier alone
-        for (int i = 0; i < 6; ++i) grid_sync<false>(p, sync_k++);
+        for (int i = 0; i < 6; ++i) grid_sync<false, kSharded>(p, sync_k++);
         goto done;
     }
 
@@ -503,7 +510,7 @@ flat_step_kernel(const __grid_constant__ StepMaps maps, const __grid_constant__ 
         // P1 +1.6 us, dropped.)
         if (warp >= 2) {
             const int slot = warp >= 6 ? warp - 6 : warp;
-            for (int u = slot * G + cta; u < p.B; u += 6 * G) text_row(p, u, lane);
+            for (int u = slot * G + cta; u < p.B; u += 6 * G) text_row<kSharded>(p, u, lane);
             if (warp == 2 && lane == 0) CVCL_STAMP(18);
         }
         if (has) {                                          // all eight warps drain the head tile
@@ -526,7 +533,7 @@ flat_step_kernel(const __grid_constant__ StepMaps maps, const __grid_constant__ 
         if (has) ++tfull_uses;
     }
     // (the ring state is only ever used by lane 0 of warps 0 and 1, which walk identical sequences)
-    grid_sync<true>(p, sync_k++);
+    grid_sync<true, kSharded>(p, sync_k++);
     if (p.phase_limit == 1) goto done;
 
     // ============================================================================ P1
@@ -575,7 +582,7 @@ flat_step_kernel(const __grid_constant__ StepMaps maps, const __grid_constant__ 
                     const int e = (c * 32 + lane) * 4;
                     const float4 t = make_float4(acc[c].x * inv, acc[c].y * inv, acc[c].z * inv, acc[c].w * inv);
                     if (p.img_f32) *reinterpret_cast<float4*>(p.img_f32 + static_cast<size_t>(r) * p.E + e) = t;
-                    for (int pp = 0; pp < p.world; ++pp)  // images are the keys of direction 1
+                    for (int pp = 0; pp < (kSharded ? p.world : 1); ++pp)  // images are the keys of direction 1
                         store_bf16x4(p.peer_kf[1][pp] + static_cast<size_t>(p.diag_off + r) * p.ldk + e, t);
                 }
             }
@@ -598,7 +605,7 @@ flat_step_kernel(const __grid_constant__ StepMaps maps, const __grid_constant__ 
         }
         if (threadIdx.x == 0) CVCL_STAMP(19);
     }
-    grid_sync<true>(p, sync_k++, 0, xepoch);               // sharded: every rank's features are in place behind this
+    grid_sync<true, kSharded>(p, sync_k++, 0, xepoch);               // sharded: every rank's features are in place behind this
     if (p.phase_limit == 2) goto done;
 
     {
@@ -704,7 +711,7 @@ flat_step_kernel(const __grid_constant__ StepMaps maps, const __grid_constant__ 
                         RowStat rs; rs.m = mx * scale; rs.l = l; rs.a = a * scale; rs.arg = arg;
                         const int pidx = (pi * p.T + j) * 2 + half;
                         p.part[z][static_cast<size_t>(pidx) * p.Bp + m] = rs;
-                        if (p.world > 1) {              // (max, sum) of this row's partial -> every rank's gathered copy
+                        if (kSharded && p.world > 1) {  // (max, sum) of this row's partial -> every rank's gathered copy
                             const size_t o = static_cast<size_t>(pidx) * p.Bg + p.diag_off + m;
                             for (int pp = 0; pp < p.world; ++pp) p.peer_part[z][pp][o] = make_float2(rs.m, rs.l);
                         }
@@ -715,7 +722,7 @@ flat_step_kernel(const __grid_constant__ StepMaps maps, const __grid_constant__ 
             if (threadIdx.x == 64) CVCL_STAMP(21);
         }
         if (has) ++tfull_uses;
-        grid_sync<false>(p, sync_k++, 1, xepoch);          // sharded: every rank's softmax partials are in place behind this
+        grid_sync<false, kSharded>(p, sync_k++, 1, xepoch);          // sharded: every rank's softmax partials are in place behind this
         if (p.phase_limit == 3) goto done;
 
         // ======================================================================== P3
@@ -770,7 +777,7 @@ flat_step_kernel(const __grid_constant__ StepMaps maps, const __grid_constant__ 
                     float lkv = INFINITY;
                     if (n < N) {
                         float lse_c;
-                        if (p.part_all[1 - z]) lse_c = merge_ml(p.part_all[1 - z] + n, p.Bg, 2 * p.nCB);
+                        if (kSharded && p.part_all[1 - z]) lse_c = merge_ml(p.part_all[1 - z] + n, p.Bg, 2 * p.nCB);
                         else {
                             float cm_, cl_, ca_; int carg_;
                             merge_stats(p.part[1 - z] + n, p.Bp, 2 * p.nCB, cm_, cl_, ca_, carg_);
@@ -900,7 +907,7 @@ flat_step_kernel(const __grid_constant__ StepMaps maps, const __grid_constant__ 
             }
         }
     }
-    grid_sync<false>(p, sync_k++);
+    grid_sync<false, kSharded>(p, sync_k++);
     if (p.phase_limit == 4) goto done;
 
     if (p.need_grads) {
@@ -992,7 +999,7 @@ flat_step_kernel(const __grid_constant__ StepMaps maps, const __grid_constant__ 
         }
         if (threadIdx.x == 0) CVCL_STAMP(26);
     }
-    if (p.need_grads) grid_sync<true>(p, sync_k++);
+    if (p.need_grads) grid_sync<true, kSharded>(p, sync_k++);
     if (p.phase_limit == 5) goto done;
 
     if (p.need_grads) {
@@ -1054,7 +1061,7 @@ flat_step_kernel(const __grid_constant__ StepMaps maps, const __grid_constant__ 
                 ptx::fence_proxy_async_smem();
                 ptx::tc_fence_before();
                 __syncthreads();
-                if (p.reduce) {
+                if (reduce) {
                     // partial tile -> scratch of the rank that owns tile t: every warp copies 16 rows out of the staging
                     // boxes with 512-byte row stores (posted stores over NVLink; measured faster than a TMA store to peer
                     // memory, which drained at ~270 GB/s)
@@ -1144,7 +1151,7 @@ flat_step_kernel(const __grid_constant__ StepMaps maps, const __grid_constant__ 
         }
         __syncthreads();
         const int n_fin = p.need_grads ? 12 + p.E : 8;
-        if (p.reduce) {                                  // this rank's partials -> slot `rank` of every rank's block
+        if (reduce) {                                    // this rank's partials -> slot `rank` of every rank's block
             for (int i = threadIdx.x; i < n_fin; i += kThreads) {
                 const float v = fin[i];
                 for (int pp = 0; pp < p.world; ++pp) p.peer_small[pp][p.rank * kSmall + i] = v;
@@ -1159,9 +1166,9 @@ flat_step_kernel(const __grid_constant__ StepMaps maps, const __grid_constant__ 
         }
     }
 
-    if (p.reduce) {
+    if (reduce) {
         // ======================================================================== P6 (sharded)
-        grid_sync<false>(p, sync_k++, 2, xepoch);          // every rank's partial tiles and scalars have landed here
+        grid_sync<false, kSharded>(p, sync_k++, 2, xepoch);          // every rank's partial tiles and scalars have landed here
         // (a) scalars + d bias: one-shot, summed locally in rank order (CTA 0)
         if (cta == 0) {
             const int n_fin = p.need_grads ? 12 + p.E : 8;
@@ -1222,7 +1229,7 @@ flat_step_kernel(const __grid_constant__ StepMaps maps, const __grid_constant__ 
                 }
             }
         }
-        grid_sync<false>(p, sync_k++, 3, xepoch);          // every rank's block holds the global sums behind this
+        grid_sync<false, kSharded>(p, sync_k++, 3, xepoch);          // every rank's block holds the global sums behind this
     }
 
 done:
@@ -1234,7 +1241,7 @@ done:
         __threadfence();
         if (atomicAdd(p.sync + 1, 1u) == static_cast<unsigned int>(G - 1)) {
             p.sync[0] = 0u; p.sync[1] = 0u; p.sync[2] = 0u;
-            if (p.epoch) *p.epoch = xepoch;
+            if (kSharded && p.epoch) *p.epoch = xepoch;
             __threadfence();
         }
     }
