@@ -217,7 +217,7 @@ int cvcl_flat_contrastive_step(const void* x, int x_is_bf16, const int64_t* ids,
  * cvcl_adamw_step's bf16_shadow output, or cast once after loading); bias/table fp32 masters.
  * log_scale_dev (nullable) is a DEVICE scalar s = -log(temperature): when given it is read by the kernel
  * (trainable temperature without a host sync, multimodal.py:711-715) and log_scale is ignored.
- * Shapes covered: E in {128,256,384,512}, K % 64 == 0, B <= 1024 (cvcl_flat_fused_supported); anything
+ * Shapes covered: E in {128,256,384,512}, K % 64 == 0, B <= 1024, L <= 256 (cvcl_flat_fused_supported); anything
  * else returns CVCL_ERR_UNSUPPORTED (callers then use cvcl_flat_contrastive_step).
  * workspace: cvcl_flat_fused_workspace_bytes bytes, 256-byte aligned, its first 1024 bytes zeroed ONCE before
  * the first call (the kernel leaves them reusable); one step in flight per workspace.
@@ -229,7 +229,7 @@ int cvcl_flat_fused_supported(int B, int L, int E, int K, int V);
 size_t cvcl_flat_fused_workspace_bytes(int B, int L, int E, int K, int V);
 /* byte offsets of the workspace blocks (tests / tools): out[0..13] = ctrl, hpart, img16, txt16, invn, part, diag,
  * lse, rb_part, dspart, dqpart, du16, dbpart, total; out[14..19] = Bp, KS, nPart, dw_bn, grid, nCB;
- * out[20..23] = dm16, cmat, QS, Vp.  ctrl + 128 holds 48 globaltimer stamps (ns) of CTA 0: [0] start,
+ * out[20..24] = dm16, cmat, QS, Vp, gdiag.  ctrl + 128 holds 48 globaltimer stamps (ns) of CTA 0: [0] start,
  * [k] after grid barrier k, [15] end, [16..28] inside the phases (csrc/fused_step.cuh: CVCL_STAMP). */
 int cvcl_flat_fused_layout(int B, int L, int E, int K, int V, long long* out, int n);
 int cvcl_flat_step_fused(const void* x16, const void* w16, const int64_t* ids, const int64_t* lens,

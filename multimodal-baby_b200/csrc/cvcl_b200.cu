@@ -820,12 +820,15 @@ namespace {
 struct FusedPlan {
     int Bp, nMB, nEB, nCB, KS, kc_per_split, num_kc, T, nPart, QS, Vp, dw_bn, grid;
     size_t off_ctrl, off_hpart, off_img16, off_txt16, off_invn, off_part, off_diag, off_lse, off_rbpart, off_dspart,
-           off_dqpart, off_du16, off_dbpart, off_dm16, off_cmat, bytes;
+           off_dqpart, off_du16, off_dbpart, off_dm16, off_cmat, off_gdiag, bytes;
 };
 // -> 0 when the persistent kernel covers the shape, else the reason (unsupported, not an error)
-const char* plan_fused(FusedPlan* f, int B, int E, int K, int V, int world = 1) {
+const char* plan_fused(FusedPlan* f, int B, int L, int E, int K, int V, int world = 1) {
     const int G = sm_count();
     if (B < 1) return "B < 1";
+    if (L < 1) return "L < 1";
+    // the token-count matrix of P1/P5 is bf16, which holds integers exactly only up to 256
+    if (L > 256) return "L > 256: a token count above 256 is not exact in the bf16 count matrix";
     if (E % 128 != 0 || E < 128 || E > 512) return "E must be 128, 256, 384 or 512";
     if (K % 64 != 0 || K < 64) return "K must be a multiple of 64";
     if (V < 1) return "V < 1";
@@ -876,6 +879,7 @@ const char* plan_fused(FusedPlan* f, int B, int E, int K, int V, int world = 1) 
     f->off_dbpart = take(4ull * G * E);
     f->off_dm16 = take(2ull * Bp * E);
     f->off_cmat = take(2ull * Bp * f->Vp);
+    f->off_gdiag = take(4ull * 2 * Bp);
     f->bytes = off;
     return nullptr;
 }
@@ -895,27 +899,24 @@ struct FusedShard {
 }  // namespace
 
 int cvcl_flat_fused_supported(int B, int L, int E, int K, int V) {
-    (void)L;
     FusedPlan f{};
-    return plan_fused(&f, B, E, K, V) == nullptr ? 1 : 0;
+    return plan_fused(&f, B, L, E, K, V) == nullptr ? 1 : 0;
 }
 
 size_t cvcl_flat_fused_workspace_bytes(int B, int L, int E, int K, int V) {
-    (void)L;
     FusedPlan f{};
-    return plan_fused(&f, B, E, K, V) == nullptr ? f.bytes : 0;
+    return plan_fused(&f, B, L, E, K, V) == nullptr ? f.bytes : 0;
 }
 
 int cvcl_flat_fused_layout(int B, int L, int E, int K, int V, long long* out, int n) {
-    (void)L;
     FusedPlan f{};
-    const char* why = plan_fused(&f, B, E, K, V);
+    const char* why = plan_fused(&f, B, L, E, K, V);
     if (why) return fail(CVCL_ERR_UNSUPPORTED, "flat_fused_layout: %s", why);
     const long long v[] = {(long long)f.off_ctrl, (long long)f.off_hpart, (long long)f.off_img16, (long long)f.off_txt16,
                            (long long)f.off_invn, (long long)f.off_part, (long long)f.off_diag, (long long)f.off_lse,
                            (long long)f.off_rbpart, (long long)f.off_dspart, (long long)f.off_dqpart, (long long)f.off_du16,
                            (long long)f.off_dbpart, (long long)f.bytes, f.Bp, f.KS, f.nPart, f.dw_bn, f.grid, f.nCB,
-                           (long long)f.off_dm16, (long long)f.off_cmat, f.QS, f.Vp};
+                           (long long)f.off_dm16, (long long)f.off_cmat, f.QS, f.Vp, (long long)f.off_gdiag};
     for (int i = 0; i < n && i < (int)(sizeof(v) / sizeof(v[0])); ++i) out[i] = v[i];
     return CVCL_OK;
 }
@@ -932,8 +933,8 @@ static int flat_step_fused_impl(const void* x16, const void* w16, const int64_t*
     const int world = sh ? sh->world : 1, rank = sh ? sh->rank : 0;
     CVCL_REQUIRE(rank >= 0 && rank < world, "flat_step_fused: rank %d outside [0,%d)", rank, world);
     FusedPlan f{};
-    if (const char* why = plan_fused(&f, B, E, K, V, world))
-        return fail(CVCL_ERR_UNSUPPORTED, "flat_step_fused: %s (B=%d E=%d K=%d world=%d)", why, B, E, K, world);
+    if (const char* why = plan_fused(&f, B, L, E, K, V, world))
+        return fail(CVCL_ERR_UNSUPPORTED, "flat_step_fused: %s (B=%d L=%d E=%d K=%d world=%d)", why, B, L, E, K, world);
     CVCL_REQUIRE(((reinterpret_cast<uintptr_t>(workspace) | reinterpret_cast<uintptr_t>(table) |
                    reinterpret_cast<uintptr_t>(bias)) & 15) == 0, "flat_step_fused: 16-byte alignment required");
     CVCL_REQUIRE(!need_grads || ((reinterpret_cast<uintptr_t>(dtable) | reinterpret_cast<uintptr_t>(dW)) & 15) == 0,
@@ -1004,6 +1005,7 @@ static int flat_step_fused_impl(const void* x16, const void* w16, const int64_t*
         p.part[z] = reinterpret_cast<RowStat*>(ws + f.off_part) + static_cast<size_t>(z) * 2 * f.nCB * f.Bp;
         p.diag[z] = reinterpret_cast<float*>(ws + f.off_diag) + z * f.Bp;
         p.lse[z] = reinterpret_cast<float*>(ws + f.off_lse) + z * f.Bp;
+        p.gdiag[z] = reinterpret_cast<float*>(ws + f.off_gdiag) + z * f.Bp;
         p.part_all[z] = (sh && world > 1) ? p.peer_part[z][rank] : nullptr;
     }
     p.rb_part = reinterpret_cast<float*>(ws + f.off_rbpart);
@@ -1097,21 +1099,18 @@ int cvcl_flat_step_fused(const void* x16, const void* w16, const int64_t* ids, c
 }
 
 int cvcl_flat_fused_sharded_supported(int B, int L, int E, int K, int V, int world) {
-    (void)L;
     FusedPlan f{};
-    return plan_fused(&f, B, E, K, V, world) == nullptr ? 1 : 0;
+    return plan_fused(&f, B, L, E, K, V, world) == nullptr ? 1 : 0;
 }
 
 size_t cvcl_flat_fused_sharded_workspace_bytes(int B, int L, int E, int K, int V, int world) {
-    (void)L;
     FusedPlan f{};
-    return plan_fused(&f, B, E, K, V, world) == nullptr ? f.bytes : 0;
+    return plan_fused(&f, B, L, E, K, V, world) == nullptr ? f.bytes : 0;
 }
 
 size_t cvcl_flat_fused_sharded_scratch_bytes(int B, int L, int E, int K, int V, int world) {
-    (void)L;
     FusedPlan f{};
-    if (plan_fused(&f, B, E, K, V, world) != nullptr || world < 2) return 0;
+    if (plan_fused(&f, B, L, E, K, V, world) != nullptr || world < 2) return 0;
     const int n_tiles5 = f.nEB * (K / 128) + ceil_div(V, 128) * f.nEB;
     const size_t nslot = ceil_div(n_tiles5, world);
     return align_up(static_cast<size_t>(world) * nslot * 128 * 128 * 4 + static_cast<size_t>(world) * fused::kSmall * 4, 256);

@@ -23,7 +23,7 @@
 //       recompute GEMM), written as the bf16 A operand straight into swizzled shared memory, then
 //       dQ_partial = Gs_tile . K_block (tcgen05) -> slab by TMA store.  P2/P3 run on QS CTAs per tile, each
 //       owning E/QS output columns of dQ (the tile GEMM is repeated: latency, not flops, is the limit here)
-//   P4  slab sum + the -2I term in fp32 + F.normalize backward; image rows -> bf16 du (operand of dW) and
+//   P4  slab sum + the diagonal of G in fp32 + F.normalize backward; image rows -> bf16 du (operand of dW) and
 //       per-CTA bias partials; text rows -> /len -> bf16 dm (operand of the embedding gradient)
 //   P5  dW = du^T x  and  d table = C^T dm  (the embedding-bag backward as a GEMM against the token counts:
 //       nn.Embedding(padding_idx=0) semantics fall out of C[:,0] = 0), both operands MN-major, read in place,
@@ -107,6 +107,7 @@ struct StepParams {
     RowStat* part[2];                    // [nCB][Bp]
     float* diag[2];                      // [Bp] logit at the positive
     float* lse[2];                       // [Bp] (local rows)
+    float* gdiag[2];                     // [Bp] bf16(Gs_ii) as P3 put it into the dQ operand (local rows)
     // sharded only (null on one GPU): the (max, sum) softmax partials of EVERY row of direction z, gathered:
     // part_all[z][partial 0..2*nCB)[global row 0..Bg) -- P2 stores its partials into every rank's copy, so the column
     // LSEs of P3 (rows that other ranks own, SURVEY 8e) need no exchange phase of their own
@@ -834,6 +835,16 @@ flat_step_kernel(const __grid_constant__ StepMaps maps, const __grid_constant__ 
                                 g[4 * q4 + q] = gg;
                             }
                         }
+                        // the diagonal stays in the bf16 operand; its rounded value goes to P4, which replaces it by the
+                        // whole G_ii in fp32: w (P_row + P_col) and -2w nearly cancel when a pair is confident, and the
+                        // bf16 rounding of the first would be left as the whole gradient (warp-uniform: one chunk of the
+                        // diagonal tile per warp)
+                        if (dcol >= n && dcol < n + 32 && qs == 0 && m < M) {
+                            float gd = 0.f;
+#pragma unroll
+                            for (int q = 0; q < 32; ++q) if (n + q == dcol) gd = g[q];
+                            p.gdiag[z][m] = __bfloat162float(__float2bfloat16_rn(gd));
+                        }
                         ds = fmaf(-2.f * w, dv, ds);
 #pragma unroll
                         for (int q = 0; q < 4; ++q) swz_st16(gs_tile, row, (c + 8 * q) * 2, pack_bf16x8(g + 8 * q));
@@ -916,7 +927,7 @@ flat_step_kernel(const __grid_constant__ StepMaps maps, const __grid_constant__ 
         // task B + r: image row r (direction 0) -> bf16 du (operand of dW) + bias partials
         const int nch = p.E >> 7;
         const size_t slab = static_cast<size_t>(p.Bp) * p.E;
-        const float dcoef = -2.f * scale * (0.5f * p.inv_rows);
+        const float wg = scale * (0.5f * p.inv_rows);
         float4 dbacc[4];
 #pragma unroll
         for (int c = 0; c < 4; ++c) dbacc[c] = make_float4(0.f, 0.f, 0.f, 0.f);
@@ -927,7 +938,7 @@ flat_step_kernel(const __grid_constant__ StepMaps maps, const __grid_constant__ 
 #pragma unroll
             for (int c = 0; c < 4; ++c) acc[c] = make_float4(0.f, 0.f, 0.f, 0.f);
             const float* base = p.dqpart + (static_cast<size_t>(z) * p.nPart * p.Bp + r) * p.E;
-            // the positives of the other modality (the -2*I term of G, in fp32) and this row's own features
+            // the positives of the other modality (the diagonal of G, in fp32) and this row's own features
             const __nv_bfloat16* posrow = p.kf16[z] + static_cast<size_t>(p.diag_off + r) * p.ldk;
             const __nv_bfloat16* qrow = p.q16[z] + static_cast<size_t>(r) * p.ldq;
             uint2 pr[4], qr[4];
@@ -941,6 +952,11 @@ flat_step_kernel(const __grid_constant__ StepMaps maps, const __grid_constant__ 
             }
             const float inv = p.normalize ? __ldcg(p.invn[z] + r) : 1.f;
             const float rs = z ? 1.f / static_cast<float>(__ldg(p.lens + r)) : 1.f;
+            // the diagonal of G in fp32: the slabs hold bf16(Gs_ii) K_i, replaced here by G_ii K_i with
+            // G_ii = w (P_row,ii - 1 + P_col,ii - 1) (at one pair, exactly 0)
+            const float dg = __ldcg(p.diag[z] + r);
+            const float dcoef = wg * (expm1f(dg - __ldcg(p.lse[z] + r)) + expm1f(dg - __ldcg(p.lse[1 - z] + r)))
+                                - __ldcg(p.gdiag[z] + r);
             for (int k0 = 0; k0 < p.nPart; k0 += 4) {
                 float4 v[4][4];
 #pragma unroll

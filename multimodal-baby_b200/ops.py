@@ -747,10 +747,11 @@ def fused_supported(B, L, E, K, V) -> bool:
 def fused_layout(B, L, E, K, V):
     """workspace block offsets of the one-kernel step (see cvcl_flat_fused_layout)."""
     import ctypes
-    arr = (ctypes.c_longlong * 24)()
-    _cabi.call("cvcl_flat_fused_layout", B, L, E, K, V, arr, 24)
+    arr = (ctypes.c_longlong * 25)()
+    _cabi.call("cvcl_flat_fused_layout", B, L, E, K, V, arr, 25)
     names = ["ctrl", "hpart", "img16", "txt16", "invn", "part", "diag", "lse", "rb_part", "dspart", "dqpart",
-             "du16", "dbpart", "bytes", "Bp", "KS", "nPart", "dw_bn", "grid", "nCB", "dm16", "cmat", "QS", "Vp"]
+             "du16", "dbpart", "bytes", "Bp", "KS", "nPart", "dw_bn", "grid", "nCB", "dm16", "cmat", "QS", "Vp",
+             "gdiag"]
     return dict(zip(names, [int(v) for v in arr]))
 
 
