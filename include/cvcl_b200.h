@@ -26,7 +26,7 @@
 extern "C" {
 #endif
 
-#define CVCL_ABI_VERSION 5
+#define CVCL_ABI_VERSION 6
 #define CVCL_OK 0
 #define CVCL_ERR_INVALID (-1)
 #define CVCL_ERR_UNSUPPORTED (-2)
@@ -158,18 +158,24 @@ int cvcl_sim_logits_fwd(const void* img, const void* txt, int ld, int Ni, int Nt
 /* ---- K5 backward --------------------------------------------------------------------------
  * (a) dL/dlogits tiles from recomputed logits: Gs0 [M0, N0] (rows = local images) and
  *     Gs1 [M1, N1] (rows = local texts), bf16, = exp(s) * coef * (softmax_row + softmax_col) with
- *     coef = upstream / (2 B_global).  The -2*I term of G = (softmax_row + softmax_col - 2 I)/(2B)
- *     is NOT in the bf16 matrix (it would dominate the rounding error); (b) adds it in fp32.
+ *     coef = upstream / (2 B_global), diagonal included.  The -2*I term of
+ *     G = (softmax_row + softmax_col - 2 I)/(2B) is NOT in the bf16 matrix (it would dominate the
+ *     rounding error): gdiag0 [M0] (gdiag1 [M1]) receives, per row m, G_ii - bf16(Gs[m, m + diag_off])
+ *     in fp32, with G_ii = w (expm1(S_ii - lse_q) + expm1(S_ii - lse_k)), w = exp(s) coef; (b) adds
+ *     gdiag[m] times the positive.  (When a pair is confident, w (P_row + P_col) and -2w nearly cancel;
+ *     the bf16 rounding of the first would otherwise be the whole gradient of the row.)
  *     lse_k0 [N0] = column LSEs seen by direction 0 (= all-gathered lse1), lse_k1 [N1] likewise.
- *     Gs1 may be NULL (single GPU: the dT GEMM reads Gs0 transposed in place).
+ *     Gs1 and gdiag1 may be NULL (single GPU: the dT GEMM reads Gs0 transposed in place, and its
+ *     diagonal is the same element, so it uses gdiag0).
  *     *dscale += sum G * logits (the logit_scale gradient, multimodal.py:711-715,783-787). */
 int cvcl_sim_infonce_bwd_g(const void* img_q, const void* txt_k, const void* txt_q, const void* img_k,
                            int ld, int M0, int N0, int M1, int N1, int E, float log_scale, int diag_off,
                            float coef, const float* lse_q0, const float* lse_k0, const float* lse_q1,
-                           const float* lse_k1, void* Gs0, int ldg0, void* Gs1, int ldg1, float* dscale,
-                           void* stream);
-/* (b) dFeat = Gs . other + diag_coef * diag_feat[m + diag_off] (the -2*I term of G, applied in
- *     fp32; diag_feat [diag_rows,E] bf16 may be NULL), followed by the F.normalize backward in the
+                           const float* lse_k1, void* Gs0, int ldg0, void* Gs1, int ldg1, float* gdiag0,
+                           float* gdiag1, float* dscale, void* stream);
+/* (b) dFeat = Gs . other + diag_coef[m] * diag_feat[m + diag_off] (diag_coef [M] = the gdiag of (a):
+ *     the diagonal of G in fp32; diag_feat [diag_rows,E] bf16 may be NULL, and with it diag_coef),
+ *     followed by the F.normalize backward in the
  *     epilogue (feat [M,E] bf16 + inv_norm).  Gs is [M,Kc] (gs_transposed = 0) or stored [Kc,M]
  *     (gs_transposed = 1: the other orientation is read in place, MN-major); other is the [Kc,E] bf16
  *     feature matrix as stored.  Exactly one output: out_f32 [M,E] (scaled by 1/row_len if given:
@@ -178,7 +184,7 @@ int cvcl_sim_infonce_bwd_g(const void* img_q, const void* txt_k, const void* txt
 int cvcl_feat_grad_norm_bwd(const void* Gs, int ldg, int gs_transposed, const void* other, int ld_other,
                             int M, int E, int Kc, const void* feat_bf16, int ld_feat, const float* inv_norm,
                             int normalize, const int64_t* row_len, const void* diag_feat, int ld_diag,
-                            int diag_rows, int diag_off, float diag_coef, float* out_f32, int ld_f32,
+                            int diag_rows, int diag_off, const float* diag_coef, float* out_f32, int ld_f32,
                             void* out_bf16, int ld_bf16, float* dbias, void* stream);
 /* same, with an optional fp32 scratch acc_scratch [M,E]: when the contraction is long (Kc >= 1536, the
  * sharded global batch) and the output has few tiles, the GEMM is split over the contraction into
@@ -187,7 +193,7 @@ int cvcl_feat_grad_norm_bwd(const void* Gs, int ldg, int gs_transposed, const vo
 int cvcl_feat_grad_norm_bwd_ws(const void* Gs, int ldg, int gs_transposed, const void* other, int ld_other,
                                int M, int E, int Kc, const void* feat_bf16, int ld_feat, const float* inv_norm,
                                int normalize, const int64_t* row_len, const void* diag_feat, int ld_diag,
-                               int diag_rows, int diag_off, float diag_coef, float* out_f32, int ld_f32,
+                               int diag_rows, int diag_off, const float* diag_coef, float* out_f32, int ld_f32,
                                void* out_bf16, int ld_bf16, float* dbias, float* acc_scratch, void* stream);
 /* (c) dW [E,K] = sum_m du[m,:]^T x[m,:]  (autograd of nn.Linear / 1x1 conv weight); du [M,E] and
  *     x [M,K] bf16 as stored (both read MN-major). */
@@ -201,6 +207,10 @@ int cvcl_head_weight_grad(const void* du, int ld_du, const void* x, int ld_x, in
  * (all fp32, overwritten), optional img/txt features fp32 [B,E].  Gradients are d(loss)/d(param)
  * for upstream = 1.  Workspace from cvcl_flat_step_workspace_bytes. */
 size_t cvcl_flat_step_workspace_bytes(int B, int L, int E, int K, int V);
+/* byte offsets of the blocks a finished cvcl_flat_contrastive_step leaves in its workspace (tests read them):
+ * out[0..11] = img16, txt16 [B,E] bf16, invn_i, invn_t, lse0, lse1 [B] fp32, G0 [B, ldB] bf16, du16 [B,E] bf16,
+ * dm [B,E] fp32 (d mean-embedding), gdiag [B] fp32, ldB, bytes. */
+int cvcl_flat_step_layout(int B, int L, int E, int K, int V, long long* out, int n);
 int cvcl_flat_contrastive_step(const void* x, int x_is_bf16, const int64_t* ids, const int64_t* lens,
                                const float* w, const float* bias, const float* table,
                                int B, int L, int E, int K, int V, int normalize, float log_scale,

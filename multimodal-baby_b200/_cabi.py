@@ -9,7 +9,7 @@ from ctypes import c_float, c_int, c_int64, c_size_t, c_void_p, c_char_p
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "lib", "libcvcl_b200.so")
-ABI_VERSION = 5
+ABI_VERSION = 6
 
 
 class CvclLibraryMissing(RuntimeError):
@@ -51,14 +51,15 @@ PROTOTYPES = {
                                      _P, _P, _I, _P]),
     "cvcl_sim_logits_fwd": (c_int, [_P, _P, _I, _I, _I, _I, _F, _P, _P, _P]),
     "cvcl_sim_infonce_bwd_g": (c_int, [_P, _P, _P, _P, _I, _I, _I, _I, _I, _I, _F, _I, _F, _P, _P, _P, _P,
-                                       _P, _I, _P, _I, _P, _P]),
+                                       _P, _I, _P, _I, _P, _P, _P, _P]),
     "cvcl_feat_grad_norm_bwd": (c_int, [_P, _I, _I, _P, _I, _I, _I, _I, _P, _I, _P, _I, _P, _P, _I, _I, _I,
-                                        _F, _P, _I, _P, _I, _P, _P]),
+                                        _P, _P, _I, _P, _I, _P, _P]),
     "cvcl_feat_grad_norm_bwd_ws": (c_int, [_P, _I, _I, _P, _I, _I, _I, _I, _P, _I, _P, _I, _P, _P, _I, _I, _I,
-                                           _F, _P, _I, _P, _I, _P, _P, _P]),
+                                           _P, _P, _I, _P, _I, _P, _P, _P]),
     "cvcl_head_weight_grad": (c_int, [_P, _I, _P, _I, _I, _I, _I, _P, _I, _P]),
     "cvcl_gemm_f32out": (c_int, [_P, _I, _I, _P, _I, _I, _I, _I, _I, _F, _P, _I, _P]),
     "cvcl_flat_step_workspace_bytes": (c_size_t, [_I, _I, _I, _I, _I]),
+    "cvcl_flat_step_layout": (c_int, [_I, _I, _I, _I, _I, _P, _I]),
     "cvcl_flat_contrastive_step": (c_int, [_P, _I, _P, _P, _P, _P, _P, _I, _I, _I, _I, _I, _I, _F, _I, _P,
                                            _P, _P, _P, _P, _P, _P, _P, _P, _P]),
     "cvcl_flat_fused_supported": (c_int, [_I, _I, _I, _I, _I]),

@@ -522,20 +522,22 @@ int cvcl_sim_logits_fwd(const void* img, const void* txt, int ld, int Ni, int Nt
 int cvcl_sim_infonce_bwd_g(const void* img_q, const void* txt_k, const void* txt_q, const void* img_k,
                            int ld, int M0, int N0, int M1, int N1, int E, float log_scale, int diag_off,
                            float coef, const float* lse_q0, const float* lse_k0, const float* lse_q1,
-                           const float* lse_k1, void* Gs0, int ldg0, void* Gs1, int ldg1, float* dscale,
-                           void* stream) {
-    CVCL_REQUIRE(img_q && txt_k && lse_q0 && lse_k0 && Gs0, "sim_infonce_bwd_g: null pointer");
-    CVCL_REQUIRE(!Gs1 || (txt_q && img_k && lse_q1 && lse_k1), "sim_infonce_bwd_g: direction 1 needs its operands");
+                           const float* lse_k1, void* Gs0, int ldg0, void* Gs1, int ldg1, float* gdiag0,
+                           float* gdiag1, float* dscale, void* stream) {
+    CVCL_REQUIRE(img_q && txt_k && lse_q0 && lse_k0 && Gs0 && gdiag0, "sim_infonce_bwd_g: null pointer");
+    CVCL_REQUIRE(!Gs1 || (txt_q && img_k && lse_q1 && lse_k1 && gdiag1), "sim_infonce_bwd_g: direction 1 needs its operands");
+    CVCL_REQUIRE(diag_off >= 0 && M0 + diag_off <= N0 && (!Gs1 || M1 + diag_off <= N1),
+                 "sim_infonce_bwd_g: positives out of range (M0=%d N0=%d M1=%d N1=%d diag_off=%d)", M0, N0, M1, N1, diag_off);
     CVCL_REQUIRE(M0 > 0 && N0 > 0 && E > 0, "sim_infonce_bwd_g: bad shape");
     GemmOperands op{}; op.ndir = Gs1 ? 2 : 1;
     op.A[0] = mat(img_q, M0, E, ld); op.B[0] = mat(txt_k, N0, E, ld); op.out[0] = mat(Gs0, M0, N0, ldg0);
     GemmShape gs{}; gs.M[0] = gs.M[1] = M0; gs.N[0] = gs.N[1] = N0; gs.K = E; gs.m_stride = kBM; gs.n_stride = kBN;
     EpiGradG::Params ep{};
     ep.scale = expf(log_scale); ep.coef = coef; ep.diag_off[0] = ep.diag_off[1] = diag_off;
-    ep.lse_q[0] = ep.lse_q[1] = lse_q0; ep.lse_k[0] = ep.lse_k[1] = lse_k0;
+    ep.lse_q[0] = ep.lse_q[1] = lse_q0; ep.lse_k[0] = ep.lse_k[1] = lse_k0; ep.gdiag[0] = ep.gdiag[1] = gdiag0;
     if (Gs1) {
         op.A[1] = mat(txt_q, M1, E, ld); op.B[1] = mat(img_k, N1, E, ld); op.out[1] = mat(Gs1, M1, N1, ldg1);
-        gs.M[1] = M1; gs.N[1] = N1; ep.lse_q[1] = lse_q1; ep.lse_k[1] = lse_k1;
+        gs.M[1] = M1; gs.N[1] = N1; ep.lse_q[1] = lse_q1; ep.lse_k[1] = lse_k1; ep.gdiag[1] = gdiag1;
     }
     ep.dscale_accum = dscale;
     if (sim_bn(N0, Gs1 ? N1 : N0) == 256) {
@@ -548,7 +550,7 @@ int cvcl_sim_infonce_bwd_g(const void* img_q, const void* txt_k, const void* txt
 int cvcl_feat_grad_norm_bwd(const void* Gs, int ldg, int gs_transposed, const void* other, int ld_other,
                             int M, int E, int Kc, const void* feat_bf16, int ld_feat, const float* inv_norm,
                             int normalize, const int64_t* row_len, const void* diag_feat, int ld_diag,
-                            int diag_rows, int diag_off, float diag_coef, float* out_f32, int ld_f32,
+                            int diag_rows, int diag_off, const float* diag_coef, float* out_f32, int ld_f32,
                             void* out_bf16, int ld_bf16, float* dbias, void* stream) {
     return cvcl_feat_grad_norm_bwd_ws(Gs, ldg, gs_transposed, other, ld_other, M, E, Kc, feat_bf16, ld_feat, inv_norm,
                                       normalize, row_len, diag_feat, ld_diag, diag_rows, diag_off, diag_coef, out_f32,
@@ -558,9 +560,10 @@ int cvcl_feat_grad_norm_bwd(const void* Gs, int ldg, int gs_transposed, const vo
 int cvcl_feat_grad_norm_bwd_ws(const void* Gs, int ldg, int gs_transposed, const void* other, int ld_other,
                                int M, int E, int Kc, const void* feat_bf16, int ld_feat, const float* inv_norm,
                                int normalize, const int64_t* row_len, const void* diag_feat, int ld_diag,
-                               int diag_rows, int diag_off, float diag_coef, float* out_f32, int ld_f32,
+                               int diag_rows, int diag_off, const float* diag_coef, float* out_f32, int ld_f32,
                                void* out_bf16, int ld_bf16, float* dbias, float* acc_scratch, void* stream) {
     CVCL_REQUIRE(Gs && other, "feat_grad_norm_bwd: null operand");
+    CVCL_REQUIRE(!diag_feat || diag_coef, "feat_grad_norm_bwd: diag_feat needs its per-row diag_coef");
     {
         // Long contraction (sharded global batch: Kc = world * b) on few output tiles: every CTA of the
         // single-kernel path would stream all of Kc serially (0.3 us per 64-wide chunk).  Split the
@@ -689,7 +692,7 @@ SideStream& side_stream() {
 
 struct FlatWs {
     __nv_bfloat16 *w16, *x16, *img16, *txt16, *G0, *du16;
-    float *invn_i, *invn_t, *lse0, *lse1, *dm, *u32;
+    float *invn_i, *invn_t, *lse0, *lse1, *gdiag, *dm, *u32;
     void* sim; int ldB; size_t bytes;
 };
 FlatWs carve_flat_ws(void* ws, int B, int L, int E, int K, int V) {
@@ -709,6 +712,7 @@ FlatWs carve_flat_ws(void* ws, int B, int L, int E, int K, int V) {
     f.invn_t = static_cast<float*>(take(4ull * B));
     f.lse0 = static_cast<float*>(take(4ull * B));
     f.lse1 = static_cast<float*>(take(4ull * B));
+    f.gdiag = static_cast<float*>(take(4ull * B));
     f.dm = static_cast<float*>(take(4ull * B * E));
     f.u32 = static_cast<float*>(take(4ull * B * E));
     f.sim = base + off;
@@ -720,6 +724,16 @@ FlatWs carve_flat_ws(void* ws, int B, int L, int E, int K, int V) {
 
 size_t cvcl_flat_step_workspace_bytes(int B, int L, int E, int K, int V) {
     return carve_flat_ws(nullptr, B, L, E, K, V).bytes;
+}
+
+int cvcl_flat_step_layout(int B, int L, int E, int K, int V, long long* out, int n) {
+    CVCL_REQUIRE(out && B > 0, "flat_step_layout: need out and B > 0");
+    const FlatWs f = carve_flat_ws(nullptr, B, L, E, K, V);
+    auto off = [](const void* p) { return static_cast<long long>(reinterpret_cast<uintptr_t>(p)); };
+    const long long v[] = {off(f.img16), off(f.txt16), off(f.invn_i), off(f.invn_t), off(f.lse0), off(f.lse1),
+                           off(f.G0), off(f.du16), off(f.dm), off(f.gdiag), f.ldB, static_cast<long long>(f.bytes)};
+    for (int i = 0; i < n && i < (int)(sizeof(v) / sizeof(v[0])); ++i) out[i] = v[i];
+    return CVCL_OK;
 }
 
 int cvcl_flat_contrastive_step(const void* x, int x_is_bf16, const int64_t* ids, const int64_t* lens,
@@ -798,18 +812,18 @@ int cvcl_flat_contrastive_step(const void* x, int x_is_bf16, const int64_t* ids,
     if (limit == 2) return CVCL_OK;
     const float coef = 0.5f / static_cast<float>(B);
     if ((rc = cvcl_sim_infonce_bwd_g(f.img16, f.txt16, nullptr, nullptr, E, B, B, 0, 0, E, log_scale, 0, coef,
-                                     f.lse0, f.lse1, nullptr, nullptr, f.G0, f.ldB, nullptr, 0, dscale, stream))) return rc;
-    const float dcoef = -2.f * expf(log_scale) * coef;
+                                     f.lse0, f.lse1, nullptr, nullptr, f.G0, f.ldB, nullptr, 0, f.gdiag, nullptr, dscale,
+                                     stream))) return rc;
     if (limit == 3) return CVCL_OK;
     CVCL_CHECK_CUDA(cudaEventRecord(ss.fork[1], st));
     CVCL_CHECK_CUDA(cudaStreamWaitEvent(ss.s, ss.fork[1], 0));
     if ((rc = cvcl_feat_grad_norm_bwd(f.G0, f.ldB, 1, f.img16, E, B, E, B, f.txt16, E, f.invn_t, normalize,
-                                      lens, f.img16, E, B, 0, dcoef, f.dm, E, nullptr, 0, nullptr, side))) return rc;
+                                      lens, f.img16, E, B, 0, f.gdiag, f.dm, E, nullptr, 0, nullptr, side))) return rc;
     // ... then the embedding scatter follows dT on the side stream while dI -> dW run on the main one
     if (limit != 4 && (rc = cvcl_embedding_scatter_add(ids, f.dm, dtable, B, L, E, V, 0, side))) return rc;
     CVCL_CHECK_CUDA(cudaEventRecord(ss.join[1], ss.s));
     if ((rc = cvcl_feat_grad_norm_bwd(f.G0, f.ldB, 0, f.txt16, E, B, E, B, f.img16, E, f.invn_i, normalize,
-                                      nullptr, f.txt16, E, B, 0, dcoef, nullptr, 0, f.du16, E, dbias, stream))) return rc;
+                                      nullptr, f.txt16, E, B, 0, f.gdiag, nullptr, 0, f.du16, E, dbias, stream))) return rc;
     if (limit != 4 && (rc = cvcl_head_weight_grad(f.du16, E, x16, K, E, K, B, dW, K, stream))) return rc;
     CVCL_CHECK_CUDA(cudaStreamWaitEvent(st, ss.join[1], 0));
     return CVCL_OK;

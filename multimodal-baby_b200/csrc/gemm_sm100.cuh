@@ -896,9 +896,12 @@ struct EpiSimStats1P {
 // ---- backward, step 1: recompute the logits tile and emit dL/dlogits (bf16) --------------
 // G = (softmax_row + softmax_col - 2*I) / (2B)  (SURVEY section 8 row a14; the autograd of
 // multimodal.py:808-810).  The bf16 matrix written here is Gs = exp(s)*coef*(softmax_row +
-// softmax_col) only: the -2*I term is ~B times larger than any other entry, and rounding it to
-// bf16 would dominate the error of every column sum of G (they cancel to ~0), so the consumer
-// (EpiNormBwd) adds it back in fp32.  dI = Gs*T - 2*exp(s)*coef*T_pos, dT likewise.
+// softmax_col) only, diagonal included: the -2*I term is ~B times larger than any other entry, and
+// rounding it to bf16 would dominate the error of every column sum of G (they cancel to ~0).  Per row
+// the epilogue also stores gdiag[m] = G_ii - bf16(Gs_ii) in fp32, G_ii = w (expm1(S_ii - lse_q) +
+// expm1(S_ii - lse_k)): w (P_row + P_col) and -2w nearly cancel when a pair is confident, and the
+// bf16 rounding of the first would otherwise be left as the whole gradient of that row.  The
+// consumers (EpiNormBwdT, featgrad_finish_kernel) add gdiag[m] * pos[m]: dI = Gs*T + gdiag o T_pos.
 // Direction z=1 (sharded runs only) has the operands swapped and emits the column block Gs^T.
 struct EpiGradG {
     static constexpr bool kClusterReduce = false;
@@ -911,6 +914,7 @@ struct EpiGradG {
         int diag_off[2];
         const float* lse_q[2];       // [M]  log-sum-exp of this direction's rows
         const float* lse_k[2];       // [N]  log-sum-exp of the other direction (columns here)
+        float* gdiag[2];             // [M]  G_ii - bf16(Gs_ii) of each row (fp32)
         float* dscale_accum;         // d loss / d s  (atomicAdd, direction 0 only; nullable)
     };
     template <int BN>
@@ -951,6 +955,14 @@ struct EpiGradG {
                     g[j] = gg;
                 }
             }
+            if (dcol >= n && dcol < n + 32 && m < M) {  // warp-uniform: one chunk of the diagonal tile per warp
+                float gd = 0.f;
+#pragma unroll
+                for (int j = 0; j < 32; ++j) if (n + j == dcol) gd = g[j];
+                const float sii = dv * p.scale;
+                const float gii = w * (expm1f(sii - __ldg(p.lse_q[cx.z] + m)) + expm1f(sii - __ldg(p.lse_k[cx.z] + dcol)));
+                p.gdiag[cx.z][m] = gii - __bfloat162float(__float2bfloat16_rn(gd));
+            }
             ds = fmaf(-2.f * w, dv, ds);
 #pragma unroll
             for (int j = 0; j < 4; ++j) swz_st16(cx.out_stage, cx.row, (c + 8 * j) * 2, pack_bf16x8(g + 8 * j));
@@ -977,8 +989,8 @@ struct EpiGradG {
     static __device__ __forceinline__ void phase2(const EpiCtx&, const GemmShape&, const Params&) {}
 };
 
-// ---- backward, step 2: dFeat = Gs * Other (+ the -2*I term), then the F.normalize backward ----
-//   acc[m,:] += diag_coef * pos[m,:]                      (pos = positives of the other modality)
+// ---- backward, step 2: dFeat = Gs * Other (+ the diagonal correction), then the F.normalize backward ----
+//   acc[m,:] += diag_coef[m] * pos[m,:]                   (pos = positives of the other modality)
 //   du = (acc - feat * <feat, acc>) * inv_norm            (cluster along N supplies the dot)
 // feat and pos tiles arrive by TMA (aux 0 / aux 1).  Output tile by TMA store: bf16 du (image side,
 // operand of the dW GEMM; + dbias column sums) or fp32 scaled by 1/len (text side: d mean-embedding).
@@ -992,11 +1004,16 @@ struct EpiNormBwdT {
         const float* inv_norm;                      // [M]
         int normalize;
         const long long* row_len;                   // [M] int64 lengths (nullable): out *= 1/len
-        int use_diag; float diag_coef;
+        int use_diag;
+        const float* diag_coef;                     // [M] gdiag of EpiGradG (read when use_diag)
         float* dbias;                               // [N] atomicAdd (nullable)
     };
+    static __device__ __forceinline__ float row_diag_coef(const EpiCtx& cx, const GemmShape& gs, const Params& p) {
+        const int m = cx.m0 + cx.row;
+        return (p.use_diag && m < gs.M[cx.z]) ? __ldg(p.diag_coef + m) : 0.f;
+    }
     template <int BN>
-    static __device__ __forceinline__ void load_acc(const EpiCtx& cx, const Params& p, int c, float* v) {
+    static __device__ __forceinline__ void load_acc(const EpiCtx& cx, const Params& p, float dc, int c, float* v) {
         ptx::tmem_ld_32x32(cx.tmem_row + c, v);
         if (p.use_diag) {
 #pragma unroll
@@ -1004,19 +1021,20 @@ struct EpiNormBwdT {
                 float d[8];
                 unpack_bf16x8(swz_ld16(cx.aux[1], cx.row, (c + 8 * j) * 2), d);
 #pragma unroll
-                for (int k = 0; k < 8; ++k) v[8 * j + k] = fmaf(p.diag_coef, d[k], v[8 * j + k]);
+                for (int k = 0; k < 8; ++k) v[8 * j + k] = fmaf(dc, d[k], v[8 * j + k]);
             }
         }
     }
     template <int BN>
     static __device__ __forceinline__ void phase1(const EpiCtx& cx, const GemmShape& gs, const Params& p) {
         const int N = gs.N[cx.z];
+        const float dc = row_diag_coef(cx, gs, p);
         float dot = 0.f;
         if (p.normalize) {
 #pragma unroll 1
             for (int c = 0; c < BN; c += 32) {
                 float v[32];
-                load_acc<BN>(cx, p, c, v);
+                load_acc<BN>(cx, p, dc, c, v);
                 const int n = cx.n0 + c;
                 if (n >= N) continue;
 #pragma unroll
@@ -1041,10 +1059,11 @@ struct EpiNormBwdT {
         for (uint32_t r = 0; r < nc; ++r) dot += ptx::ld_dsmem_f32(my, r);
         const float inv = (p.normalize && rv) ? __ldg(p.inv_norm + m) : 1.f;
         const float rs = (p.row_len && rv) ? 1.f / static_cast<float>(p.row_len[m]) : 1.f;
+        const float dc = row_diag_coef(cx, gs, p);
 #pragma unroll 1
         for (int c = 0; c < BN; c += 32) {
             float v[32];
-            load_acc<BN>(cx, p, c, v);
+            load_acc<BN>(cx, p, dc, c, v);
             const int n = cx.n0 + c;
             if (p.normalize) {
 #pragma unroll

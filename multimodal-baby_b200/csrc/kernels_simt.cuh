@@ -1331,7 +1331,7 @@ __global__ void __launch_bounds__(256) rownorm_bwd_kernel(const float* g, const 
 // second half of the split-K feature-gradient path (long contractions: sharded global batches).
 // acc [M, E] fp32 holds Gs . other summed over the K-splits; this warp-per-row pass applies what the
 // EpiNormBwdT epilogue does in the single-kernel path, in the same order:
-//   g = acc + diag_coef * diag[m + diag_off];  du = (g - feat <feat, g>) * inv_norm;  out = du / len
+//   g = acc + diag_coef[m] * diag[m + diag_off];  du = (g - feat <feat, g>) * inv_norm;  out = du / len
 // Outputs: fp32 [M, ld_f32] (may alias acc) or bf16 [M, ld_bf16]; dbias[E] += column sums (shared-memory
 // pre-reduction over the 8 rows of a block, then one global atomic per column and block).
 __device__ __forceinline__ float4 load_bf16x4(const __nv_bfloat16* p) {
@@ -1343,7 +1343,7 @@ __device__ __forceinline__ float4 load_bf16x4(const __nv_bfloat16* p) {
 
 __global__ void __launch_bounds__(256) featgrad_finish_kernel(const float* acc, int ld_acc, const __nv_bfloat16* feat,
                                                               int ld_feat, const __nv_bfloat16* diag, int ld_diag,
-                                                              int diag_rows, int diag_off, float diag_coef,
+                                                              int diag_rows, int diag_off, const float* diag_coef,
                                                               const float* inv_norm, int normalize,
                                                               const long long* row_len, int M, int E, float* out_f32,
                                                               int ld_f32, __nv_bfloat16* out_bf16, int ld_bf16,
@@ -1361,6 +1361,7 @@ __global__ void __launch_bounds__(256) featgrad_finish_kernel(const float* acc, 
         float4 g[kMaxVec], f[kMaxVec];
         float dot = 0.f;
         const bool use_diag = diag != nullptr && m + diag_off < diag_rows;
+        const float dc = use_diag ? __ldg(diag_coef + m) : 0.f;
 #pragma unroll
         for (int c = 0; c < kMaxVec; ++c) {
             g[c] = make_float4(0.f, 0.f, 0.f, 0.f); f[c] = g[c];
@@ -1369,8 +1370,8 @@ __global__ void __launch_bounds__(256) featgrad_finish_kernel(const float* acc, 
                 g[c] = *reinterpret_cast<const float4*>(acc + static_cast<size_t>(m) * ld_acc + e);
                 if (use_diag) {
                     const float4 d = load_bf16x4(diag + static_cast<size_t>(m + diag_off) * ld_diag + e);
-                    g[c].x = fmaf(diag_coef, d.x, g[c].x); g[c].y = fmaf(diag_coef, d.y, g[c].y);
-                    g[c].z = fmaf(diag_coef, d.z, g[c].z); g[c].w = fmaf(diag_coef, d.w, g[c].w);
+                    g[c].x = fmaf(dc, d.x, g[c].x); g[c].y = fmaf(dc, d.y, g[c].y);
+                    g[c].z = fmaf(dc, d.z, g[c].z); g[c].w = fmaf(dc, d.w, g[c].w);
                 }
                 if (normalize) f[c] = load_bf16x4(feat + static_cast<size_t>(m) * ld_feat + e);
             }
@@ -1616,8 +1617,11 @@ __global__ void __launch_bounds__(256) match_grad_kernel(const float* match_r, c
     if (idx < static_cast<long long>(b) * N) {
         const int i = static_cast<int>(idx / cols), t = static_cast<int>(idx % cols);
         const float x = (z ? match_c : match_r)[idx] * scale;
-        float gg = z ? __expf(x - lse0_all[i]) + __expf(x - lse1[t]) : __expf(x - lse0[i]) + __expf(x - lse1_all[t]);
-        if (z ? i == t + diag_off : t == i + diag_off) gg -= 2.f;
+        const float lr = z ? lse0_all[i] : lse0[i], lc = z ? lse1[t] : lse1_all[t];
+        // the positive as (P_row - 1) + (P_col - 1) with expm1: P_row + P_col - 2 cancels when the pair is confident,
+        // and the rounding of the exponentials would be left as the whole value (at one pair it is exactly 0)
+        float gg = (z ? i == t + diag_off : t == i + diag_off) ? expm1f(x - lr) + expm1f(x - lc)
+                                                                : __expf(x - lr) + __expf(x - lc);
         gg *= coef;
         (z ? dmatch_c : dmatch_r)[idx] = gg * scale;
         ds = gg * x;

@@ -570,31 +570,33 @@ def sim_infonce_bwd(img_q: Tensor, txt_k: Tensor, txt_q: Tensor, img_k: Tensor, 
     G0 = torch.empty((M0, ld0), dtype=torch.bfloat16, device=dev)
     G1 = None if single else torch.empty((M1, ld1), dtype=torch.bfloat16, device=dev)
     ds = torch.zeros((1,), dtype=torch.float32, device=dev)
+    # the diagonal of G in fp32, per row: G_ii - bf16(Gs_ii) (dT of one GPU reads Gs0^T, whose diagonal is gd0's)
+    gd0 = torch.empty((M0,), dtype=torch.float32, device=dev)
+    gd1 = gd0 if single else torch.empty((M1,), dtype=torch.float32, device=dev)
     _cabi.call("cvcl_sim_infonce_bwd_g", _p(img_q), _p(txt_k), _p(txt_q), _p(img_k), E, M0, N0, M1, N1, E,
                float(log_scale), int(diag_off), float(coef), _p(lse_q0), _p(lse_k0), _p(lse_q1), _p(lse_k1),
-               _p(G0), ld0, _p(G1), ld1, _p(ds), _stream())
+               _p(G0), ld0, _p(G1), ld1, _p(gd0), None if single else _p(gd1), _p(ds), _stream())
     dimg = torch.empty((M0, E), dtype=torch.float32, device=dev)
     dtxt = torch.empty((M1, E), dtype=torch.float32, device=dev)
-    dcoef = -2.0 * math.exp(log_scale) * coef            # the -2*I term of G, applied in fp32
     if min(N0, N1) >= 4096:
         # long contraction: plain 128 x 256-tile GEMMs (higher tensor throughput), then the fp32
-        # diagonal term as one axpy over [M,E]
+        # diagonal term as one addcmul over [M,E]
         _cabi.call("cvcl_gemm_f32out", _p(G0), ld0, 0, _p(txt_k), E, 1, M0, E, N0, 1.0, _p(dimg), E, _stream())
         if single:
             _cabi.call("cvcl_gemm_f32out", _p(G0), ld0, 1, _p(img_k), E, 1, M1, E, N1, 1.0, _p(dtxt), E, _stream())
         else:
             _cabi.call("cvcl_gemm_f32out", _p(G1), ld1, 0, _p(img_k), E, 1, M1, E, N1, 1.0, _p(dtxt), E, _stream())
-        dimg.add_(txt_k[diag_off:diag_off + M0].float(), alpha=dcoef)
-        dtxt.add_(img_k[diag_off:diag_off + M1].float(), alpha=dcoef)
+        dimg.addcmul_(txt_k[diag_off:diag_off + M0].float(), gd0[:, None])
+        dtxt.addcmul_(img_k[diag_off:diag_off + M1].float(), gd1[:, None])
         return dimg, dtxt, ds
     _cabi.call("cvcl_feat_grad_norm_bwd", _p(G0), ld0, 0, _p(txt_k), E, M0, E, N0, None, 0, None, 0, None,
-               _p(txt_k), E, N0, int(diag_off), dcoef, _p(dimg), E, None, 0, None, _stream())
+               _p(txt_k), E, N0, int(diag_off), _p(gd0), _p(dimg), E, None, 0, None, _stream())
     if single:      # dT = Gs^T . I: the same Gs read MN-major, no second orientation needed
         _cabi.call("cvcl_feat_grad_norm_bwd", _p(G0), ld0, 1, _p(img_k), E, M1, E, N1, None, 0, None, 0, None,
-                   _p(img_k), E, N1, int(diag_off), dcoef, _p(dtxt), E, None, 0, None, _stream())
+                   _p(img_k), E, N1, int(diag_off), _p(gd1), _p(dtxt), E, None, 0, None, _stream())
     else:
         _cabi.call("cvcl_feat_grad_norm_bwd", _p(G1), ld1, 0, _p(img_k), E, M1, E, N1, None, 0, None, 0, None,
-                   _p(img_k), E, N1, int(diag_off), dcoef, _p(dtxt), E, None, 0, None, _stream())
+                   _p(img_k), E, N1, int(diag_off), _p(gd1), _p(dtxt), E, None, 0, None, _stream())
     return dimg, dtxt, ds
 
 
@@ -742,6 +744,15 @@ def fused_supported(B, L, E, K, V) -> bool:
     if ok is None:
         ok = _FUSED_OK[key] = bool(_cabi.load().cvcl_flat_fused_supported(B, L, E, K, V))
     return ok
+
+
+def flat_step_layout(B, L, E, K, V):
+    """workspace block offsets of the multi-kernel step after it ran (see cvcl_flat_step_layout)."""
+    import ctypes
+    arr = (ctypes.c_longlong * 12)()
+    _cabi.call("cvcl_flat_step_layout", B, L, E, K, V, arr, 12)
+    names = ["img16", "txt16", "invn_i", "invn_t", "lse0", "lse1", "G0", "du16", "dm", "gdiag", "ldB", "bytes"]
+    return dict(zip(names, [int(v) for v in arr]))
 
 
 def fused_layout(B, L, E, K, V):
@@ -999,25 +1010,25 @@ def flat_step_sharded(x, ids, lens, w, bias, table, log_scale, normalize, need_g
         ds, db, dtable, dW = split_flat_grads(stats[8:], E, K, V)
         ldg = _pad8(Bg)
         G0 = torch.empty((B, ldg), **bf); G1 = torch.empty((B, ldg), **bf)
+        gdiag = torch.empty((2, B), **f32)          # per row: G_ii - bf16(Gs_ii) of each direction
         coef = 0.5 / Bg
         C("cvcl_sim_infonce_bwd_g", _p(img_l), _p(txt_a), _p(txt_l), _p(img_a), 2 * E, B, Bg, B, Bg, E,
           float(log_scale), rank * B, coef, _p(lse[0]), _p(lse1_all), _p(lse[1]), _p(lse0_all),
-          _p(G0), ldg, _p(G1), ldg, _p(ds), st)
+          _p(G0), ldg, _p(G1), ldg, _p(gdiag[0]), _p(gdiag[1]), _p(ds), st)
         if phase_limit == 5:
             return stats, img_f, txt_f
-        dcoef = -2.0 * math.exp(log_scale) * coef
         du16 = torch.empty((B, E), **bf); dm = torch.empty((B, E), **f32)
         # ---- backward: dT -> embedding scatter (side) || dI -> dW (main)
         side.wait_stream(main)
         with torch.cuda.stream(side):
             ss = side.cuda_stream
             C("cvcl_feat_grad_norm_bwd", _p(G1), ldg, 0, _p(img_a), 2 * E, B, E, Bg, _p(txt_l), 2 * E, _p(invn_t),
-              int(normalize), _p(lens), _p(img_a), 2 * E, Bg, rank * B, dcoef, _p(dm), E, None, 0, None, ss)
+              int(normalize), _p(lens), _p(img_a), 2 * E, Bg, rank * B, _p(gdiag[1]), _p(dm), E, None, 0, None, ss)
             C("cvcl_embedding_scatter_add", _p(ids), _p(dm), _p(dtable), B, L, E, V, 0, ss)
         # long contraction (Bg >= 1536): the library splits it over the SMs into this fp32 scratch
         acc_i = torch.empty((B, E), **f32) if Bg >= 1536 else None
         C("cvcl_feat_grad_norm_bwd_ws", _p(G0), ldg, 0, _p(txt_a), 2 * E, B, E, Bg, _p(img_l), 2 * E, _p(invn_i),
-          int(normalize), None, _p(txt_a), 2 * E, Bg, rank * B, dcoef, None, 0, _p(du16), E, _p(db), _p(acc_i), st)
+          int(normalize), None, _p(txt_a), 2 * E, Bg, rank * B, _p(gdiag[0]), None, 0, _p(du16), E, _p(db), _p(acc_i), st)
         C("cvcl_head_weight_grad", _p(du16), E, _p(x16), K, E, K, B, _p(dW), K, st)
         main.wait_stream(side)        # every side-stream use is ordered before anything that follows
     if phase_limit == 6:

@@ -11,7 +11,9 @@ magnitude tighter than a whole-step comparison, and a failure names the phase.
 
 Test infrastructure.
 """
+import json
 import math
+import os
 
 import numpy as np
 import torch
@@ -117,6 +119,31 @@ def counts(ids, V):
 
 
 # ------------------------------------------------------------------------------------------------ reference
+class Gates:
+    """collects every gate of one case, appends the measured values to the file named by the environment variable
+    `report_env` (JSON lines) when it is set, then fails with every gate that did not hold"""
+    def __init__(self, name, report_env):
+        self.name, self.report_env, self.values, self.failed = name, report_env, {}, []
+
+    def le(self, key, value, limit):
+        value = float(value)
+        self.values[key] = value
+        if not (value <= limit):
+            self.failed.append("%s = %.3e > %.1e" % (key, value, limit))
+
+    def true(self, key, cond, info=None):
+        self.values[key] = bool(cond) if info is None else info
+        if not cond:
+            self.failed.append("%s failed (%s)" % (key, info))
+
+    def finish(self):
+        path = os.environ.get(self.report_env)
+        if path:
+            with open(path, "a") as fh:
+                fh.write(json.dumps({"case": self.name, **self.values}) + "\n")
+        assert not self.failed, "%s: %s" % (self.name, "; ".join(self.failed))
+
+
 def worst_row(got, ref):
     """max over rows of |got - ref|_2 / |ref|_2 (rows that are zero on both sides count 0)."""
     got = got.double().reshape(got.shape[0], -1); ref = ref.double().reshape(ref.shape[0], -1)

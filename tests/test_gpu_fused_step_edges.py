@@ -9,9 +9,7 @@ world 1 bit-identical to the single-GPU one.
 
 The committed gates are about 4x the worst errors measured on a B200; DESIGN section 4 lists both.
 Set FUSED_EDGES_REPORT=<file> to append every case's measured values to <file> as JSON lines."""
-import json
 import math
-import os
 
 import numpy as np
 import pytest
@@ -43,27 +41,8 @@ GATE = dict(                # measured maximum over the cases on a B200 (1000 W)
 NEAR_TIE = 1e-6             # DESIGN section 4: an fp64 top-two gap below 1e-6 max|S| may go either way
 
 
-class Gates:
-    def __init__(self, name):
-        self.name, self.values, self.failed = name, {}, []
-
-    def le(self, key, value, limit):
-        value = float(value)
-        self.values[key] = value
-        if not (value <= limit):
-            self.failed.append("%s = %.3e > %.1e" % (key, value, limit))
-
-    def true(self, key, cond, info=None):
-        self.values[key] = bool(cond) if info is None else info
-        if not cond:
-            self.failed.append("%s failed (%s)" % (key, info))
-
-    def finish(self):
-        path = os.environ.get("FUSED_EDGES_REPORT")
-        if path:
-            with open(path, "a") as fh:
-                fh.write(json.dumps({"case": self.name, **self.values}) + "\n")
-        assert not self.failed, "%s: %s" % (self.name, "; ".join(self.failed))
+def Gates(name):
+    return F.Gates(name, "FUSED_EDGES_REPORT")
 
 
 @pytest.fixture(scope="module")

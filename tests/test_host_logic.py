@@ -31,7 +31,7 @@ def _lit(**kw):
 
 
 # ------------------------------------------------------------------------------ C ABI surface
-def test_library_exports_every_declared_symbol():
+def test_library_exports_every_declared_symbol_at_the_header_abi_version():
     hdr = open(os.path.join(ROOT, "include", "cvcl_b200.h")).read()
     declared = sorted(set(re.findall(r"\b(cvcl_[a-z0-9_]+)\s*\(", hdr)))
     assert len(declared) >= 25
@@ -40,7 +40,9 @@ def test_library_exports_every_declared_symbol():
         assert hasattr(lib, name), "libcvcl_b200.so does not export %s" % name
     # the ctypes prototype table covers exactly the header
     assert sorted(cv._cabi.PROTOTYPES) == declared
-    assert cv._cabi.load().cvcl_abi_version() == cv._cabi.ABI_VERSION == 5
+    # library, bindings and header agree on the ABI version (6: per-row diagonal of G in the InfoNCE backward)
+    header_abi = int(re.search(r"#define CVCL_ABI_VERSION (\d+)", hdr).group(1))
+    assert cv._cabi.load().cvcl_abi_version() == cv._cabi.ABI_VERSION == header_abi == 6
 
 
 def test_library_links_no_torch_and_is_sm100a():
