@@ -17,13 +17,6 @@ constexpr int kBN = 128;
 constexpr int kStages = 4;
 
 inline cudaStream_t as_stream(void* s) { return reinterpret_cast<cudaStream_t>(s); }
-// the fused step zeroes the split-K scratch on its side stream; it tells the head entry point so
-inline bool& head_scratch_zeroed() { static thread_local bool v = false; return v; }
-inline bool head_splitk_disabled() {
-    static int v = -1;
-    if (v < 0) { const char* e = getenv("CVCL_B200_HEAD_SPLITK"); v = (e && e[0] == '0') ? 1 : 0; }
-    return v == 1;
-}
 inline int warps_grid(long long n_warps, int block = 256) {
     return static_cast<int>((n_warps * 32 + block - 1) / block);
 }
@@ -375,10 +368,12 @@ static int gemm_f32out_limited(const void* A, int lda, int a_mn, const void* Bm,
 }
 
 // ------------------------------------------------------------------------------------ K2
-int cvcl_head_proj_norm_fwd(const void* x, int ldx, const void* w, int ldw, const float* bias,
-                            int M, int E, int K, int normalize,
-                            float* out_f32, int ld_f32, void* out_bf16, int ld_bf16,
-                            float* inv_norm, void* stream) {
+// scratch_zeroed: out_f32 is already zero (the multi-kernel step clears it on its side stream), so the
+// split-K path skips its memset
+static int head_proj_norm(const void* x, int ldx, const void* w, int ldw, const float* bias,
+                          int M, int E, int K, int normalize,
+                          float* out_f32, int ld_f32, void* out_bf16, int ld_bf16,
+                          float* inv_norm, bool scratch_zeroed, void* stream) {
     CVCL_REQUIRE(x && w, "head_proj_norm_fwd: null operand");
     CVCL_REQUIRE(M > 0 && E > 0 && K > 0, "head_proj_norm_fwd: bad shape M=%d E=%d K=%d", M, E, K);
     const int cluster = ceil_div(E, kBN);
@@ -395,12 +390,12 @@ int cvcl_head_proj_norm_fwd(const void* x, int ldx, const void* w, int ldw, cons
         const int tiles = ceil_div(M, kBM) * ceil_div(E, kBN);
         const int chunks = ceil_div(K, kBK);
         if (out_f32 && tiles * 4 <= sm_count() && chunks >= 16 && ld_f32 % 4 == 0 && E % 4 == 0 &&
-            (reinterpret_cast<uintptr_t>(out_f32) & 15) == 0 && !head_splitk_disabled()) {
+            (reinterpret_cast<uintptr_t>(out_f32) & 15) == 0) {
             int splits = sm_count() / tiles;
             if (splits > chunks / 4) splits = chunks / 4;
             while (splits > 1 && ceil_div(chunks, splits) * (splits - 1) >= chunks) --splits;
             if (splits > 1) {
-                if (!head_scratch_zeroed())
+                if (!scratch_zeroed)
                     CVCL_CHECK_CUDA(cudaMemsetAsync(out_f32, 0, sizeof(float) * static_cast<size_t>(M) * ld_f32, as_stream(stream)));
                 gs.k_splits = splits;
                 EpiAtomicAddF32::Params ea{}; ea.C = out_f32; ea.ldc = ld_f32; ea.alpha = 1.f;
@@ -423,6 +418,14 @@ int cvcl_head_proj_norm_fwd(const void* x, int ldx, const void* w, int ldw, cons
     if (ceil_div(M, kBM) * cluster > 2 * sm_count())
         return launch_gemm<kBN, 3, EpiHeadNorm, false, false>(op, gs, ep, cluster, as_stream(stream));
     return launch_gemm<kBN, 6, EpiHeadNorm, false, false>(op, gs, ep, cluster, as_stream(stream));
+}
+
+int cvcl_head_proj_norm_fwd(const void* x, int ldx, const void* w, int ldw, const float* bias,
+                            int M, int E, int K, int normalize,
+                            float* out_f32, int ld_f32, void* out_bf16, int ld_bf16,
+                            float* inv_norm, void* stream) {
+    return head_proj_norm(x, ldx, w, ldw, bias, M, E, K, normalize, out_f32, ld_f32, out_bf16, ld_bf16, inv_norm,
+                          false, stream);
 }
 
 // ------------------------------------------------------------------------------------ K3+K4
@@ -752,10 +755,6 @@ int cvcl_flat_contrastive_step(const void* x, int x_is_bf16, const int64_t* ids,
     int rc;
     if ((rc = ss.init())) return rc;
     void* side = ss.s;
-    // measurement hook (tools/step_phases.py): stop after phase k of {1 encoders, 2 similarity + InfoNCE,
-    // 3 Gs, 4 dI and dT}; 11 / 12 run only the head chain / only the text encoder of phase 1
-    int limit = 0;
-    if (const char* e = getenv("CVCL_B200_STEP_PHASES")) limit = atoi(e);
     // ---- forward: [memsets -> text encoder] (side) || [cast W -> head GEMM] (main)
     CVCL_CHECK_CUDA(cudaEventRecord(ss.fork[0], st));
     CVCL_CHECK_CUDA(cudaStreamWaitEvent(ss.s, ss.fork[0], 0));
@@ -778,14 +777,9 @@ int cvcl_flat_contrastive_step(const void* x, int x_is_bf16, const int64_t* ids,
         }
         CVCL_CHECK_CUDA(cudaEventRecord(ss.join[2], ss.s2));
     }
-    if (limit != 11 && (rc = cvcl_text_encoder_fwd(ids, lens, table, B, L, E, V, normalize, 0, 1.f, txt_feat_f32, f.txt16, E,
-                                                   f.invn_t, nullptr, nullptr, status, side))) return rc;
+    if ((rc = cvcl_text_encoder_fwd(ids, lens, table, B, L, E, V, normalize, 0, 1.f, txt_feat_f32, f.txt16, E,
+                                    f.invn_t, nullptr, nullptr, status, side))) return rc;
     CVCL_CHECK_CUDA(cudaEventRecord(ss.join[0], ss.s));
-    if (limit == 12) {
-        CVCL_CHECK_CUDA(cudaStreamWaitEvent(st, ss.join[0], 0));
-        if (need_grads) CVCL_CHECK_CUDA(cudaStreamWaitEvent(st, ss.join[2], 0));
-        return CVCL_OK;
-    }
     if ((rc = cvcl_cast_transpose(w, 0, f.w16, nullptr, 1, E, K, K, K, 0, 0, 0, 0, stream))) return rc;
     const void* x16 = x;
     if (!x_is_bf16 || (reinterpret_cast<uintptr_t>(x) & 15)) {
@@ -793,15 +787,9 @@ int cvcl_flat_contrastive_step(const void* x, int x_is_bf16, const int64_t* ids,
         x16 = f.x16;
     }
     CVCL_CHECK_CUDA(cudaStreamWaitEvent(st, ss.fork[2], 0));
-    head_scratch_zeroed() = true;
-    rc = cvcl_head_proj_norm_fwd(x16, K, f.w16, K, bias, B, E, K, normalize, img_f32, E, f.img16, E, f.invn_i, stream);
-    head_scratch_zeroed() = false;
-    if (rc) return rc;
+    if ((rc = head_proj_norm(x16, K, f.w16, K, bias, B, E, K, normalize, img_f32, E, f.img16, E, f.invn_i, true,
+                             stream))) return rc;
     CVCL_CHECK_CUDA(cudaStreamWaitEvent(st, ss.join[0], 0));
-    if (limit == 1 || limit == 11) {
-        if (need_grads) CVCL_CHECK_CUDA(cudaStreamWaitEvent(st, ss.join[2], 0));
-        return CVCL_OK;
-    }
     // ---- K3 + K4
     if ((rc = sim_infonce_fwd_impl(f.img16, f.txt16, f.txt16, f.img16, E, B, B, B, B, E, log_scale, 0,
                                    1.f / static_cast<float>(B), f.sim, f.lse0, f.lse1, nullptr, nullptr, out5, stream,
@@ -809,22 +797,20 @@ int cvcl_flat_contrastive_step(const void* x, int x_is_bf16, const int64_t* ids,
     if (!need_grads) return CVCL_OK;
     // ---- K5: Gs (one orientation) -> dI (K-major Gs, main) || dT (the same Gs read MN-major, side)
     CVCL_CHECK_CUDA(cudaStreamWaitEvent(st, ss.join[2], 0));     // gradient accumulators are zero (ds is the first user)
-    if (limit == 2) return CVCL_OK;
     const float coef = 0.5f / static_cast<float>(B);
     if ((rc = cvcl_sim_infonce_bwd_g(f.img16, f.txt16, nullptr, nullptr, E, B, B, 0, 0, E, log_scale, 0, coef,
                                      f.lse0, f.lse1, nullptr, nullptr, f.G0, f.ldB, nullptr, 0, f.gdiag, nullptr, dscale,
                                      stream))) return rc;
-    if (limit == 3) return CVCL_OK;
     CVCL_CHECK_CUDA(cudaEventRecord(ss.fork[1], st));
     CVCL_CHECK_CUDA(cudaStreamWaitEvent(ss.s, ss.fork[1], 0));
     if ((rc = cvcl_feat_grad_norm_bwd(f.G0, f.ldB, 1, f.img16, E, B, E, B, f.txt16, E, f.invn_t, normalize,
                                       lens, f.img16, E, B, 0, f.gdiag, f.dm, E, nullptr, 0, nullptr, side))) return rc;
     // ... then the embedding scatter follows dT on the side stream while dI -> dW run on the main one
-    if (limit != 4 && (rc = cvcl_embedding_scatter_add(ids, f.dm, dtable, B, L, E, V, 0, side))) return rc;
+    if ((rc = cvcl_embedding_scatter_add(ids, f.dm, dtable, B, L, E, V, 0, side))) return rc;
     CVCL_CHECK_CUDA(cudaEventRecord(ss.join[1], ss.s));
     if ((rc = cvcl_feat_grad_norm_bwd(f.G0, f.ldB, 0, f.txt16, E, B, E, B, f.img16, E, f.invn_i, normalize,
                                       nullptr, f.txt16, E, B, 0, f.gdiag, nullptr, 0, f.du16, E, dbias, stream))) return rc;
-    if (limit != 4 && (rc = cvcl_head_weight_grad(f.du16, E, x16, K, E, K, B, dW, K, stream))) return rc;
+    if ((rc = cvcl_head_weight_grad(f.du16, E, x16, K, E, K, B, dW, K, stream))) return rc;
     CVCL_CHECK_CUDA(cudaStreamWaitEvent(st, ss.join[1], 0));
     return CVCL_OK;
 }

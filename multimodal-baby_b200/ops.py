@@ -667,7 +667,7 @@ def split_flat_grads(flat: Tensor, E: int, K: int, V: int):
 # (FusedAdamW: cvcl_adamw_step's bf16_shadow output) hand it over, so no cast runs at all.
 _SHADOWS = {}
 _FUSED_WS = {}
-FUSED_STEP = True          # False (or CVCL_B200_FUSED=0): always use the multi-kernel step
+FUSED_STEP = True          # False: always use the multi-kernel step, single-GPU and sharded
 
 
 def _shadow_entry(w):
@@ -721,23 +721,10 @@ def _fused_workspace(dev, B, L, E, K, V):
 
 
 _FUSED_OK = {}
-_FUSED_ENV = None
-
-
-def _fused_env() -> bool:
-    global _FUSED_ENV
-    if _FUSED_ENV is None:
-        import os
-        _FUSED_ENV = os.environ.get("CVCL_B200_FUSED", "1") != "0"
-    return _FUSED_ENV
 
 
 def fused_supported(B, L, E, K, V) -> bool:
-    global _FUSED_ENV
-    if _FUSED_ENV is None:
-        import os
-        _FUSED_ENV = os.environ.get("CVCL_B200_FUSED", "1") != "0"
-    if not (FUSED_STEP and _FUSED_ENV):
+    if not FUSED_STEP:
         return False
     key = (B, L, E, K, V)
     ok = _FUSED_OK.get(key)
@@ -893,16 +880,14 @@ def flat_contrastive_loss(x, ids, lens, w, bias, table, s, normalize=True, want_
 
 
 def flat_step_sharded(x, ids, lens, w, bias, table, log_scale, normalize, need_grads, want_features, group,
-                      stats_slot=0, phase_limit=None):
+                      stats_slot=0):
     """The flat train step with the batch sharded by pairs over `group` (SURVEY 8e): local encoders,
     ONE all-gather of the bf16 [img|txt] features, row-block + column-block InfoNCE, one all-gather of
     the LSEs, local backward, ONE all-reduce of [out5 | ds | db | dtable | dW].
     -> (stats_flat, img_feat | None, txt_feat | None); stats_flat = [out5(8) | split_flat_grads layout].
     With the peer-memory exchange (sharding.PeerExchange) the three collectives are single kernels over
     NVLink peer memory and stats_flat is the persistent symmetric block `stats_slot`: valid until the
-    next call with the same slot.  phase_limit (measurement hook, tools/sharded_phases.py): stop after
-    phase k of {1 local encoders, 2 feature exchange, 3 similarity + InfoNCE, 4 LSE exchange, 5 Gs,
-    6 local backward}; every rank must pass the same value."""
+    next call with the same slot."""
     from . import sharding
     _need_cuda(x, ids, lens, w, bias, table)
     world, rank = sharding.group_info(group)
@@ -927,8 +912,7 @@ def flat_step_sharded(x, ids, lens, w, bias, table, log_scale, normalize, need_g
     n_stats = 8 + (n_g if need_grads else 0)
     # the three collectives run over peer-mapped symmetric memory when available (sharding.PeerExchange):
     # the arena is sized for the training step and shared with the forward-only call
-    use_fused = (world > 1 and phase_limit is None and FUSED_STEP and _fused_env()
-                 and bool(lib.cvcl_flat_fused_sharded_supported(B, L, E, K, V, world)))
+    use_fused = world > 1 and FUSED_STEP and bool(lib.cvcl_flat_fused_sharded_supported(B, L, E, K, V, world))
     # (the one-kernel step keeps its per-tile gradient scratch in the same arena)
     min_scr = int(lib.cvcl_flat_fused_sharded_scratch_bytes(B, L, E, K, V, world)) if use_fused else 0
     px = sharding.PeerExchange.get(group, B, E, 8 + n_g, dev, min_scr) if world > 1 else None
@@ -980,23 +964,16 @@ def flat_step_sharded(x, ids, lens, w, bias, table, log_scale, normalize, need_g
     C("cvcl_head_proj_norm_fwd", _p(x16), K, _p(w16), K, _p(bias), B, E, K, int(normalize), _p(img_u), E,
       _p(img_l), 2 * E, _p(invn_i), st)
     main.wait_stream(side)
-    if phase_limit == 1:
-        main.wait_stream(zero)
-        return stats, img_f, txt_f
     if px is not None:       # one kernel: 16-byte stores into every rank's gathered buffer (NVLink) + barrier
         feats_all = px.gather_feats(st)
     else:
         feats_all = sharding.all_gather_rows(feats, group, world)      # [Bg, 2E] (NCCL)
     img_a, txt_a = feats_all[:, :E], feats_all[:, E:]
     main.wait_stream(zero)               # the similarity kernel accumulates out5 into stats[0:8]
-    if phase_limit == 2:
-        return stats, img_f, txt_f
     ws = torch.empty((lib.cvcl_sim_workspace_bytes(B, Bg, B, Bg),), dtype=torch.uint8, device=dev)
     lse = px.lse if px is not None else torch.empty((2, B), **f32)
     C("cvcl_sim_infonce_fwd", _p(img_l), _p(txt_a), _p(txt_l), _p(img_a), 2 * E, B, Bg, B, Bg, E,
       float(log_scale), rank * B, 1.0 / Bg, _p(ws), _p(lse[0]), _p(lse[1]), None, None, _p(stats), 0, st)
-    if phase_limit == 3:
-        return stats, img_f, txt_f
     if need_grads:
         if px is not None:
             lse_all = px.gather_lse(st)
@@ -1005,8 +982,6 @@ def flat_step_sharded(x, ids, lens, w, bias, table, log_scale, normalize, need_g
         else:
             lse_all = lse
         lse0_all, lse1_all = lse_all[0].reshape(-1), lse_all[1].reshape(-1)
-        if phase_limit == 4:
-            return stats, img_f, txt_f
         ds, db, dtable, dW = split_flat_grads(stats[8:], E, K, V)
         ldg = _pad8(Bg)
         G0 = torch.empty((B, ldg), **bf); G1 = torch.empty((B, ldg), **bf)
@@ -1015,8 +990,6 @@ def flat_step_sharded(x, ids, lens, w, bias, table, log_scale, normalize, need_g
         C("cvcl_sim_infonce_bwd_g", _p(img_l), _p(txt_a), _p(txt_l), _p(img_a), 2 * E, B, Bg, B, Bg, E,
           float(log_scale), rank * B, coef, _p(lse[0]), _p(lse1_all), _p(lse[1]), _p(lse0_all),
           _p(G0), ldg, _p(G1), ldg, _p(gdiag[0]), _p(gdiag[1]), _p(ds), st)
-        if phase_limit == 5:
-            return stats, img_f, txt_f
         du16 = torch.empty((B, E), **bf); dm = torch.empty((B, E), **f32)
         # ---- backward: dT -> embedding scatter (side) || dI -> dW (main)
         side.wait_stream(main)
@@ -1031,8 +1004,6 @@ def flat_step_sharded(x, ids, lens, w, bias, table, log_scale, normalize, need_g
           int(normalize), None, _p(txt_a), 2 * E, Bg, rank * B, _p(gdiag[0]), None, 0, _p(du16), E, _p(db), _p(acc_i), st)
         C("cvcl_head_weight_grad", _p(du16), E, _p(x16), K, E, K, B, _p(dW), K, st)
         main.wait_stream(side)        # every side-stream use is ordered before anything that follows
-    if phase_limit == 6:
-        return stats, img_f, txt_f
     if px is not None:       # one kernel: barrier, two-shot in-place sum over peer memory, barrier
         px.allreduce_stats(stats_slot, n_stats, st)
     elif world > 1:
