@@ -435,6 +435,22 @@ int cvcl_conv1x1_f32(const float* x, const float* w, const float* bias, int B, i
 int cvcl_spatial_max_scores_f32(const float* img, const float* tok, const int64_t* lens, const int* txt_index, int M,
                                 int HW, int E, int C, int L, int n_way, float log_scale, float* out, void* stream);
 
+/* ---- text-to-location attention maps for spatial embeddings (fp32 SIMT) -------------------------
+ * The per-location terms of the spatial similarity (multimodal.py:771-780) before its max / mean reductions; the
+ * reference returns no such tensor, these are the summands of its own forward.  Image m is paired with label
+ * c = txt_index[m] (NULL = identity, then C >= M):
+ *   token_maps[m,l,p] = <img[m,p,:], tok[c,l,:]>                          for l < len[c]; exactly 0 for l >= len[c]
+ *   utt_maps[m,p]     = (sum_{l < len[c]} token_maps[m,l,p]) / len[c]     (position order; len 0 gives NaN)
+ *   token_argmax[m,l] = first p attaining max_p token_maps[m,l,p] (a NaN wins), -1 for l >= len[c]
+ * img [M,HW,E] fp32 normalised location features (NHWC rows), tok [C,L,E] fp32 per-token text features, lens [C];
+ * token_maps [M,L,HW] and token_argmax [M,L] are nullable, utt_maps [M,HW].  Match units (no exp(s)).  A label
+ * index outside [0, C) gives NaN maps and arg-max -1.  The dots are bit-identical to the ones
+ * cvcl_spatial_max_scores_f32 takes the maximum of in trial mode; no atomics (a replay is bit-identical).
+ * HW <= 256; the HW x E block must fit in shared memory (49 x 1024 does). */
+int cvcl_spatial_attention_f32(const float* img, const float* tok, const int64_t* lens, const int* txt_index, int M,
+                               int HW, int E, int C, int L, float* token_maps, float* utt_maps, int* token_argmax,
+                               void* stream);
+
 #ifdef __cplusplus
 }
 #endif

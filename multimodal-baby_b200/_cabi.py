@@ -101,6 +101,7 @@ PROTOTYPES = {
     "cvcl_eval_nway_fwd": (c_int, [_P, _P, _P, _I, _I, _I, _I, _F, _P, _P, _P]),
     "cvcl_conv1x1_f32": (c_int, [_P, _P, _P, _I, _I, _I, _I, _P, _P]),
     "cvcl_spatial_max_scores_f32": (c_int, [_P, _P, _P, _P, _I, _I, _I, _I, _I, _I, _F, _P, _P]),
+    "cvcl_spatial_attention_f32": (c_int, [_P, _P, _P, _P, _I, _I, _I, _I, _I, _P, _P, _P, _P]),
 }
 
 _lib = None

@@ -56,6 +56,42 @@ SimWs carve_sim_ws(void* ws, int M0, int N0, int M1, int N1) {
     return w;
 }
 
+// Launch plan of spatial_max_scores_f32_kernel and spatial_attention_f32_kernel, which share the image staging and
+// the chunk dots: token rows per chunk (tt), k-split lanes per work item (ks), shared-memory row stride of the image
+// block (ld4, float4 units) and the dynamic shared memory.  A dot depends on ks only, so the two kernels planned
+// with the same rows_wanted compute the same bits.
+struct SpatialPlan {
+    int tt, ks, ld4;
+    size_t smem;
+    int max_smem, dev;
+};
+
+int spatial_plan(const char* who, int HW, int E, int rows_wanted, SpatialPlan& pl) {
+    const int E4 = E / 4;
+    // token rows per chunk: every row a label needs in one chunk where possible, at most 4 rows per work item and
+    // 256 work items per block
+    int tt = (rows_wanted + 3) / 4 * 4;
+    const int tt_cap = 4 * (256 / HW) < 64 ? 4 * (256 / HW) : 64;
+    if (tt > tt_cap) tt = tt_cap;
+    CVCL_CHECK_CUDA(cudaGetDevice(&pl.dev));
+    CVCL_CHECK_CUDA(cudaDeviceGetAttribute(&pl.max_smem, cudaDevAttrMaxSharedMemoryPerBlockOptin, pl.dev));
+    int ks = 0, ld4 = 0;
+    size_t smem = 0;
+    for (;; tt -= 4) {
+        CVCL_REQUIRE(tt >= 4, "%s: the %d x %d image block does not fit in shared memory", who, HW, E);
+        const int items = (tt / 4) * HW;
+        ks = 1;
+        while (ks < 32 && 2 * ks * items <= 256 && E4 % (2 * ks) == 0) ks *= 2;
+        // quarter-warps of 8 lanes read 8 distinct 16-byte bank groups when the row stride is = ks (mod 8)
+        ld4 = ks >= 8 ? E4 : E4 + ((ks - E4 % 8) + 8) % 8;
+        smem = static_cast<size_t>(HW) * ld4 * 16 + static_cast<size_t>(tt) * E4 * 16 +
+               static_cast<size_t>(tt) * HW * 4 + static_cast<size_t>(tt) * 12 + 8;
+        if (smem <= static_cast<size_t>(pl.max_smem)) break;
+    }
+    pl.tt = tt; pl.ks = ks; pl.ld4 = ld4; pl.smem = smem;
+    return CVCL_OK;
+}
+
 }  // namespace
 
 extern "C" {
@@ -249,41 +285,52 @@ int cvcl_spatial_max_scores_f32(const float* img, const float* tok, const int64_
     CVCL_REQUIRE(n_way == 0 || txt_index || M / n_way <= C,
                  "spatial_max_scores_f32: %d trials without txt_index need as many labels (C=%d)", M / n_way, C);
     if (M == 0) return CVCL_OK;
-    const int E4 = E / 4;
-    // token rows per chunk: every row a label needs in one chunk where possible, at most 4 rows per work item and
-    // 256 work items per block
-    const int rows_wanted = n_way > 0 ? L : (C * L < 64 ? C * L : 64);
-    int tt = (rows_wanted + 3) / 4 * 4;
-    const int tt_cap = 4 * (256 / HW) < 64 ? 4 * (256 / HW) : 64;
-    if (tt > tt_cap) tt = tt_cap;
-    int max_smem = 0, dev = 0;
-    CVCL_CHECK_CUDA(cudaGetDevice(&dev));
-    CVCL_CHECK_CUDA(cudaDeviceGetAttribute(&max_smem, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev));
-    int ks = 0, ld4 = 0;
-    size_t smem = 0;
-    for (;; tt -= 4) {
-        CVCL_REQUIRE(tt >= 4, "spatial_max_scores_f32: the %d x %d image block does not fit in shared memory", HW, E);
-        const int items = (tt / 4) * HW;
-        ks = 1;
-        while (ks < 32 && 2 * ks * items <= 256 && E4 % (2 * ks) == 0) ks *= 2;
-        // quarter-warps of 8 lanes read 8 distinct 16-byte bank groups when the row stride is = ks (mod 8)
-        ld4 = ks >= 8 ? E4 : E4 + ((ks - E4 % 8) + 8) % 8;
-        smem = static_cast<size_t>(HW) * ld4 * 16 + static_cast<size_t>(tt) * E4 * 16 +
-               static_cast<size_t>(tt) * HW * 4 + static_cast<size_t>(tt) * 12 + 8;
-        if (smem <= static_cast<size_t>(max_smem)) break;
-    }
+    SpatialPlan pl{};
+    const int rc = spatial_plan("spatial_max_scores_f32", HW, E, n_way > 0 ? L : (C * L < 64 ? C * L : 64), pl);
+    if (rc != CVCL_OK) return rc;
     static thread_local unsigned attr_mask = 0;         // per device: function attributes live in the device's context
-    const int attr_dev = dev >= 0 && dev < 32 ? dev : 0;
+    const int attr_dev = pl.dev >= 0 && pl.dev < 32 ? pl.dev : 0;
     if (!((attr_mask >> attr_dev) & 1u)) {
         CVCL_CHECK_CUDA(cudaFuncSetAttribute(spatial_max_scores_f32_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                             max_smem));
+                                             pl.max_smem));
         attr_mask |= 1u << attr_dev;
     }
     SpatialMaxScoreParams p{};
     p.img = img; p.tok = tok; p.lens = reinterpret_cast<const long long*>(lens); p.txt_index = txt_index;
-    p.M = M; p.HW = HW; p.E = E; p.C = C; p.L = L; p.n_way = n_way; p.tt = tt; p.ks = ks; p.ld4 = ld4;
+    p.M = M; p.HW = HW; p.E = E; p.C = C; p.L = L; p.n_way = n_way; p.tt = pl.tt; p.ks = pl.ks; p.ld4 = pl.ld4;
     p.scale = expf(log_scale); p.out = out;
-    CVCL_CHECK_CUDA(launch_pdl(spatial_max_scores_f32_kernel, dim3(M), dim3(256), smem, as_stream(stream), p));
+    CVCL_CHECK_CUDA(launch_pdl(spatial_max_scores_f32_kernel, dim3(M), dim3(256), pl.smem, as_stream(stream), p));
+    count_launch();
+    return CVCL_OK;
+}
+
+int cvcl_spatial_attention_f32(const float* img, const float* tok, const int64_t* lens, const int* txt_index, int M,
+                               int HW, int E, int C, int L, float* token_maps, float* utt_maps, int* token_argmax,
+                               void* stream) {
+    CVCL_REQUIRE(img && tok && lens && utt_maps, "spatial_attention_f32: null pointer");
+    CVCL_REQUIRE(M >= 0 && C > 0 && L > 0, "spatial_attention_f32: bad shape M=%d C=%d L=%d", M, C, L);
+    CVCL_REQUIRE(HW > 0 && HW <= 256, "spatial_attention_f32: HW=%d must be in [1, 256]", HW);
+    CVCL_REQUIRE(E > 0 && E % 4 == 0, "spatial_attention_f32: E=%d must be a multiple of 4", E);
+    CVCL_REQUIRE(((reinterpret_cast<uintptr_t>(img) | reinterpret_cast<uintptr_t>(tok)) & 15) == 0,
+                 "spatial_attention_f32: 16-byte alignment required");
+    CVCL_REQUIRE(txt_index || M <= C, "spatial_attention_f32: %d images without txt_index need as many labels (C=%d)",
+                 M, C);
+    if (M == 0) return CVCL_OK;
+    SpatialPlan pl{};
+    const int rc = spatial_plan("spatial_attention_f32", HW, E, L, pl);     // the plan of the scores' trial mode
+    if (rc != CVCL_OK) return rc;
+    static thread_local unsigned attr_mask = 0;         // per device: function attributes live in the device's context
+    const int attr_dev = pl.dev >= 0 && pl.dev < 32 ? pl.dev : 0;
+    if (!((attr_mask >> attr_dev) & 1u)) {
+        CVCL_CHECK_CUDA(cudaFuncSetAttribute(spatial_attention_f32_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                             pl.max_smem));
+        attr_mask |= 1u << attr_dev;
+    }
+    SpatialAttentionParams p{};
+    p.img = img; p.tok = tok; p.lens = reinterpret_cast<const long long*>(lens); p.txt_index = txt_index;
+    p.M = M; p.HW = HW; p.E = E; p.C = C; p.L = L; p.tt = pl.tt; p.ks = pl.ks; p.ld4 = pl.ld4;
+    p.token_maps = token_maps; p.utt_maps = utt_maps; p.token_argmax = token_argmax;
+    CVCL_CHECK_CUDA(launch_pdl(spatial_attention_f32_kernel, dim3(M), dim3(256), pl.smem, as_stream(stream), p));
     count_launch();
     return CVCL_OK;
 }

@@ -933,6 +933,72 @@ __global__ void __launch_bounds__(256) conv1x1_f32_kernel(const float* x, const 
     }
 }
 
+// Shared by spatial_max_scores_f32_kernel and spatial_attention_f32_kernel.  Both run on the launch plan of
+// spatial_plan (cvcl_b200.cu), so the dots they compute are the same bits.
+//
+// Stages the image's HW x E block into shared memory (row stride ld4 float4, padded so the quarter-warps of a
+// k-split read distinct banks), four 16-byte loads in flight per thread.
+__device__ __forceinline__ void spatial_stage_image(float4* img_s, const float4* src, int HW, int E4, int ld4,
+                                                    int tid) {
+    const int n4 = HW * E4;
+    for (int i0 = tid; i0 < n4; i0 += 4 * 256) {
+        float4 v[4];
+#pragma unroll
+        for (int u = 0; u < 4; ++u) {
+            const int i = i0 + u * 256;
+            if (i < n4) v[u] = __ldcs(src + i);
+        }
+#pragma unroll
+        for (int u = 0; u < 4; ++u) {
+            const int i = i0 + u * 256;
+            if (i < n4) { const int q = i / E4; img_s[q * ld4 + (i - q * E4)] = v[u]; }
+        }
+    }
+}
+
+// dots[r * HW + q] = <img_s[q], tok_s[r]> for the token rows of a chunk.  Thread (w, ks) = (tid / KS, tid % KS)
+// owns work item w = (group of 4 token rows, location q) of the first n_items and the k-slice ks (float4 indices
+// ks, ks + KS, ...): four fp32 FMA chains, then a fixed butterfly over the KS lanes of the item.  Every thread of the
+// block calls it.
+__device__ __forceinline__ void spatial_chunk_dots(const float4* img_s, const float4* tok_s, float* dots, int n_items,
+                                                   int HW, int E4, int ld4, int KS, int w, int ks) {
+    float acc[4] = {0.f, 0.f, 0.f, 0.f};
+    const int g = w / HW, q = w - g * HW;
+    if (w < n_items) {
+        const float4* xr = img_s + q * ld4;
+        const float4* t0 = tok_s + static_cast<size_t>(g) * 4 * E4;
+#pragma unroll 4                     // explicit: left to the compiler, the unroll depends on the calling kernel
+        for (int i = ks; i < E4; i += KS) {
+            const float4 xv = xr[i];
+#pragma unroll
+            for (int r = 0; r < 4; ++r) {
+                const float4 tv = t0[r * E4 + i];
+                acc[r] = fmaf(xv.x, tv.x, acc[r]); acc[r] = fmaf(xv.y, tv.y, acc[r]);
+                acc[r] = fmaf(xv.z, tv.z, acc[r]); acc[r] = fmaf(xv.w, tv.w, acc[r]);
+            }
+        }
+    }
+    for (int o = KS >> 1; o > 0; o >>= 1)
+#pragma unroll
+        for (int r = 0; r < 4; ++r) acc[r] += __shfl_xor_sync(0xffffffffu, acc[r], o);
+    if (w < n_items && ks == 0)
+#pragma unroll
+        for (int r = 0; r < 4; ++r) dots[(g * 4 + r) * HW + q] = acc[r];
+}
+
+// Maximum of a row of HW dots and the first location attaining it; a NaN location wins and stays (torch.amax,
+// torch.argmax).
+__device__ __forceinline__ float spatial_row_max(const float* row, int HW, int& arg) {
+    float mx = -INFINITY;
+    int a = 0;
+    for (int q = 0; q < HW; ++q) {
+        const float v = row[q];
+        if (mx == mx && !(v <= mx)) { mx = v; a = q; }
+    }
+    arg = a;
+    return mx;
+}
+
 // Spatial "max" score in fp32 for evaluation (multimodal.py:771-780):
 //   logit[m, c] = scale * (sum_{l < len[c]} max_p <img[m,p,:], tok[c,l,:]>) / len[c]
 // Rows of a label past its length are <pad> rows, zero after the per-token normalisation, and add exactly 0 in the
@@ -971,21 +1037,8 @@ __global__ void __launch_bounds__(256) spatial_max_scores_f32_kernel(const Spati
     int* slot_l = slot_c + p.tt;                                                 // [tt] position (-1: last of label)
     int* ctrl = slot_l + p.tt;                                                   // [0] rows in the chunk, [1] done
 
-    const float4* src = reinterpret_cast<const float4*>(p.img) + static_cast<size_t>(m) * p.HW * E4;
-    const int n4 = p.HW * E4;
-    for (int i0 = tid; i0 < n4; i0 += 4 * 256) {                                 // 4 loads in flight per thread
-        float4 v[4];
-#pragma unroll
-        for (int u = 0; u < 4; ++u) {
-            const int i = i0 + u * 256;
-            if (i < n4) v[u] = __ldcs(src + i);
-        }
-#pragma unroll
-        for (int u = 0; u < 4; ++u) {
-            const int i = i0 + u * 256;
-            if (i < n4) { const int q = i / E4; img_s[q * p.ld4 + (i - q * E4)] = v[u]; }
-        }
-    }
+    spatial_stage_image(img_s, reinterpret_cast<const float4*>(p.img) + static_cast<size_t>(m) * p.HW * E4, p.HW, E4,
+                        p.ld4, tid);
 
     int c_cur = 0, c_end = p.C, l_cur = 0;           // thread 0's cursor over (label, position)
     float run = 0.f;                                 // thread 0's running sum of the current label
@@ -1037,38 +1090,11 @@ __global__ void __launch_bounds__(256) spatial_max_scores_f32_kernel(const Spati
             tok_s[i] = v;
         }
         __syncthreads();
-        const int n_items = ((nt + 3) >> 2) * p.HW;
-        {
-            float acc[4] = {0.f, 0.f, 0.f, 0.f};
-            const int g = w / p.HW, q = w - g * p.HW;
-            if (w < n_items) {
-                const float4* xr = img_s + q * p.ld4;
-                const float4* t0 = tok_s + static_cast<size_t>(g) * 4 * E4;
-                for (int i = ks; i < E4; i += p.ks) {
-                    const float4 xv = xr[i];
-#pragma unroll
-                    for (int r = 0; r < 4; ++r) {
-                        const float4 tv = t0[r * E4 + i];
-                        acc[r] = fmaf(xv.x, tv.x, acc[r]); acc[r] = fmaf(xv.y, tv.y, acc[r]);
-                        acc[r] = fmaf(xv.z, tv.z, acc[r]); acc[r] = fmaf(xv.w, tv.w, acc[r]);
-                    }
-                }
-            }
-            for (int o = p.ks >> 1; o > 0; o >>= 1)
-#pragma unroll
-                for (int r = 0; r < 4; ++r) acc[r] += __shfl_xor_sync(0xffffffffu, acc[r], o);
-            if (w < n_items && ks == 0)
-#pragma unroll
-                for (int r = 0; r < 4; ++r) dots[(g * 4 + r) * p.HW + q] = acc[r];
-        }
+        spatial_chunk_dots(img_s, tok_s, dots, ((nt + 3) >> 2) * p.HW, p.HW, E4, p.ld4, p.ks, w, ks);
         __syncthreads();
         if (tid < nt) {
-            float mx = -INFINITY;
-            for (int q = 0; q < p.HW; ++q) {
-                const float v = dots[tid * p.HW + q];
-                if (mx == mx && !(v <= mx)) mx = v;                  // a NaN location wins and stays
-            }
-            tmax[tid] = mx;
+            int arg;
+            tmax[tid] = spatial_row_max(dots + tid * p.HW, p.HW, arg);
         }
         __syncthreads();
         if (tid == 0) {
@@ -1083,6 +1109,82 @@ __global__ void __launch_bounds__(256) spatial_max_scores_f32_kernel(const Spati
             }
         }
     }
+}
+
+// Text-to-location attention maps in fp32: the per-location terms of the spatial similarity (multimodal.py:771-780)
+// before its reductions.  Image m is paired with label c = txt_index[m] (identity when null):
+//   token_maps[m, l, p] = <img[m,p,:], tok[c,l,:]>                           l < len[c]; exactly 0 for l >= len[c]
+//   utt_maps[m, p]      = (sum_{l < len[c]} token_maps[m, l, p]) / len[c]    sum in position order; len 0 gives NaN
+//   token_argmax[m, l]  = first p attaining max_p token_maps[m, l, p] (a NaN wins); -1 for l >= len[c]
+// One block per image on the launch plan and the helpers of spatial_max_scores_f32_kernel: the image block is
+// staged once, the label's token rows follow in chunks of tt rows, and the dots of a chunk are the ones that kernel
+// takes the maximum of, bit for bit.  A chunk's token-map rows are one contiguous run of nt * HW floats, written
+// from the dots tile with coalesced stores.  Thread q < HW keeps the running sum of location q across chunks.
+// A label index outside [0, C) gives NaN maps and arg-max -1.  No atomics: a replay is bit-identical.
+struct SpatialAttentionParams {
+    const float* img;          // [M, HW, E] fp32, normalised location features (NHWC rows)
+    const float* tok;          // [C, L, E]  fp32 per-token text features
+    const long long* lens;     // [C]
+    const int* txt_index;      // [M] (nullable)
+    int M, HW, E, C, L;
+    int tt, ks, ld4;           // launch plan, as SpatialMaxScoreParams
+    float* token_maps;         // [M, L, HW] (nullable)
+    float* utt_maps;           // [M, HW]
+    int* token_argmax;         // [M, L] (nullable)
+};
+
+__global__ void __launch_bounds__(256) spatial_attention_f32_kernel(const SpatialAttentionParams p) {
+    extern __shared__ __align__(16) unsigned char sat_smem[];
+    ptx::pdl_launch_dependents(); ptx::pdl_wait();
+    const int m = blockIdx.x;
+    const int tid = threadIdx.x;
+    const int E4 = p.E >> 2;
+    float4* img_s = reinterpret_cast<float4*>(sat_smem);                         // [HW][ld4]
+    float4* tok_s = img_s + static_cast<size_t>(p.HW) * p.ld4;                   // [tt][E4]
+    float* dots = reinterpret_cast<float*>(tok_s + static_cast<size_t>(p.tt) * E4);   // [tt][HW]
+    float* tmap = p.token_maps ? p.token_maps + static_cast<size_t>(m) * p.L * p.HW : nullptr;
+    int* targ = p.token_argmax ? p.token_argmax + static_cast<size_t>(m) * p.L : nullptr;
+    float* umap = p.utt_maps + static_cast<size_t>(m) * p.HW;
+
+    const int c = p.txt_index ? __ldg(p.txt_index + m) : m;
+    if (c < 0 || c >= p.C) {
+        const float nan = __int_as_float(0x7fffffff);
+        if (tmap) for (int i = tid; i < p.L * p.HW; i += 256) tmap[i] = nan;
+        if (targ) for (int l = tid; l < p.L; l += 256) targ[l] = -1;
+        for (int q = tid; q < p.HW; q += 256) umap[q] = nan;
+        return;
+    }
+    spatial_stage_image(img_s, reinterpret_cast<const float4*>(p.img) + static_cast<size_t>(m) * p.HW * E4, p.HW, E4,
+                        p.ld4, tid);
+    const long long len = __ldg(p.lens + c);
+    const int n = static_cast<int>(len < 0 ? 0 : (len > p.L ? p.L : len));
+    const float4* trows = reinterpret_cast<const float4*>(p.tok) + static_cast<size_t>(c) * p.L * E4;
+    const int ks = tid & (p.ks - 1);
+    const int w = tid / p.ks;
+    float run = 0.f;                                 // thread q < HW: sum over the label's tokens at location q
+    for (int l0 = 0; l0 < n; l0 += p.tt) {
+        const int nt = n - l0 < p.tt ? n - l0 : p.tt;
+        __syncthreads();                             // previous chunk consumed (and the image block stored)
+        for (int i = tid; i < p.tt * E4; i += 256)
+            tok_s[i] = i < nt * E4 ? __ldg(trows + static_cast<size_t>(l0) * E4 + i) : make_float4(0.f, 0.f, 0.f, 0.f);
+        __syncthreads();
+        spatial_chunk_dots(img_s, tok_s, dots, ((nt + 3) >> 2) * p.HW, p.HW, E4, p.ld4, p.ks, w, ks);
+        __syncthreads();
+        if (tmap)
+            for (int i = tid; i < nt * p.HW; i += 256) tmap[static_cast<size_t>(l0) * p.HW + i] = dots[i];
+        if (tid < p.HW)
+            for (int r = 0; r < nt; ++r) run += dots[r * p.HW + tid];
+        if (targ && tid < nt) {
+            int arg;
+            spatial_row_max(dots + tid * p.HW, p.HW, arg);
+            targ[l0 + tid] = arg;
+        }
+    }
+    if (tmap)
+        for (int i = tid; i < (p.L - n) * p.HW; i += 256) tmap[static_cast<size_t>(n) * p.HW + i] = 0.f;
+    if (targ)
+        for (int l = n + tid; l < p.L; l += 256) targ[l] = -1;
+    if (tid < p.HW) umap[tid] = run / static_cast<float>(len);
 }
 
 // g[n,:] from u[n,:] and target[n,:]: one warp per image (F.normalize backward, eps 1e-12)

@@ -9,6 +9,8 @@ names, argument meaning, return tuples, error behaviour) for the hot path only:
       .forward(image, text, text_length, return_image_features=False,
                return_text_outputs=False)                                     multimodal.py:746-794
       .calculate_contrastive_loss(x, y, y_len) -> 10-tuple                    multimodal.py:796-822
+      .spatial_attention_maps(image, text, text_length, text_index=None, out_size=None)
+                                      -> (utterance, token maps, arg-max)     per-location terms of :771-780
 
 `vision_encoder` / `text_encoder` may be the REFERENCE's own VisionEncoder / TextEncoder objects
 (that is the drop-in case: replace the MultiModalModel import in multimodal_lit.py) or the minimal
@@ -293,6 +295,37 @@ class MultiModalModel(nn.Module):
         if self.embedding_type == "spatial":
             feat = feat.permute(0, 3, 1, 2)                 # [B,E,H,W] view, as the reference returns
         return feat, fmap
+
+    @torch.no_grad()
+    def spatial_attention_maps(self, image, text, text_length, text_index=None, out_size=None):
+        """Text-to-location attention maps of a spatial-embedding model, fp32 end to end.  The reference has no
+        function that returns them: they are the per-location terms of its own similarity (multimodal.py:771-780)
+        before the max / mean reductions, so no Grad-CAM is needed to see where a word lands.
+        image: what encode_image takes (images, or with trunk="pooled" the layer4 maps [N, 2048, h, w]); the head
+        runs in fp32 (ops.conv1x1_f32).  text / text_length [C, L] / [C] token rows; text_index [N] picks the row of
+        every image (None: C >= N, image n uses row n).
+        -> (utterance maps [N, 1, h, w] = sum_{l < len} token maps / len, resized to out_size = (H, W) or H with
+        F.interpolate(bicubic, align_corners=False) semantics when given (the layout attention_maps.gradCAM returns);
+        token maps [N, L, h, w] = <location, token> at feature resolution, exactly 0 past the length; token arg-max
+        int32 [N, L] = first location (p = y * w + x) of each token's maximum, the one the sim="max" score takes,
+        -1 past the length).  Match units (cosines when normalize_features), no temperature."""
+        if self.embedding_type != "spatial":
+            raise NotImplementedError("spatial_attention_maps needs embedding_type='spatial'; for a flat model use "
+                                      "attention_maps.gradCAM")
+        boundary, _ = self._trunk(image)
+        if boundary.dim() != 4:
+            raise ValueError("spatial_attention_maps: the trunk gave %s, not a layer4 map [N, C, h, w]"
+                             % (tuple(boundary.shape),))
+        w, b = self._head()
+        N, _, h, wd = boundary.shape
+        rows = ops.conv1x1_f32(boundary, w, b).view(N, h * wd, -1)
+        tok, _ = ops.text_features_spatial(text, text_length, self.text_embed.embedding.weight, self.normalize_features)
+        maps, utt, arg = ops.spatial_attention_f32(rows, tok, text_length, text_index, bool(self.normalize_features))
+        utt = utt.view(N, 1, h, wd)
+        if out_size is not None:
+            H, W = (out_size, out_size) if isinstance(out_size, int) else out_size
+            utt = ops.bicubic_upsample(utt, int(H), int(W))
+        return utt, maps.view(N, -1, h, wd), arg
 
     def encode_text(self, text, text_length):
         _check_dropout(self.text_embed)

@@ -136,6 +136,9 @@ class MultiModalLitModel(_Base):
         text_features, _ = self.model.encode_text(y, y_len)
         return text_features
 
+    def attention_maps(self, image, text, text_length, text_index=None, out_size=None):
+        return self.model.spatial_attention_maps(image, text, text_length, text_index, out_size)
+
     def tokenize(self, texts):
         """multimodal_lit.py:161-190: [<sos>] + ids + [<eos>], truncated to 25, padded with 0."""
         max_seq_len = MAX_LEN_UTTERANCE

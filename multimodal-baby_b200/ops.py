@@ -15,6 +15,8 @@ Reference call sites replaced (paths relative to the reference repo):
   eval_nway         multimodal/multimodal_lit.py:466-511, eval.py:196-214
   conv1x1_f32, eval_nway_spatial, classify_ncat_spatial
                     the same evaluation for spatial embeddings (multimodal/multimodal.py:181-185, 757-787)
+  spatial_attention_f32
+                    the per-location terms of the spatial similarity, before its reductions (multimodal/multimodal.py:771-780)
 """
 from __future__ import annotations
 
@@ -1241,6 +1243,60 @@ def _(img, txt, lens, sim, normalize, log_scale, want_logits=True):
     N, C = img.shape[0], txt.shape[0]
     return (img.new_empty((N,), dtype=torch.int32),
             img.new_empty((N, C) if want_logits else (0,), dtype=torch.float32))
+
+
+@torch.library.custom_op(_NS + "::spatial_attention_f32", mutates_args=())
+def spatial_attention_f32(img: Tensor, tok: Tensor, lens: Tensor, text_index: Optional[Tensor], normalize: bool,
+                          want_tokens: bool = True) -> Tuple[Tensor, Tensor, Tensor]:
+    """Text-to-location attention maps of a spatial-embedding model in fp32 (cvcl_spatial_attention_f32): the
+    per-location terms of the spatial similarity (multimodal.py:771-780) before its max / mean reductions.  The
+    reference has no function that returns them; they are the summands of its own forward.
+    img [M, HW, E] head outputs before normalisation (NHWC rows), normalised per location when `normalize`;
+    tok [C, L, E] per-token text features (ops.text_features_spatial, normalised per token iff `normalize`), lens [C];
+    text_index [M] picks the label of every image (None: C >= M, image m uses label m).
+    -> (token_maps [M, L, HW] | empty, utt_maps [M, HW], token_argmax int32 [M, L] | empty), in match units:
+      token_maps[m, l, p] = <x[m, p], tok[c, l]> for l < len[c], exactly 0 past the length;
+      utt_maps[m, p] = sum_{l < len} token_maps[m, l, p] / len (len 0 gives NaN); its mean over p is the sim="mean"
+      match, and sum_l max_p token_maps[m, l, p] / len is the sim="max" match;
+      token_argmax[m, l] = first location of max_p token_maps[m, l, p] (a NaN wins), -1 past the length.
+    A text_index outside [0, C) gives NaN maps.  want_tokens=False returns only the utterance maps."""
+    if img.dim() != 3:
+        raise ValueError("spatial_attention_f32: img %s is not [M, HW, E]" % (tuple(img.shape),))
+    M, HW, E = img.shape
+    if tok.dim() != 3 or tok.shape[2] != E:
+        raise ValueError("spatial_attention_f32: tok %s is not per-token text features [C, L, %d]" % (tuple(tok.shape), E))
+    C, L, _ = tok.shape
+    if lens.dim() != 1 or lens.shape[0] != C:
+        raise ValueError("spatial_attention_f32: lens %s does not fit %d labels" % (tuple(lens.shape), C))
+    if text_index is not None:
+        if tuple(text_index.shape) != (M,):
+            raise ValueError("spatial_attention_f32: text_index %s does not fit %d images" % (tuple(text_index.shape), M))
+        text_index = text_index.to(torch.int32).contiguous()
+    elif C < M:
+        raise ValueError("spatial_attention_f32: %d images without text_index need as many labels (got %d)" % (M, C))
+    _need_cuda(img, tok, lens, text_index)
+    rows = _location_rows(img, normalize)
+    tok = _f32(tok)
+    lens = _i64(lens)
+    utt = torch.empty((M, HW), dtype=torch.float32, device=img.device)
+    if want_tokens:
+        maps = torch.empty((M, L, HW), dtype=torch.float32, device=img.device)
+        arg = torch.empty((M, L), dtype=torch.int32, device=img.device)
+    else:
+        maps = utt.new_empty((0,))
+        arg = utt.new_empty((0,), dtype=torch.int32)
+    _cabi.call("cvcl_spatial_attention_f32", _p(rows), _p(tok), _p(lens), _p(text_index), M, HW, E, C, L,
+               _p(maps) if want_tokens else None, _p(utt), _p(arg) if want_tokens else None, _stream())
+    return maps, utt, arg
+
+
+@spatial_attention_f32.register_fake
+def _(img, tok, lens, text_index, normalize, want_tokens=True):
+    M, HW, _ = img.shape
+    L = tok.shape[1]
+    return (img.new_empty((M, L, HW) if want_tokens else (0,), dtype=torch.float32),
+            img.new_empty((M, HW), dtype=torch.float32),
+            img.new_empty((M, L) if want_tokens else (0,), dtype=torch.int32))
 
 
 @torch.no_grad()
