@@ -193,6 +193,26 @@ __device__ __forceinline__ unsigned int ld_acquire_sys(const unsigned int* p) {
     return v;
 }
 
+// The spin of a grid barrier after its first 4096 failed probes (in practice a barrier completes long before):
+// the globaltimer is sampled every 4096 probes from here on, and a wait longer than timeout_ns stores `code` into
+// *fault and traps.  kSys: wait at system scope until the word has reached `target` as a wrapping epoch (cross-rank
+// flags, sharded instance only); else at GPU scope until the counter is >= target.  Out of line because a step never
+// gets here: inlined, this fault path sat in every barrier of the instruction stream that each launch fetches again
+// after the L2 flush between steps.
+template <bool kSys>
+__device__ __noinline__ void grid_wait_cold(const unsigned int* w, unsigned int target, unsigned long long timeout_ns,
+                                            int* fault, int code) {
+    const unsigned long long t0 = globaltimer_ns();
+    unsigned int it = 0;
+    while (kSys ? static_cast<int>(ld_acquire_sys(w) - target) < 0 : ld_acquire_gpu(w) < target) {
+        if ((++it & 4095u) == 0 && globaltimer_ns() - t0 > timeout_ns) {
+            if (fault) atomicExch(fault, code);
+            __threadfence_system();
+            __trap();
+        }
+    }
+}
+
 // xstage >= 0 (sharded runs; only the kSharded instance has this code): the barrier also spans the ranks.  Every
 // CTA fences its stores at system scope before it arrives; the LAST local arrival (it has seen all the others
 // through the counter) stores this launch's epoch into flag word [xstage][rank] of every peer, and every CTA then also waits until its own
@@ -215,7 +235,6 @@ CVCL_HELPER void grid_sync(const StepParams& p, int k, int xstage = -1, unsigned
         }
         prev = __shfl_sync(0xffffffffu, prev, 0);
         __syncwarp();                       // memory ordering lane 0 -> the signalling lanes (shfl alone gives none)
-        unsigned int it = 0; unsigned long long t0 = 0;
         if (cross) {
             const bool peer = lane < p.world && lane != p.rank;
             // the LAST local arrival has seen every other CTA's arrival (each behind that CTA's system-scope fence):
@@ -223,31 +242,24 @@ CVCL_HELPER void grid_sync(const StepParams& p, int k, int xstage = -1, unsigned
             if (prev == target - 1 && peer) st_release_sys(p.peer_flags[lane] + xstage * 8 + p.rank, epoch);
             if (peer) {
                 const unsigned int* w = p.peer_flags[p.rank] + xstage * 8 + lane;
+                unsigned int it = 0;
+#pragma unroll 1
                 while (static_cast<int>(ld_acquire_sys(w) - epoch) < 0) {
-                    if ((++it & 4095u) == 0) {
-                        const unsigned long long now = globaltimer_ns();
-                        if (t0 == 0) t0 = now;
-                        else if (now - t0 > p.xtimeout_ns) {      // a peer never reached this step
-                            if (p.fault) atomicExch(p.fault, 200 + 10 * xstage + lane);
-                            __threadfence_system();
-                            __trap();
-                        }
+                    if (++it == 4096u) {              // fault code 200 + 10 xstage + lane: a peer never reached this step
+                        grid_wait_cold<true>(w, epoch, p.xtimeout_ns, p.fault, 200 + 10 * xstage + lane);
+                        break;
                     }
                 }
             }
             __syncwarp();
-            it = 0; t0 = 0;
         }
         if (lane == 0) {
+            unsigned int it = 0;
+#pragma unroll 1
             while (ld_acquire_gpu(p.sync) < target) {
-                if ((++it & 4095u) == 0) {
-                    const unsigned long long now = globaltimer_ns();
-                    if (t0 == 0) t0 = now;
-                    else if (now - t0 > 2000000000ull) {              // 2 s: a CTA never arrived
-                        if (p.fault) atomicExch(p.fault, 100 + k);
-                        __threadfence_system();
-                        __trap();
-                    }
+                if (++it == 4096u) {                  // fault code 100 + k after 2 s: a CTA never arrived
+                    grid_wait_cold<false>(p.sync, target, 2000000000ull, p.fault, 100 + k);
+                    break;
                 }
             }
             fence_proxy_async_all();                                  // thread 0 = warp 0 lane 0 issues the TMA loads
@@ -338,6 +350,19 @@ CVCL_HELPER void stage_f32_cols(uint32_t tmem_row, int tc0, int sc0, int ncols, 
             swz_st16(stage, row, (sc0 + c + 4 * j) * 4, q);
         }
     }
+}
+
+// v[i] for a per-thread i in [0, 32): a select tree over the five bits of i, 31 selects (a 32-way compare / select
+// scan takes twice the instructions, and indexing v with i would put it in local memory)
+CVCL_HELPER float select32(const float (&v)[32], int i) {
+    float s[16];
+#pragma unroll
+    for (int q = 0; q < 16; ++q) s[q] = (i & 1) ? v[2 * q + 1] : v[2 * q];
+#pragma unroll
+    for (int b = 1; b < 5; ++b)
+#pragma unroll
+        for (int q = 0; q < (16 >> b); ++q) s[q] = ((i >> b) & 1) ? s[2 * q + 1] : s[2 * q];
+    return s[0];
 }
 
 // online merge of per-tile softmax partials (strict >: the first tile wins ties, as torch.argmax does);
@@ -453,6 +478,7 @@ flat_step_kernel(const __grid_constant__ StepMaps maps, const __grid_constant__ 
     const unsigned int xepoch = (kSharded && p.epoch) ? *reinterpret_cast<volatile unsigned int*>(p.epoch) + 1u : 0u;
 
     if (p.phase_limit == 100) {            // measurement: the cost of the grid barrier alone
+#pragma unroll 1                           // one barrier body in the instruction stream, not six
         for (int i = 0; i < 6; ++i) grid_sync<false, kSharded>(p, sync_k++);
         goto done;
     }
@@ -690,12 +716,7 @@ flat_step_kernel(const __grid_constant__ StepMaps maps, const __grid_constant__ 
                             for (int q = 31; q >= 0; --q) if (v[q] == cm) k = q;
                             arg = n + k;
                         }
-                        if (dcol >= n && dcol < n + 32 && m < M) {
-                            float dv = 0.f;
-#pragma unroll
-                            for (int q = 0; q < 32; ++q) if (n + q == dcol) dv = v[q];
-                            p.diag[z][m] = dv * scale;
-                        }
+                        if (dcol >= n && dcol < n + 32 && m < M) p.diag[z][m] = select32(v, dcol - n) * scale;
                         const float nm = fmaxf(mx, cm);
                         const float corr = exp2f((mx - nm) * sc2);
                         l *= corr; a *= corr;
@@ -817,11 +838,8 @@ flat_step_kernel(const __grid_constant__ StepMaps maps, const __grid_constant__ 
                         float v[32];
                         ptx::tmem_ld_32x32(tmem_row + 128 * j + c, v);
                         const int n = n0 + c;
-                        float dv = 0.f;
-                        if (dcol >= n && dcol < n + 32) {
-#pragma unroll
-                            for (int q = 0; q < 32; ++q) if (n + q == dcol) dv = v[q];
-                        }
+                        const bool has_diag = dcol >= n && dcol < n + 32;     // warp-uniform: one chunk per warp
+                        const float dv = has_diag ? select32(v, dcol - n) : 0.f;
                         float g[32];
 #pragma unroll
                         for (int q4 = 0; q4 < 8; ++q4) {
@@ -837,12 +855,10 @@ flat_step_kernel(const __grid_constant__ StepMaps maps, const __grid_constant__ 
                         }
                         // the diagonal stays in the bf16 operand; its rounded value goes to P4, which replaces it by the
                         // whole G_ii in fp32: w (P_row + P_col) and -2w nearly cancel when a pair is confident, and the
-                        // bf16 rounding of the first would be left as the whole gradient (warp-uniform: one chunk of the
-                        // diagonal tile per warp)
-                        if (dcol >= n && dcol < n + 32 && qs == 0 && m < M) {
-                            float gd = 0.f;
-#pragma unroll
-                            for (int q = 0; q < 32; ++q) if (n + q == dcol) gd = g[q];
+                        // bf16 rounding of the first would be left as the whole gradient.  G_ii is recomputed from dv by
+                        // the expression that gave g[dcol - n] above (the same float, without a second 32-way scan)
+                        if (has_diag && qs == 0 && m < M) {
+                            const float gd = exp2f(fmaf(dv, sc2, -lq)) + exp2f(fmaf(dv, sc2, -lk[128 * j + dcol - n0]));
                             p.gdiag[z][m] = __bfloat162float(__float2bfloat16_rn(gd));
                         }
                         ds = fmaf(-2.f * w, dv, ds);

@@ -4,7 +4,9 @@ Every phase of the step runs once per launch and the L2 flush between training s
 the instruction bytes a phase walks through are a cost of their own.  This disassembles the library with
 `nvdisasm --print-line-info-inline` (the library is built with -lineinfo), attributes each instruction to the line
 of the kernel body it was inlined into, and groups the lines by the phase markers of csrc/fused_step.cuh
-(`// ===... P<k>`, the final sums, the exit).  Runs on the CPU.
+(`// ===... P<k>`, the final sums, the exit).  The subroutines placed after the kernel body in its section (the
+compiler's slow paths, the `__noinline__` fault helpers) are counted as "out of line": a step does not walk through
+them.  Runs on the CPU.
 
     python tools/sass_phases.py [library] [--source fused_step.cuh] [--json]
 
@@ -73,16 +75,22 @@ def disassemble(lib, tmp):
 
 def count(text, lookup, src_name):
     """{kernel symbol: OrderedDict(phase -> instructions)}"""
-    out, cur, where = {}, None, None
+    out, cur, where, sub = {}, None, None, False
     for line in text.splitlines():
         if line.startswith("//----") and ".text." in line:
             sym = line.split(".text.", 1)[1].split()[0]
             cur = OrderedDict() if "flat_step_kernel" in sym else None
             if cur is not None:
                 out[sym] = cur
-            where = None
+            where, sub = None, False
             continue
         if cur is None:
+            continue
+        if "@function" in line and ".type" in line:
+            # the subroutines placed after the kernel body in its section (out-of-line helpers, the compiler's
+            # slow paths): never part of the phases, whatever line was seen last
+            sub = line.split()[1].split(",")[0] != sym
+            where = None
             continue
         if "//##" in line:
             # the outermost location of the inlining chain is the line of the kernel body
@@ -91,7 +99,7 @@ def count(text, lookup, src_name):
             where = lookup(int(n)) if os.path.basename(f) == src_name else None
             continue
         if INSN.match(line):
-            key = where or "out of line"
+            key = "out of line" if sub else (where or "out of line")
             cur[key] = cur.get(key, 0) + 1
     return out
 
