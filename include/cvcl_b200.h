@@ -111,6 +111,18 @@ int cvcl_normalize_rows_f32(const float* src, float* dst, long long M, int E, vo
 int cvcl_row_argmax_f32(const float* scores, long long ld, long long M, int N, int col0, int merge, float* best,
                         int* arg, void* stream);
 
+/* Cross-modal retrieval selection (image->text and text->image recall@K, median rank): for each of the M full query
+ * rows of scores [M,N] (leading dimension ld), row m being query q0 + m, orders the N keys as
+ * torch.sort(row, descending=True, stable=True) does (a NaN above every number, -0 == +0, equal values by ascending
+ * key index) and writes
+ *   topk_idx [M,k] int32 / topk_val [M,k] fp32   the first k keys of that order and their scores;
+ *   rank [M] int32                               the 0-based position of the query's first positive, -1 without one.
+ * Positives: with q_group [Nq] and k_group [N] (int64), the keys n with k_group[n] == q_group[q0 + m]; with both NULL
+ * (pair mode), the key n == q0 + m.  1 <= k <= min(64, N).  One block per row; the row is read once, and a second
+ * time only when the first positive lies outside the top-k.  No atomics on global data (a replay is bit-identical). */
+int cvcl_rank_topk_f32(const float* scores, long long ld, long long M, int N, long long q0, const int64_t* q_group,
+                       const int64_t* k_group, int k, int* topk_idx, float* topk_val, int* rank, void* stream);
+
 /* its backward: dst [B,HW,E] fp32 = g [B,E] broadcast over the locations (autograd of the sum, multimodal.py:765). */
 int cvcl_spatial_pool_bwd(const float* g, int B, int HW, int E, float* dst, void* stream);
 

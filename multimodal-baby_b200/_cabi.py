@@ -45,6 +45,7 @@ PROTOTYPES = {
     "cvcl_linear_f32": (c_int, [_P, _I, _P, _I, _P, _I, _I, _I, _P, _I, _P]),
     "cvcl_normalize_rows_f32": (c_int, [_P, _P, _L, _I, _P]),
     "cvcl_row_argmax_f32": (c_int, [_P, _L, _L, _I, _I, _I, _P, _P, _P]),
+    "cvcl_rank_topk_f32": (c_int, [_P, _L, _L, _I, _L, _P, _P, _I, _P, _P, _P, _P]),
     "cvcl_head_proj_norm_fwd": (c_int, [_P, _I, _P, _I, _P, _I, _I, _I, _I, _P, _I, _P, _I, _P, _P]),
     "cvcl_sim_workspace_bytes": (c_size_t, [_I, _I, _I, _I]),
     "cvcl_sim_infonce_fwd": (c_int, [_P, _P, _P, _P, _I, _I, _I, _I, _I, _I, _F, _I, _F, _P, _P, _P, _P,

@@ -355,6 +355,22 @@ int cvcl_row_argmax_f32(const float* scores, long long ld, long long M, int N, i
     return CVCL_OK;
 }
 
+int cvcl_rank_topk_f32(const float* scores, long long ld, long long M, int N, long long q0, const int64_t* q_group,
+                       const int64_t* k_group, int k, int* topk_idx, float* topk_val, int* rank, void* stream) {
+    CVCL_REQUIRE(scores && topk_idx && topk_val && rank, "rank_topk_f32: null pointer");
+    CVCL_REQUIRE(!q_group == !k_group, "rank_topk_f32: q_group and k_group are both given or both NULL");
+    CVCL_REQUIRE(M >= 0 && M <= 0x7fffffffLL && N > 0 && ld >= N && q0 >= 0,
+                 "rank_topk_f32: bad shape M=%lld N=%d ld=%lld q0=%lld", M, N, ld, q0);
+    CVCL_REQUIRE(k >= 1 && k <= kRankMaxK && k <= N, "rank_topk_f32: k=%d must be in [1, min(%d, N=%d)]", k,
+                 kRankMaxK, N);
+    if (M == 0) return CVCL_OK;
+    CVCL_CHECK_CUDA(launch_pdl(rank_topk_f32_kernel, dim3(static_cast<unsigned>(M)), dim3(kRankThreads), 0,
+                               as_stream(stream), scores, ld, N, q0, reinterpret_cast<const long long*>(q_group),
+                               reinterpret_cast<const long long*>(k_group), k, topk_idx, topk_val, rank));
+    count_launch();
+    return CVCL_OK;
+}
+
 int cvcl_spatial_pool_bwd(const float* g, int B, int HW, int E, float* dst, void* stream) {
     CVCL_REQUIRE(g && dst, "spatial_pool_bwd: null pointer");
     CVCL_REQUIRE(E > 0 && E % 4 == 0 && HW > 0, "spatial_pool_bwd: bad shape");

@@ -870,6 +870,130 @@ __global__ void __launch_bounds__(256) row_argmax_f32_kernel(const float* scores
     }
 }
 
+// Retrieval order of a query row, the order of torch.sort(row, descending=True, stable=True): a NaN ranks above every
+// number, -0 equals +0, and equal values (NaNs among themselves) go by ascending key index.  rank_key packs that order
+// into one integer that is larger for every earlier key: the order-preserving bits of the value in the high word (every
+// NaN all ones), the complement of the index in the low word.  The keys of a row are distinct and never 0.
+__device__ __forceinline__ unsigned long long rank_key(float v, int n) {
+    unsigned int u = 0xffffffffu;
+    if (v == v) {
+        u = __float_as_uint(v == 0.f ? 0.f : v);
+        u = (u & 0x80000000u) ? ~u : (u | 0x80000000u);
+    }
+    return (static_cast<unsigned long long>(u) << 32) | static_cast<unsigned int>(~n);
+}
+
+constexpr int kRankThreads = 256;
+constexpr int kRankPer = 4;                               // keys per thread per tile
+constexpr int kRankTile = kRankThreads * kRankPer;
+constexpr int kRankCap = 2 * kRankTile;                   // candidate list (keys)
+constexpr int kRankMaxK = 64;
+
+// Bitonic sort of buf[0, cnt) into descending key order, padded with 0 keys to a power of two (<= kRankCap).  Every
+// thread of the block calls it; it ends on a barrier.
+__device__ __forceinline__ void rank_sort_desc(unsigned long long* buf, int cnt, int tid) {
+    int n = 2;
+    while (n < cnt) n <<= 1;
+    for (int i = cnt + tid; i < n; i += kRankThreads) buf[i] = 0ull;
+    __syncthreads();
+    for (int size = 2; size <= n; size <<= 1)
+        for (int stride = size >> 1; stride > 0; stride >>= 1) {
+            for (int i = tid; i < (n >> 1); i += kRankThreads) {
+                const int lo = 2 * i - (i & (stride - 1)), hi = lo + stride;
+                const unsigned long long a = buf[lo], b = buf[hi];
+                if ((a < b) == ((lo & size) == 0)) { buf[lo] = b; buf[hi] = a; }
+            }
+            __syncthreads();
+        }
+}
+
+// Cross-modal retrieval selection, one block per query row of scores [M, N] (leading dimension ld; row m is global
+// query q0 + m).  Outputs for row m: the first k keys of the row's retrieval order (topk_idx [M, k], their scores
+// topk_val [M, k]) and rank[m], the 0-based position in that order of the row's first positive, -1 without one.  The
+// positives of query q are the keys n with k_group[n] == q_group[q], or the key n == q when the groups are null.
+// Pass 1 reads the row once: each 1024-key tile appends the keys above the running threshold to a shared candidate
+// list; when the list could overflow, it is sorted and cut to its first k, whose last key becomes the threshold.  The
+// same pass finds p*, the largest key among the positives.  The final list, sorted, gives the top-k; rank = the
+// number of keys above p*, counted in the top-k when p* is there and else by a second read of the row.  The list
+// order depends on the shared-memory append order, but the keys are distinct, so the sorted list does not: no data
+// atomics reach global memory and a replay is bit-identical.
+__global__ void __launch_bounds__(kRankThreads) rank_topk_f32_kernel(const float* scores, long long ld, int N,
+                                                                    long long q0, const long long* q_group,
+                                                                    const long long* k_group, int k, int* topk_idx,
+                                                                    float* topk_val, int* rank) {
+    __shared__ unsigned long long cand[kRankCap];
+    __shared__ unsigned long long red[kRankThreads / 32];
+    __shared__ unsigned long long s_thr;
+    __shared__ int s_cnt, s_sum[kRankThreads / 32];
+    ptx::pdl_launch_dependents(); ptx::pdl_wait();
+    const long long m = blockIdx.x;
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const float* row = scores + m * ld;
+    const long long q = q0 + m;
+    const long long g = q_group ? __ldg(q_group + q) : 0;
+    if (tid == 0) { s_cnt = 0; s_thr = 0ull; }
+    unsigned long long pos = 0ull;                        // largest positive key this thread has seen (0: none)
+    for (int base = 0; base < N; base += kRankTile) {
+        float v[kRankPer];
+#pragma unroll
+        for (int u = 0; u < kRankPer; ++u) {
+            const int n = base + u * kRankThreads + tid;
+            v[u] = n < N ? __ldg(row + n) : 0.f;
+        }
+        __syncthreads();                                  // the previous tile's appends are in
+        const int cnt = s_cnt;
+        __syncthreads();                                  // every thread has read cnt before this tile appends
+        if (cnt > kRankCap - kRankTile) {                 // block-uniform: cut the list to its first k
+            rank_sort_desc(cand, cnt, tid);
+            if (tid == 0) { s_cnt = k; s_thr = cand[k - 1]; }
+            __syncthreads();
+        }
+        const unsigned long long thr = s_thr;
+#pragma unroll
+        for (int u = 0; u < kRankPer; ++u) {
+            const int n = base + u * kRankThreads + tid;
+            if (n >= N) continue;
+            const unsigned long long key = rank_key(v[u], n);
+            const bool positive = q_group ? __ldg(k_group + n) == g : n == q;
+            if (positive && key > pos) pos = key;
+            if (key > thr) cand[atomicAdd(&s_cnt, 1)] = key;
+        }
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+        const unsigned long long other = __shfl_xor_sync(0xffffffffu, pos, o);
+        if (other > pos) pos = other;
+    }
+    if (lane == 0) red[warp] = pos;
+    __syncthreads();
+    const int cnt = s_cnt;                                // >= k: the threshold stays below the k-th key seen
+    for (int w = 0; w < kRankThreads / 32; ++w) pos = red[w] > pos ? red[w] : pos;
+    rank_sort_desc(cand, cnt, tid);
+    for (int i = tid; i < k; i += kRankThreads) {
+        const int n = static_cast<int>(~static_cast<unsigned int>(cand[i]));
+        topk_idx[m * k + i] = n;
+        topk_val[m * k + i] = __ldg(row + n);
+    }
+    if (pos == 0ull) {                                    // no positive
+        if (tid == 0) rank[m] = -1;
+        return;
+    }
+    int above = 0;
+    if (pos >= cand[k - 1]) {                             // p* is in the top-k
+        for (int i = tid; i < k; i += kRankThreads) above += cand[i] > pos;
+    } else {                                              // second read of the row
+        for (int n = tid; n < N; n += kRankThreads) above += rank_key(__ldg(row + n), n) > pos;
+    }
+    above = __reduce_add_sync(0xffffffffu, above);
+    if (lane == 0) s_sum[warp] = above;
+    __syncthreads();
+    if (tid == 0) {
+        int r = 0;
+        for (int w = 0; w < kRankThreads / 32; ++w) r += s_sum[w];
+        rank[m] = r;
+    }
+}
+
 // out[b*HW + p, e] = bias[e] + sum_k W[e,k] x[b,k,p]: the spatial 1x1-conv head in fp32 (reference Conv2d(2048, E, 1),
 // multimodal.py:181-185), reading the layer4 map x [B,K,HW] in the NCHW layout the trunk emits and writing NHWC rows.
 // Same tiling and fp32 FMA order as linear_f32_kernel (64 x 64 tile, 4 x 4 per thread, 16-deep k slabs); only the

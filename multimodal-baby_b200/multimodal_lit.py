@@ -11,6 +11,7 @@ Keeps the caller-facing API of the reference's Lightning wrapper that touches th
       .joint_loss_epoch_end / *_epoch_end  (example-weighted epoch metrics)      :376-444, :450-541
       .configure_optimizers()                                                    :112-128
       .evaluate_trials(...)  batched replacement of the per-trial loop of eval.py:175-266
+      .evaluate_retrieval(...)  image->text / text->image top-K, ranks and recall@K over a held-out split
 
 pytorch_lightning is optional (absent in this image): the class derives from
 `pl.LightningModule` when importable, else from `nn.Module` with no-op `log` /
@@ -288,6 +289,48 @@ class MultiModalLitModel(_Base):
             w, b = m._head()
             feats = ops.linear_f32(feats, w, b)
         return ops.classify_ncat(feats, txt, bool(m.normalize_features), s, want_logits)
+
+    @torch.no_grad()
+    def evaluate_retrieval(self, frame_features, text_ids, text_lens, frame_group=None, text_group=None, k=10,
+                           recall_at=(1, 5, 10), from_trunk_boundary=True, block_bytes=1 << 30):
+        """Image->text and text->image retrieval over a held-out split: for every frame, where its utterances rank
+        among all N_txt utterances, and for every utterance, where its frames rank among all N_img frames.
+        frame_features as classify_frames takes them ([N_img, 2048] trunk-boundary rows or [N_img, E] head outputs;
+        spatial models [N_img, 2048, H, W] layer4 maps or [N_img, E, H, W] head outputs); text_ids / text_lens
+        [N_txt, L] / [N_txt].  The scores are the fp32 values classify_frames takes its arg-max of.  Without groups
+        frame i and text i are the pair (N_img == N_txt); with frame_group [N_img] / text_group [N_txt] (int64) every
+        text of a frame's group is a positive of it and the other way round: give repeated utterances one id, or use
+        the category of each frame with the category labels as the texts.  Exact: keys ordered as
+        torch.sort(descending=True, stable=True) orders them, 1 <= k <= min(64, N_img, N_txt).  The score blocks
+        stay under block_bytes.  -> {"image_to_text": d, "text_to_image": d} with d holding "topk", "logits", "rank",
+        "recall" {K: R@K}, "median_rank", "mean_rank", "n_queries" (see ops.retrieval_f32)."""
+        m = self.model
+        w, b = m._head()
+        if text_ids.dim() != 2 or tuple(text_lens.shape) != (text_ids.shape[0],):
+            raise ValueError("evaluate_retrieval: text_ids %s / text_lens %s are not [N_txt, L] / [N_txt]"
+                             % (tuple(text_ids.shape), tuple(text_lens.shape)))
+        spatial = m.embedding_type == "spatial"
+        chans = w.shape[1] if from_trunk_boundary else w.shape[0]
+        if frame_features.dim() != (4 if spatial else 2) or frame_features.shape[1] != chans:
+            raise ValueError("evaluate_retrieval: a %s model takes %s of shape [N, %d%s], got %s"
+                             % ("spatial" if spatial else "flat", "head outputs" if not from_trunk_boundary else
+                                "layer4 maps" if spatial else "trunk-boundary rows", chans, ", H, W" if spatial else "",
+                                tuple(frame_features.shape)))
+        recall_at = tuple(recall_at)
+        ops.check_retrieval_args(frame_features.shape[0], text_ids.shape[0], frame_group, text_group, k, recall_at,
+                                 block_bytes, "evaluate_retrieval")
+        s = ops._scalar(m.logit_neg_log_temperature)
+        if spatial:
+            img = self._spatial_head_outputs(frame_features, (), from_trunk_boundary, "evaluate_retrieval")
+            txt = self._spatial_text(text_ids, text_lens, img.shape[1])
+            return ops.retrieval_f32(img, txt, text_lens, m.sim, bool(m.normalize_features), s, frame_group,
+                                     text_group, k, recall_at, block_bytes)
+        txt = ops.text_features_flat(text_ids, text_lens, m.text_embed.embedding.weight, normalize=False)
+        feats = frame_features.float()
+        if from_trunk_boundary:
+            feats = ops.linear_f32(feats, w, b)
+        return ops.retrieval_f32(feats, txt, None, "flat", bool(m.normalize_features), s, frame_group, text_group, k,
+                                 recall_at, block_bytes)
 
     def _spatial_head_outputs(self, x, lead, from_trunk_boundary, who):
         """[N, *lead, channels, H, W] -> head outputs before normalisation as NHWC rows [N*prod(lead), H*W, E]:

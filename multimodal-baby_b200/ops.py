@@ -17,6 +17,8 @@ Reference call sites replaced (paths relative to the reference repo):
                     the same evaluation for spatial embeddings (multimodal/multimodal.py:181-185, 757-787)
   spatial_attention_f32
                     the per-location terms of the spatial similarity, before its reductions (multimodal/multimodal.py:771-780)
+  retrieval_f32     image->text / text->image retrieval (top-K, rank of the first positive, recall@K) on the
+                    evaluation scores above
 """
 from __future__ import annotations
 
@@ -1315,6 +1317,144 @@ def cosine_nearest(queries: Tensor, keys: Tensor, chunk: int = 16384) -> Tuple[T
         _cabi.call("cvcl_row_argmax_f32", _p(scores), scores.shape[1], Nq, scores.shape[1], c0, int(c0 > 0),
                    _p(best), _p(arg), _stream())
     return best, arg
+
+
+# ----------------------------------------------------------------------------------------
+# cross-modal retrieval: exact top-K, ranks and recall@K in both directions
+# ----------------------------------------------------------------------------------------
+RETRIEVAL_MAX_K = 64
+
+
+def check_retrieval_args(n_img: int, n_txt: int, frame_group: Optional[Tensor], text_group: Optional[Tensor],
+                         k: int, recall_at, block_bytes: int, who: str = "retrieval_f32"):
+    """The argument checks of retrieval_f32, raised as ValueError before any device work."""
+    if n_img < 1 or n_txt < 1:
+        raise ValueError("%s: needs at least one frame and one text (got %d and %d)" % (who, n_img, n_txt))
+    if (frame_group is None) != (text_group is None):
+        raise ValueError("%s: frame_group and text_group are given together or not at all" % who)
+    if frame_group is None:
+        if n_img != n_txt:
+            raise ValueError("%s: pair mode (no groups) pairs frame i with text i and needs as many frames as texts "
+                             "(got %d and %d)" % (who, n_img, n_txt))
+    else:
+        for name, grp, n in (("frame_group", frame_group, n_img), ("text_group", text_group, n_txt)):
+            if grp.dtype != torch.int64 or tuple(grp.shape) != (n,):
+                raise ValueError("%s: %s must be int64 [%d], got %s %s" % (who, name, n, grp.dtype, tuple(grp.shape)))
+    kmax = min(RETRIEVAL_MAX_K, n_img, n_txt)
+    if isinstance(k, bool) or not isinstance(k, int) or not 1 <= k <= kmax:
+        raise ValueError("%s: k=%r must be an int in [1, min(%d, N_img, N_txt)] = [1, %d]"
+                         % (who, k, RETRIEVAL_MAX_K, kmax))
+    if any(isinstance(K, bool) or not isinstance(K, int) or K < 1 for K in recall_at):
+        raise ValueError("%s: recall_at=%r must hold positive ints" % (who, tuple(recall_at)))
+    if isinstance(block_bytes, bool) or not isinstance(block_bytes, int) or block_bytes < 1:
+        raise ValueError("%s: block_bytes=%r must be a positive int" % (who, block_bytes))
+
+
+def _row_blocks(n: int, rows: int, min_rows: int = 1):
+    """[q0, q1) blocks of `rows` query rows covering [0, n), every block at least min(min_rows, n) rows long (a
+    short tail joins the block before it)."""
+    rows = max(rows, min_rows)
+    starts = list(range(0, n, rows))
+    if len(starts) > 1 and n - starts[-1] < min_rows:
+        starts.pop()
+    return list(zip(starts, starts[1:] + [n]))
+
+
+def _retrieval_direction(score_block, n_q: int, n_k: int, q_group, k_group, k: int, scale: Optional[float],
+                         block_bytes: int, min_rows: int, dev) -> Tuple[Tensor, Tensor, Tensor]:
+    """The query rows in blocks of fp32 scores under block_bytes, each block ranked by cvcl_rank_topk_f32.
+    -> (topk, logits = scale * gathered scores (the scores themselves when scale is None), rank)."""
+    topk = torch.empty((n_q, k), dtype=torch.int32, device=dev)
+    val = torch.empty((n_q, k), dtype=torch.float32, device=dev)
+    rank = torch.empty((n_q,), dtype=torch.int32, device=dev)
+    for q0, q1 in _row_blocks(n_q, max(1, block_bytes // (4 * n_k)), min_rows):
+        s = score_block(q0, q1)
+        _cabi.call("cvcl_rank_topk_f32", _p(s), n_k, q1 - q0, n_k, q0, _p(q_group), _p(k_group), k,
+                   _p(topk[q0:]), _p(val[q0:]), _p(rank[q0:]), _stream())
+        del s
+    return topk, (val if scale is None else val * scale), rank
+
+
+def _retrieval_metrics(rank: Tensor, recall_at) -> Tensor:
+    """[recall@K..., mean rank, median rank, n_queries] fp64 on the device, over the queries with a positive;
+    ranks 1-based, the median the lower middle value (torch.median)."""
+    has = rank >= 0
+    n = has.sum()
+    nf = n.double()
+    recall = torch.stack([(has & (rank < K)).sum() for K in recall_at]).double() / nf if recall_at else nf.new_empty(0)
+    mean = ((rank.double() + 1) * has).sum() / nf
+    srt = torch.sort(torch.where(has, rank, torch.full_like(rank, 0x7fffffff))).values
+    med = srt.gather(0, ((n - 1).clamp(min=0) // 2).view(1)).double() + 1
+    med = torch.where(n > 0, med, torch.full_like(med, float("nan")))
+    return torch.cat([recall, mean.view(1), med, nf.view(1)])
+
+
+@torch.no_grad()
+def retrieval_f32(img: Tensor, txt: Tensor, lens: Optional[Tensor], sim: str, normalize: bool, log_scale: float,
+                  frame_group: Optional[Tensor] = None, text_group: Optional[Tensor] = None, k: int = 10,
+                  recall_at=(1, 5, 10), block_bytes: int = 1 << 30) -> dict:
+    """Cross-modal retrieval over a held-out split, both directions, exact and fp32 end to end.
+    sim="flat":  img [N_img, E] / txt [N_txt, E] features before normalisation (normalised iff `normalize`);
+    sim="mean":  img [N_img, HW, E] head outputs (normalised per location iff `normalize`), txt the pooled text
+                 factor [N_txt, E];
+    sim="max":   img as for "mean", txt per-token text features [N_txt, L, E] with lens [N_txt].
+    The scores are the fp32 values classify_ncat / classify_ncat_spatial take their arg-max of: linear_f32 on the
+    (normalised) rows for flat, on the pooled factors for mean, cvcl_spatial_max_scores_f32 (exp(s) included) for max.
+    Each query row orders the keys as torch.sort(row, descending=True, stable=True): a NaN first, ties by ascending
+    key index.  Positives: key i of query i (pair mode, N_img == N_txt), or with frame_group [N_img] / text_group
+    [N_txt] (int64) every key whose group equals the query's.  The score blocks hold at most block_bytes of fp32 query
+    rows (at least one row; a text->image "max" block at least ceil(64 / L) texts, so that the scores kernel plans
+    every block alike and computes the same bits), so the [N_img, N_txt] matrix exists only when it fits.
+    -> {"image_to_text": d, "text_to_image": d}, d = {"topk": int32 [Nq, k], "logits": fp32 [Nq, k] (exp(s) * score),
+        "rank": int32 [Nq] (0-based position of the first positive, -1 without one), "recall": {K: fraction of the
+        queries with a positive whose rank < K}, "mean_rank", "median_rank" (1-based, lower median),
+        "n_queries": queries with a positive}.  One device-to-host read, at the end."""
+    if sim not in ("flat", "mean", "max"):
+        raise ValueError("retrieval_f32: sim must be 'flat', 'mean' or 'max' (got %r)" % (sim,))
+    if sim == "flat":
+        if img.dim() != 2 or txt.dim() != 2 or img.shape[1] != txt.shape[1]:
+            raise ValueError("retrieval_f32: flat features must be img [N_img, E] and txt [N_txt, E], got %s and %s"
+                             % (tuple(img.shape), tuple(txt.shape)))
+    else:
+        if img.dim() != 3:
+            raise ValueError("retrieval_f32: img %s is not [N_img, HW, E]" % (tuple(img.shape),))
+        _check_spatial_text(txt, lens, sim, img.shape[2], "retrieval_f32")
+    recall_at = tuple(recall_at)
+    check_retrieval_args(img.shape[0], txt.shape[0], frame_group, text_group, k, recall_at, block_bytes)
+    _need_cuda(img, txt, lens if sim == "max" else None, frame_group, text_group)
+    fg = _i64(frame_group) if frame_group is not None else None
+    tg = _i64(text_group) if text_group is not None else None
+    n_img, n_txt = img.shape[0], txt.shape[0]
+    min_t2i = 1
+    if sim == "max":
+        rows = _location_rows(img, normalize)
+        tok, lens = _f32(txt), _i64(lens)
+        i2t = lambda q0, q1: _spatial_max_scores(rows[q0:q1], tok, lens, None, 0, log_scale)          # noqa: E731
+        t2i = lambda q0, q1: _spatial_max_scores(rows, tok[q0:q1], lens[q0:q1], None, 0,               # noqa: E731
+                                                 log_scale).t().contiguous()
+        min_t2i = -(-RETRIEVAL_MAX_K // tok.shape[1])     # the plan depends on min(texts * L, 64) token rows
+        scale = None                                      # the max scores carry exp(s) already
+    else:
+        if sim == "flat":
+            i = normalize_rows_f32(img) if normalize else _f32(img)
+            t = normalize_rows_f32(txt) if normalize else _f32(txt)
+        else:
+            i, t = _raw(spatial_pool_fwd)(_location_rows(img, normalize)), _f32(txt)
+        i2t = lambda q0, q1: linear_f32(i[q0:q1], t, None)                                             # noqa: E731
+        t2i = lambda q0, q1: linear_f32(t[q0:q1], i, None)                                             # noqa: E731
+        scale = math.exp(float(log_scale))
+    out, metrics = {}, []
+    for name, block, nq, nk, qg, kg, mr in (("image_to_text", i2t, n_img, n_txt, fg, tg, 1),
+                                            ("text_to_image", t2i, n_txt, n_img, tg, fg, min_t2i)):
+        topk, logits, rank = _retrieval_direction(block, nq, nk, qg, kg, k, scale, block_bytes, mr, img.device)
+        out[name] = {"topk": topk, "logits": logits, "rank": rank}
+        metrics.append(_retrieval_metrics(rank, recall_at))
+    host = torch.stack(metrics).cpu().tolist()
+    nr = len(recall_at)
+    for name, h in zip(out, host):
+        out[name].update(recall={K: h[j] for j, K in enumerate(recall_at)}, mean_rank=h[nr], median_rank=h[nr + 1],
+                         n_queries=int(h[nr + 2]))
+    return out
 
 
 # ----------------------------------------------------------------------------------------
